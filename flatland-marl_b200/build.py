@@ -26,7 +26,7 @@ def needs_build():
     if not os.path.exists(LIB):
         return True
     t = os.path.getmtime(LIB)
-    srcs = [os.path.join(HERE, "csrc", f) for f in os.listdir(os.path.join(HERE, "csrc")) if f.endswith((".cu", ".cuh"))]
+    srcs = [os.path.join(HERE, "csrc", f) for f in os.listdir(os.path.join(HERE, "csrc")) if f.endswith((".cu", ".cuh", ".h"))]
     return any(os.path.getmtime(p) > t for p in srcs + [HDR])
 
 
