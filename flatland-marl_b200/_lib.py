@@ -11,6 +11,7 @@ ACTION_ABSENT = 255
 ST_STEP_AFTER_DONE, ST_AUTO_RESET, ST_BAD_CELL = 1, 2, 4
 FLAG_AUTO_RESET, FLAG_FRESH_AGENTS = 1, 2
 RESET_KEEP_SCHEDULE, RESET_KEEP_ARRIVAL = 1, 2
+COPY_WORLD, COPY_STATE = 1, 2
 
 # field order of struct FlBatch (include/flatland_b200.h)
 _FIELDS = [("E", "i"), ("N", "i"), ("H", "i"), ("W", "i"), ("n_slots", "i"), ("S", "i"), ("ent_cap", "i"), ("grid_stride", "i"),
@@ -36,7 +37,7 @@ class FlObsBuffers(C.Structure):
 
 
 EXPORTS = ["fl_abi_version", "fl_batch_sizeof", "fl_error_string", "fl_distance_map", "fl_distance_map_ids", "fl_walk_tables", "fl_walk_tables_ids", "fl_reset", "fl_reset_ex", "fl_step",
-           "fl_observe", "fl_observe_override", "fl_observe_plan", "fl_observe_ws_words", "fl_batch_slice", "fl_step_observe_host", "fl_step_observe_host_compact", "fl_wire_bytes", "fl_host_threads", "fl_launch_count", "fl_profile_num_kernels", "fl_profile_kernel_name",
+           "fl_observe", "fl_observe_override", "fl_observe_plan", "fl_observe_ws_words", "fl_batch_slice", "fl_copy_envs", "fl_step_observe_host", "fl_step_observe_host_compact", "fl_wire_bytes", "fl_host_threads", "fl_launch_count", "fl_profile_num_kernels", "fl_profile_kernel_name",
            "fl_profile_enable", "fl_profile_collect"]
 
 _lib = None
@@ -84,6 +85,8 @@ def lib():
     L.fl_observe_plan.argtypes = [C.POINTER(FlBatch), P, C.c_int]
     L.fl_observe_plan.restype = C.c_int
     L.fl_batch_slice.argtypes = [C.POINTER(FlBatch), C.c_int64, C.c_int64, C.POINTER(FlBatch)]
+    L.fl_copy_envs.argtypes = [C.POINTER(FlBatch), C.POINTER(FlBatch), P, P, C.c_int64, C.c_uint32, C.POINTER(FlObsBuffers),
+                               C.POINTER(FlObsBuffers), P]
     L.fl_profile_num_kernels.restype = C.c_int
     L.fl_profile_kernel_name.restype = C.c_char_p
     L.fl_profile_kernel_name.argtypes = [C.c_int]
@@ -91,7 +94,7 @@ def lib():
     L.fl_profile_enable.restype = None
     L.fl_profile_collect.argtypes = [P, P, C.c_int]
     L.fl_profile_collect.restype = C.c_int
-    for f in ("fl_distance_map", "fl_distance_map_ids", "fl_walk_tables", "fl_walk_tables_ids", "fl_reset", "fl_reset_ex", "fl_step", "fl_observe", "fl_step_observe_host", "fl_batch_slice"):
+    for f in ("fl_distance_map", "fl_distance_map_ids", "fl_walk_tables", "fl_walk_tables_ids", "fl_reset", "fl_reset_ex", "fl_step", "fl_observe", "fl_step_observe_host", "fl_batch_slice", "fl_copy_envs"):
         getattr(L, f).restype = C.c_int
     if L.fl_batch_sizeof() != C.sizeof(FlBatch):
         raise FlatlandB200Error("FlBatch layout mismatch: library %d bytes, binding %d bytes"

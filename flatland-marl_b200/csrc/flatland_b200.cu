@@ -32,6 +32,7 @@
 #include "observe.cuh"
 #include "bfs.cuh"
 #include "wire.cuh"
+#include "copy.cuh"
 #include "expand_pool.h"
 
 #include <chrono>
@@ -47,8 +48,8 @@ std::atomic<uint64_t> g_launches{0};
 
 // Optional per-kernel timing (fl_profile_*): every launch is bracketed by CUDA events recorded on the
 // launching stream; fl_profile_collect turns them into per-kernel totals.  Off by default.
-enum KernelId : int { K_BFS = 0, K_RESET, K_STEP, K_OBSERVE, K_WALKS, K_OBSERVE_INDEX, K_OBSERVE_TREES, K_PACK, K_COUNT };
-const char *const kKernelNames[K_COUNT] = {"k_bfs", "k_reset", "k_step", "k_observe", "k_walks", "k_observe_index", "k_observe_trees", "k_pack"};
+enum KernelId : int { K_BFS = 0, K_RESET, K_STEP, K_OBSERVE, K_WALKS, K_OBSERVE_INDEX, K_OBSERVE_TREES, K_PACK, K_COPY, K_COUNT };
+const char *const kKernelNames[K_COUNT] = {"k_bfs", "k_reset", "k_step", "k_observe", "k_walks", "k_observe_index", "k_observe_trees", "k_pack", "k_copy_envs"};
 struct ProfRec { int id; cudaEvent_t a, b; };
 std::mutex g_prof_mu;
 bool g_prof_on = false;
@@ -496,19 +497,61 @@ int fl_batch_slice(const FlBatch *b, int64_t e0, int64_t n, FlBatch *out) {
     if (!b || !out || e0 < 0 || n <= 0 || e0 + n > b->E) return FL_ERR_BAD_ARG;
     *out = *b;
     out->E = n;
-    const int64_t N = b->N;
-#define FL_ADV(field, per_env) out->field = b->field ? b->field + (size_t)e0 * (size_t)(per_env) : b->field;
-    FL_ADV(grid, b->grid_stride) FL_ADV(slot_rc, b->n_slots * 2) FL_ADV(dist, b->dist_stride) FL_ADV(max_steps, 1)
-    FL_ADV(init_rc, N * 2) FL_ADV(tgt_rc, N * 2) FL_ADV(init_dir, N) FL_ADV(max_count, N) FL_ADV(slot, N) FL_ADV(speed, N)
-    FL_ADV(earliest, N) FL_ADV(latest, N) FL_ADV(sched, b->S * N)
-    FL_ADV(ridx, b->ridx_stride) FL_ADV(srec, b->state_stride) FL_ADV(wrec, b->state_stride * 4) FL_ADV(whoff, b->state_stride)
-    FL_ADV(wlist, b->wlist_stride) FL_ADV(whits, b->whits_stride) FL_ADV(kcls, b->state_stride) FL_ADV(sdist, b->n_slots * b->state_stride) FL_ADV(gtab, b->n_slots * b->state_stride) FL_ADV(walk_total, 4)
-    FL_ADV(rc, N * 2) FL_ADV(old_rc, N * 2) FL_ADV(dir, N) FL_ADV(old_dir, N) FL_ADV(state, N) FL_ADV(ctr, N) FL_ADV(mal, N)
-    FL_ADV(saved, N) FL_ADV(sig_mal, N) FL_ADV(deadlocked, N) FL_ADV(done, N) FL_ADV(nmal, N) FL_ADV(arrival, N)
-    FL_ADV(elapsed, 1) FL_ADV(sched_pos, 1) FL_ADV(done_all, 1) FL_ADV(status, 1)
-    FL_ADV(stats, 4) FL_ADV(entries, b->ent_cap) FL_ADV(segs, b->seg_stride) FL_ADV(debug_clocks, 32) FL_ADV(obs_ws, b->ws_stride) FL_ADV(tree_cache, b->N * FL_TREE_CACHE_WORDS) FL_ADV(path_cache, b->N * b->pc_stride)
+#define FL_ADV(field, per_env, part) out->field = b->field ? b->field + (size_t)e0 * (size_t)(per_env) : b->field;
+    FL_BATCH_FIELDS(FL_ADV, b)
 #undef FL_ADV
     return FL_OK;
+}
+
+int fl_copy_envs(const FlBatch *src, const FlBatch *dst, const int32_t *d_src_ids, const int32_t *d_dst_ids, int64_t n,
+                 uint32_t parts, const FlObsBuffers *d_src_out, const FlObsBuffers *d_dst_out, void *stream) {
+    if (!src || !dst || !d_src_ids || !d_dst_ids || (parts & ~(FL_COPY_WORLD | FL_COPY_STATE))) return FL_ERR_BAD_ARG;
+    const bool outs = d_src_out && d_dst_out;
+    if (!parts && !outs) return FL_ERR_BAD_ARG;
+    if ((d_src_out != nullptr) != (d_dst_out != nullptr)) return FL_ERR_BAD_ARG;
+    if (src->E <= 0 || dst->E <= 0 || src->N <= 0 || src->N != dst->N || n <= 0 || n > dst->E) return FL_ERR_BAD_ARG;
+    if (parts & FL_COPY_WORLD) {
+        // the world part depends on every shape and table stride; the tables must be built (state_stride > 0)
+        if (src->H != dst->H || src->W != dst->W || src->n_slots != dst->n_slots || src->S != dst->S ||
+            src->grid_stride != dst->grid_stride || src->dist_stride != dst->dist_stride || src->ridx_stride != dst->ridx_stride ||
+            src->state_stride != dst->state_stride || src->wlist_stride != dst->wlist_stride ||
+            src->whits_stride != dst->whits_stride || src->pc_stride != dst->pc_stride || src->state_stride <= 0)
+            return FL_ERR_BAD_ARG;
+        // a cache present in the destination only would keep entries of the world it held before
+        if (!src->tree_cache != !dst->tree_cache || !src->path_cache != !dst->path_cache) return FL_ERR_BAD_ARG;
+    }
+    CopyPlan plan;
+    plan.n_ranges = 0;
+    int64_t voff = 0;
+    bool missing = false;
+    auto add = [&](const void *s, void *d, int64_t bytes) {
+        if (!s || !d) { missing = true; return; }
+        plan.r[plan.n_ranges++] = {static_cast<const char *>(s), static_cast<char *>(d), bytes, voff};
+        voff += (bytes + 15) / 16 * 16;
+    };
+#define FL_RANGE(field, per_env, part)                                                                                   \
+    if ((part) & parts) {                                                                                                  \
+        if (((part) & FL_PART_OPTIONAL) && !src->field) {}                                                                 \
+        else add(src->field, (void *)dst->field, (int64_t)(per_env) * (int64_t)sizeof(*src->field));                   \
+    }
+    FL_BATCH_FIELDS(FL_RANGE, src)
+#undef FL_RANGE
+    if (outs) {
+#define FL_RANGE(field, per_env) add(d_src_out->field, d_dst_out->field, (int64_t)(per_env) * (int64_t)sizeof(*d_src_out->field));
+        FL_OBS_FIELDS(FL_RANGE, src->N)
+#undef FL_RANGE
+    }
+    if (missing) return FL_ERR_BAD_ARG;
+    plan.chunks = (voff + COPY_CHUNK - 1) / COPY_CHUNK;
+    plan.src_E = src->E;
+    plan.dst_E = dst->E;
+    if (n * plan.chunks > 0x7fffffffll) return FL_ERR_BAD_ARG;
+    cudaStream_t st = (cudaStream_t)stream;
+    {
+        LaunchScope ls(K_COPY, st);
+        k_copy_envs<<<(unsigned)(n * plan.chunks), COPY_THREADS, 0, st>>>(plan, d_src_ids, d_dst_ids);
+    }
+    return finish(cudaGetLastError());
 }
 
 namespace {

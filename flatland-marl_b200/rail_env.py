@@ -11,7 +11,15 @@ solution/eval_env.py, solution/demo.py and solution/plfActor.py of the reference
 World generation stays reference Python (north star): `RailEnv(...)` with generator arguments
 imports the reference's `flatland` package for rail/line/timetable generation at reset time and
 uploads the result; `RailEnv.from_world(world)` / `RailEnv.view(batch, e)` need no reference.
+
+copy.deepcopy(env) gives an independent environment, as on the reference: it gets its own batch of one environment, a
+device copy of env's slot (BatchedRailEnv.fork_of: world, tables, caches, state, schedule position and the current
+observation), whether env owns its batch or is a view into a shared one, plus copies of the host attributes (dones,
+rewards, observation, elapsed steps, world dict), a new TreeObsForRailEnv bound to the copy and a deep copy of the
+reference environment that generates its worlds, if any.  Given the same action dicts, the copy then returns what env
+returns, across episode ends too; stepping one leaves the other unchanged.
 """
+import copy
 from enum import IntEnum
 
 import numpy as np
@@ -188,9 +196,28 @@ class RailEnv:
 
     @classmethod
     def view(cls, batch, worlds, e):
-        """A reference-API view of environment e of an existing batch (stepping is done on the batch)."""
+        """A reference-API view of environment e of an existing batch (stepping is done on the batch).  The view goes stale
+        when its slot gets another environment (BatchedRailEnv.replace_worlds, copy_from, restore): build a new one."""
         w = worlds[e]
         return cls(width=int(w["W"]), height=int(w["H"]), number_of_agents=int(w["N"]), world=w, batch=batch, index=e)
+
+    def __deepcopy__(self, memo):
+        """An independent environment with its own batch of one (see the module docstring)."""
+        new = RailEnv.__new__(RailEnv)
+        memo[id(self)] = new
+        new.width, new.height, new.number_of_agents, new.device = self.width, self.height, self.number_of_agents, self.device
+        new.world = copy.deepcopy(self.world, memo)
+        new._batch = None if self._batch is None else BatchedRailEnv.fork_of(self._batch, [self._e])
+        new._e = 0
+        new._ref_env = copy.deepcopy(self._ref_env, memo)
+        new._gen_args = copy.deepcopy(self._gen_args, memo)
+        new.obs_builder = TreeObsForRailEnv()
+        new.obs_builder.set_env(new)
+        new.dones, new.rewards_dict = dict(self.dones), dict(self.rewards_dict)
+        new.obs_dict = copy.deepcopy(self.obs_dict, memo)
+        new._max_episode_steps, new._elapsed_steps, new._was_reset = self._max_episode_steps, self._elapsed_steps, self._was_reset
+        new._cache = {}
+        return new
 
     # -- host mirrors ----------------------------------------------------------------------------
     def _state_host(self):

@@ -260,6 +260,24 @@ int fl_step_observe_host(const FlBatch *b, const uint8_t *h_actions, uint8_t *d_
                          const FlObsBuffers *d_out, const FlObsBuffers *h_out, uint32_t flags,
                          int n_chunks, void *stream, void *copy_stream);
 
+/* fl_copy_envs parts */
+#define FL_COPY_WORLD 1u   /* world, schedule, reset-time tables, tree/path caches */
+#define FL_COPY_STATE 2u   /* agent and environment state, status and stats included */
+
+/* copy.deepcopy(env) of the reference (rail_env.py RailEnv is a plain Python object) for many environments in one launch:
+ * slot d_dst_ids[i] of `dst` becomes slot d_src_ids[i] of `src` (device int32[n] each) for the requested parts; the output
+ * rows (observation tensors, rewards, dones) are copied too when d_src_out and d_dst_out are both non-NULL (host structs of
+ * device pointers, [E][...] as in fl_step_observe_host).  Given the same actions, a copied slot then produces the same bytes
+ * as its source, across episode ends too (the schedule rows and sched_pos travel with it).  The per-call scratch of
+ * fl_observe (entries, segs, obs_ws, debug_clocks) is never copied.  `src` may equal `dst`; one source may feed several
+ * destinations; the destination ids must be distinct, and within one batch no id may be both a source and a destination
+ * (the caller's to guarantee, as with fl_distance_map_ids).  A snapshot store is a batch with only the state pointers set:
+ * the shapes and pointers are checked per requested part.  FL_ERR_BAD_ARG before any CUDA call when n is out of range, a
+ * pointer a requested part needs is NULL in either batch, the two batches differ in a shape or stride the requested parts
+ * depend on, or the tree / path caches are present in one batch only (FL_COPY_WORLD).  One launch (k_copy_envs). */
+int fl_copy_envs(const FlBatch *src, const FlBatch *dst, const int32_t *d_src_ids, const int32_t *d_dst_ids, int64_t n,
+                 uint32_t parts, const FlObsBuffers *d_src_out, const FlObsBuffers *d_dst_out, void *stream);
+
 /* The same step with a compact device-to-host format (csrc/wire.cuh): instead of copying 2,438 bytes per agent, a pack
  * kernel rewrites each environment range into ~1.1 KB per agent — tree nodes that are the all -1 "no branch" vector as one
  * bit, adjacency / orders as int8, the 70 flag entries of the attribute vector as bits, every other float as its own 32
