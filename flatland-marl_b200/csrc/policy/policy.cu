@@ -18,12 +18,14 @@
 //                 the row's thread straight from TMEM.
 //   k_tree_leaf   leaves of the Tree-LSTM (K = 12: one MMA k-step), two 192-column accumulators, 16 epilogue warps.
 //   k_prep / k_tree_plan / k_head_final / k_choose: casts, level lists, final 128->5/1 layers, action choice.
+//   rollout.cuh: seeded sampling with log-probabilities (k_sample) and GAE (k_gae) for PPO rollouts.
 #include <cstdlib>
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <math_constants.h>
 
 #include "../../../include/flatland_policy_b200.h"
+#include "rollout.cuh"
 #include "umma.cuh"
 
 using namespace umma;
@@ -1151,21 +1153,7 @@ __global__ void __launch_bounds__(256) k_head_final(const bf16 *__restrict__ y2,
 __global__ void k_choose(const float *__restrict__ logits, const uint8_t *__restrict__ valid, uint8_t *__restrict__ actions, long long n) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    float x[5];
-    int idx[5], cnt = 0;
-    for (int j = 0; j < 5; j++)
-        if (valid[i * 5 + j]) { x[cnt] = logits[i * 5 + j]; idx[cnt++] = j; }
-    if (cnt == 0) { actions[i] = 0; return; }
-    float mx = x[0];
-    for (int j = 1; j < cnt; j++) mx = fmaxf(mx, x[j]);
-    float ex[5], sum = 0.0f;
-    for (int j = 0; j < cnt; j++) { ex[j] = expf(x[j] - mx); sum += ex[j]; }
-    double cdf[5], run = 0.0;
-    for (int j = 0; j < cnt; j++) { run += (double)(ex[j] / sum); cdf[j] = run; }
-    int pick = cnt - 1;
-    for (int j = 0; j < cnt; j++)
-        if (cdf[j] / run > 0.3745401188473625) { pick = j; break; }
-    actions[i] = (uint8_t)idx[pick];
+    actions[i] = rollout::masked_choice(logits + i * 5, valid + i * 5, 0.3745401188473625, nullptr);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1520,6 +1508,28 @@ int fl_policy_forward_f32(const float *const *wts, void *d_workspace, size_t wor
 int fl_policy_choose_actions(const float *d_logits, const uint8_t *d_valid_actions, uint8_t *d_actions, int64_t n, void *stream) {
     if (n <= 0) return -1;
     k_choose<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(d_logits, d_valid_actions, d_actions, n);
+    g_launches++;
+    return (int)cudaGetLastError();
+}
+
+int fl_policy_sample_actions(const float *d_logits, const uint8_t *d_valid_actions, int64_t E, int64_t N, int64_t env_offset,
+                             uint64_t seed, uint64_t step, uint8_t *d_actions, float *d_log_probs, void *stream) {
+    if (!d_logits || !d_valid_actions || !d_actions || !d_log_probs || E <= 0 || N <= 0 || env_offset < 0) return -1;
+    if (env_offset > (1ll << 32) - E) return -1;                      // the environment id is one 32-bit counter word
+    if (N > (1ll << 32) || E > (1ll << 38) / N) return -1;             // agent word; the grid's x extent
+    const long long n = E * N;
+    rollout::k_sample<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(d_logits, d_valid_actions, E, N, env_offset, seed,
+                                                                                   step, d_actions, d_log_probs);
+    g_launches++;
+    return (int)cudaGetLastError();
+}
+
+int fl_policy_gae(const int32_t *d_rewards, const uint8_t *d_dones, const float *d_values, const uint8_t *d_acted, int64_t T,
+                  int64_t E, int64_t N, float gamma, float lam, float *d_advantages, float *d_returns, void *stream) {
+    if (!d_rewards || !d_dones || !d_values || !d_acted || !d_advantages || !d_returns || T <= 0 || E <= 0 || N <= 0) return -1;
+    if (T >= (1ll << 31) || E >= (1ll << 31) || N >= (1ll << 31) || (T + 1) * E > (1ll << 62) / (N + 1)) return -1;
+    rollout::k_gae<<<(unsigned)((E + 3) / 4), 128, 0, (cudaStream_t)stream>>>(d_rewards, d_dones, d_values, d_acted, T, E, N,
+                                                                              (double)gamma, (double)lam, d_advantages, d_returns);
     g_launches++;
     return (int)cudaGetLastError();
 }

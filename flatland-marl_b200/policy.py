@@ -19,7 +19,7 @@ LIB_PATH = os.path.join(HERE, "csrc", "policy", "libflatland_policy_b200.so")
 LAYERS = pw.N_TRANSFORMER
 
 EXPORTS = ["fl_policy_abi_version", "fl_policy_workspace_bytes", "fl_policy_forward", "fl_policy_workspace_bytes_f32",
-           "fl_policy_forward_f32", "fl_policy_choose_actions",
+           "fl_policy_forward_f32", "fl_policy_choose_actions", "fl_policy_sample_actions", "fl_policy_gae",
            "fl_policy_linear", "fl_policy_linear_debug", "fl_policy_debug_clocks", "fl_policy_launch_count"]
 
 
@@ -56,6 +56,10 @@ def lib():
     L.fl_policy_forward_f32.argtypes = [P, P, C.c_size_t, C.c_int64, C.c_int64, P, P, P, P, P, P, P]
     L.fl_policy_choose_actions.restype = C.c_int
     L.fl_policy_choose_actions.argtypes = [P, P, P, C.c_int64, P]
+    L.fl_policy_sample_actions.restype = C.c_int
+    L.fl_policy_sample_actions.argtypes = [P, P, C.c_int64, C.c_int64, C.c_int64, C.c_uint64, C.c_uint64, P, P, P]
+    L.fl_policy_gae.restype = C.c_int
+    L.fl_policy_gae.argtypes = [P, P, P, P, C.c_int64, C.c_int64, C.c_int64, C.c_float, C.c_float, P, P, P]
     L.fl_policy_linear.restype = C.c_int
     L.fl_policy_linear.argtypes = [P, C.c_int64, P, P, P, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int, P]
     L.fl_policy_debug_clocks.restype = None
@@ -173,6 +177,7 @@ class BatchedActor:
             self._f32 = (tens, ptrs)
         self._ws = None
         self._out = None
+        self._sampled = None
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
@@ -212,14 +217,41 @@ class BatchedActor:
         """Actor._choose_action, soft mode (plfActor.py:27-44), for every agent: uint8 [E,N] device tensor."""
         E, N = int(logits.shape[0]), int(logits.shape[1])
         _, (_, _, actions) = self._buffers(E, N)
-        va = valid_actions
-        if va.dtype == torch.bool:
-            va = va.to(torch.uint8)
-        if va.device != self.device or va.dtype != torch.uint8 or not va.is_contiguous():
-            raise ValueError("valid_actions must be a contiguous uint8/bool tensor on %s" % self.device)
+        va = self._valid_u8(valid_actions)
         _check(self.lib.fl_policy_choose_actions(logits.data_ptr(), va.data_ptr(), actions.data_ptr(), E * N, self._stream()),
                "fl_policy_choose_actions")
         return actions
+
+    def _valid_u8(self, valid_actions):
+        va = valid_actions.to(torch.uint8) if valid_actions.dtype == torch.bool else valid_actions
+        if va.device != self.device or va.dtype != torch.uint8 or not va.is_contiguous():
+            raise ValueError("valid_actions must be a contiguous uint8/bool tensor on %s" % self.device)
+        return va
+
+    def sample_actions(self, logits, valid_actions, seed, step, env_offset=0):
+        """Exploration for PPO rollouts (fl_policy_sample_actions): the soft choice of choose_actions with a seeded uniform
+        per agent, drawn from Philox4x32-10 at counter (step, env_offset + e, agent) and key `seed`, so that the draw of an
+        agent depends only on (seed, step, global environment id, agent).  A shard of a multi-GPU sweep passes env_offset =
+        its first global environment id (shard_range).  Returns (actions uint8 [E,N], log_probs float32 [E,N]): the chosen
+        actions and their log-probabilities under the masked softmax of `logits` (log pi_old of the PPO ratio), device
+        tensors reused by the next call."""
+        E, N = int(logits.shape[0]), int(logits.shape[1])
+        if self._sampled is None or self._sampled[0].shape != (E, N):
+            self._sampled = (torch.empty((E, N), dtype=torch.uint8, device=self.device),
+                             torch.empty((E, N), dtype=torch.float32, device=self.device))
+        self._sample_into(logits, valid_actions, seed, step, env_offset, *self._sampled)
+        return self._sampled
+
+    def _sample_into(self, logits, valid_actions, seed, step, env_offset, actions, log_probs):
+        if logits.device != self.device or logits.dtype != torch.float32 or not logits.is_contiguous() or logits.shape[2:] != (5,):
+            raise ValueError("logits must be a contiguous float32 [E,N,5] tensor on %s" % self.device)
+        va = self._valid_u8(valid_actions)
+        E, N = int(logits.shape[0]), int(logits.shape[1])
+        if tuple(va.shape) != (E, N, 5):
+            raise ValueError("valid_actions must be [E,N,5] like logits")
+        _check(self.lib.fl_policy_sample_actions(logits.data_ptr(), va.data_ptr(), E, N, int(env_offset), int(seed) & (2 ** 64 - 1),
+                                                 int(step) & (2 ** 64 - 1), actions.data_ptr(), log_probs.data_ptr(), self._stream()),
+               "fl_policy_sample_actions")
 
     def get_actions(self, obs, valid_actions=None):
         """Actor.get_actions (plfActor.py:15-25) for the whole batch: observation dict -> actions uint8 [E,N]

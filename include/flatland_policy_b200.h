@@ -99,6 +99,39 @@ int fl_policy_forward_f32(const float *const *d_weights, void *d_workspace, size
 int fl_policy_choose_actions(const float *d_logits, const uint8_t *d_valid_actions, uint8_t *d_actions,
                              int64_t n_agents_total, void *stream);
 
+/* Exploration for PPO rollouts: the same masked soft choice as fl_policy_choose_actions, with a seeded uniform per agent and
+ * step in place of the fixed one (csrc/policy/rollout.cuh).  d_logits [E][N][5] f32, d_valid_actions [E][N][5] u8,
+ * d_actions [E][N] u8, d_log_probs [E][N] f32.
+ *
+ * Uniform of agent i of row e: Philox4x32-10 (Random123 constants and round function) with
+ *   counter = (step & 0xffffffff, step >> 32, env_offset + e, i),  key = (seed & 0xffffffff, seed >> 32),
+ * output words x0 x1 x2 x3;  u = ((x0 >> 5) * 67108864.0 + (x1 >> 6)) / 9007199254740992.0   (53 bits, in [0, 1), float64).
+ * Choice: the first valid action whose normalised cumulative probability (fp32 exponentials of logit - max over the valid
+ * actions, cumulated in float64) exceeds u; no valid action -> 0.
+ * log_probs: fp32 (x_a - max) - log(sum of those exponentials) of the chosen action a; 0 when no action is valid.
+ * The draw depends only on (seed, step, env_offset + e, i): a shard that passes env_offset = its first global environment id
+ * samples exactly what one device sampling the whole batch would.  FL_ERR_BAD_ARG before any CUDA call for a NULL pointer,
+ * E <= 0, N <= 0, env_offset < 0 or env_offset + E > 2^32. */
+int fl_policy_sample_actions(const float *d_logits, const uint8_t *d_valid_actions, int64_t E, int64_t N,
+                             int64_t env_offset, uint64_t seed, uint64_t step,
+                             uint8_t *d_actions, float *d_log_probs, void *stream);
+
+/* Generalised advantage estimation over a rollout buffer of T steps of E environments with N agents each.
+ * d_rewards [T+1][E][N] i32 and d_dones [T+1][E][N+1] u8 are the rows the batch returned (row k + 1: after step k; row 0 is
+ * not read; of d_dones only column N, "__all__", is read); d_values [T+1][E] f32 the critic values of rows 0..T;
+ * d_acted [T][E] u8: 0 where step k only reset an environment whose episode had ended (its action was ignored).
+ * With r_k+1 = mean over agents of rewards[k+1][e][:] (the critic is a mean over agents) and d_k+1 = dones[k+1][e][N]:
+ *   delta_k = r_k+1 + gamma V_k+1 (1 - d_k+1) - V_k
+ *   A_k     = delta_k + gamma lam (1 - d_k+1) A_k+1,   A_T = 0,  A_k+1 as stored
+ *   R_k     = A_k + V_k
+ *   A_k = R_k = 0 where acted[k][e] == 0.
+ * An episode that ends at its step limit is terminal (the limit is part of the environment): no bootstrap.  Float64
+ * arithmetic, fp32 results d_advantages, d_returns [T][E].  One warp per environment.  FL_ERR_BAD_ARG before any CUDA call
+ * for a NULL pointer or T, E, N <= 0. */
+int fl_policy_gae(const int32_t *d_rewards, const uint8_t *d_dones, const float *d_values, const uint8_t *d_acted,
+                  int64_t T, int64_t E, int64_t N, float gamma, float lam,
+                  float *d_advantages, float *d_returns, void *stream);
+
 /* One dense layer on the tensor-core path, exposed for tests: C[M][ldc] (bf16) = act(A[M][K] . W[N][K]^T + bias),
  * K and N multiples of 64 / 128, act 0 = none, 1 = GELU(erf). */
 int fl_policy_linear(const uint16_t *d_a, int64_t lda, const uint16_t *d_w, const float *d_bias, uint16_t *d_c,
