@@ -174,6 +174,10 @@ DEVI uint32_t pack_entry(int agent, int t0, int t1, int dh, int dp, int dn, uint
 DEVI uint32_t entry_extra(int tpc, bool done) {
     return (tpc <= 8 ? (uint32_t)(tpc - 1) << 16 : 1u << 20) | ((uint32_t)done << 19);
 }
+// acc |= x when cond != 0, as one predicated OR (the compiler's select + OR is one more instruction per index entry)
+DEVI void or_if(unsigned &acc, unsigned x, unsigned cond) {
+    asm("{\n.reg .pred p;\nsetp.ne.u32 p, %2, 0;\n@p or.b32 %0, %0, %1;\n}" : "+r"(acc) : "r"(x), "r"(cond));
+}
 // rows an entry's agent spends per cell (info: the agents' records, only read for speeds below 1/8)
 DEVI int entry_tpc(uint32_t en, const uint32_t *info) { return ((en >> 20) & 1u) ? (int)(info[en & 1023u] >> 24) : (int)((en >> 16) & 7u) + 1; }
 DEVI uint32_t entry_sort_key(uint32_t en) { return en >> 22; }          // 10 bits: long-lived first, then by t0
@@ -471,7 +475,7 @@ k_observe(FlBatch b, ObsLayout lay, float *__restrict__ out_attr, float *__restr
 #define OBS_TICK(k) do { if (dbg && tid == 0) dbg[(MODE == OBS_TREES ? 16 : 0) + (k)] = clock64(); } while (0)
     if (dbg && tid == 0) {
         dbg[MODE == OBS_TREES ? 31 : 15] = clock64();
-        if (MODE != OBS_TREES || n_parts == 1) { dbg[12] = 0; dbg[13] = 0; dbg[14] = 0; }
+        if (MODE != OBS_TREES || n_parts == 1) { dbg[12] = 0; dbg[13] = 0; dbg[14] = 0; for (int k = 26; k <= 30; k++) dbg[k] = 0; }
     }
     // ---- phase 0: TMA bulk copies of the static world ---------------------------------------------
     const bool use_tma = MODE == OBS_TREES || lay.grid >= 0 || lay.ridx >= 0 || lay.srec >= 0 || lay.wrec >= 0 || lay.whoff >= 0 ||
@@ -1376,6 +1380,7 @@ k_observe(FlBatch b, ObsLayout lay, float *__restrict__ out_attr, float *__restr
                 const int nq = min(qn, 32);
                 if (dbg && lane == 0) atomicAdd(reinterpret_cast<unsigned long long *>(&dbg[14]), 1ull);
                 bool f_conf = false;
+                unsigned cases = 0;                                                 // (debug counters, see below)
                 uint2 q = make_uint2(0u, 0u);
                 if (lane < nq) {
                     q = sq[lane];
@@ -1384,30 +1389,38 @@ k_observe(FlBatch b, ObsLayout lay, float *__restrict__ out_attr, float *__restr
                     const unsigned bk = kcls ? (unsigned)kcls[rail] : rail;
                     const uint32_t s0 = ks[(int)bk - 1], s1 = ks[bk];
                     const int pre = max(0, pt - 1), post = min(NPRED - 1, pt + 1);
-                    unsigned acc = 0;
-                    const int nb = (int)((q.y >> 16) & 15u);
-                    auto candidate = [&](uint32_t en, int t0) {
-                        const int ag = (int)(en & 1023);
-                        const int t1 = entry_long_lived(en) ? NPRED - 1 : (t0 ? t0 + entry_tpc(en, A.info) - 1 : 0);
-                        if (t1 < pre) return;
-                        const int dh = (int)((en >> 10) & 3), dpv = (int)((en >> 12) & 3), dn = (int)((en >> 14) & 3);
-                        const bool done = (en >> 19) & 1u;
-                        const bool in_cur = t0 <= pt && pt <= t1, in_pre = t0 <= pre && pre <= t1,
-                                   in_post = t0 <= post && post <= t1;
-                        const int pdir = pt < t0 ? dpv : (pt > t1 ? dn : dh);  // always the direction at row pt
-                        const bool cf = (d != pdir && tbit(nb, (pdir + 2) & 3)) || done;
-                        const bool other = ag != h;
-                        const unsigned m_in = (in_cur ? 1u : 0u) | (in_pre ? 2u : 0u) | (in_post ? 4u : 0u);   // rows of the window the entry covers
-                        acc |= (other ? m_in : 0u) | (cf ? m_in << 3 : 0u);
+                    // Everything that depends on the cell alone is settled before the first entry, so that an entry costs a few
+                    // shifts.  m4 below is the entry's rows of the window, shifted left by 2 (bit 2: pt, 3: pre, 4: post).
+                    // * Rows: byte k of GE holds the rows at or after t0 = pt - 1 + k, byte k of LE the rows at or before
+                    //   t1 = pt + 1 - k; a clamping shift by 8 k with k >= 0 selects the byte (k >= 4 reads 0).  Where the window
+                    //   is cut (pt = 0: pre = pt, pt = 500: post = pt) the coinciding rows are set together, as the three separate
+                    //   interval tests set them.
+                    // * The entry's direction at row pt is dh when the entry covers pt, dpv when its interval starts after pt (it
+                    //   then covers post alone, m4 = 16) and dn when it ends before pt (pre alone, m4 = 8): nibble m4 / 4 of PD is
+                    //   the bit position of that direction in the entry.  (Its odd neighbour nibbles never reach the low five bits
+                    //   that a wrapping shift uses: all entries of PD are even.)
+                    // * It crosses the observer when it moves in a direction p != d whose reverse leaves the cell
+                    //   (tbit(nb, (p + 2) & 3) is bit p ^ 1 of nb); Xrep repeats that 4-bit mask over the word, so that a
+                    //   rotation by any amount whose low two bits are p brings bit p to bit 0.
+                    const unsigned nb = (q.y >> 16) & 15u;
+                    const unsigned Xrep = (((nb & 5u) << 1 | (nb >> 1 & 5u)) & ~(1u << d)) * 0x11111111u;
+                    const uint32_t GE = 0x0010141Cu | (pt == 0 ? 0x0800u : 0u), LE = 0x00080C1Cu | (pt == NPRED - 1 ? 0x1000u : 0u);
+                    constexpr uint32_t PD = 0xAAACAEAAu;
+                    const int cge = 8 - 8 * pt, cle = 8 * pt + 8;                // GE shift = 8 t0 + cge, LE shift = cle - 8 t1
+                    unsigned acc_o = 0, acc_c = 0;                               // m4 of the entries of other agents / of crossing ones
+                    auto visit = [&](uint32_t en, uint32_t m4) {
+                        const uint32_t pdir = __funnelshift_r(en, 0u, PD >> m4);                    // low two bits: direction
+                        or_if(acc_o, m4, (en ^ (uint32_t)h) & 1023u);
+                        or_if(acc_c, m4, (__funnelshift_r(Xrep, Xrep, pdir) | en >> 19) & 1u);     // crosses, or its agent is DONE
                     };
                     uint32_t idx = s0;
-                    for (; idx < s1; idx++) {                                    // long-lived entries come first
+                    for (; idx < s1; idx++) {                                    // long-lived entries come first: t1 = 500
                         const uint32_t en = ent_at(idx);
-                        if (!entry_long_lived(en)) break;
-                        const int t0 = entry_t0(en);
-                        if (t0 > post) break;                                    // ordered by t0: none of the rest has started yet
-                        candidate(en, t0);
+                        const int t0 = (int)entry_sort_key(en);
+                        if (t0 > post) break;                                    // a regular entry, or none of the rest has started yet
+                        visit(en, __funnelshift_rc(GE, 0u, (unsigned)max(8 * t0 + cge, 0)) & 0x1Cu);
                     }
+                    if (dbg && idx > s0) cases |= 8u;
                     // regular entries follow, ordered by t0: only those with pre - tpc_max < t0 <= post can matter.  The search runs
                     // on the bucket's sort key (long-lived entries first), so long-lived entries still ahead of idx are skipped too
                     const int t_lo = pre - tpc_max + 1;
@@ -1417,16 +1430,47 @@ k_observe(FlBatch b, ObsLayout lay, float *__restrict__ out_attr, float *__restr
                         const uint32_t mid = (lo + hi) >> 1;
                         if (ent_at(mid) < (key_lo << 22)) lo = mid + 1; else hi = mid;
                     }
-                    for (idx = lo; idx < s1; idx++) {
-                        const uint32_t en = ent_at(idx);
-                        const int t0 = entry_t0(en);
-                        if (t0 > post) break;
-                        candidate(en, t0);
+                    // Two entries per round, loaded together.  The entries that matter are a prefix (sorted by t0, up to the first t0
+                    // past post, which covers no row); the round's second entry is the later one, so it alone decides the break.
+                    // Past the bucket's end reads a sentinel entry whose t0 is past every window.
+                    constexpr uint32_t PAST = 0xFFC00000u;
+                    for (idx = lo;; idx += 2) {
+                        uint32_t en2[2];
+                        int tpc1[2];                                             // rows per cell - 1
+#pragma unroll
+                        for (int u = 0; u < 2; u++) {
+                            en2[u] = idx + u < s1 ? ent_at(idx + u) : PAST;
+                            tpc1[u] = (int)((en2[u] >> 16) & 7u);
+                        }
+                        if ((en2[0] | en2[1]) & (1u << 20)) {                    // slower than 1/8: rare, kept off the common path
+#pragma unroll
+                            for (int u = 0; u < 2; u++) tpc1[u] = entry_tpc(en2[u], A.info) - 1;
+                            if (dbg) cases |= 16u;
+                        }
+#pragma unroll
+                        for (int u = 0; u < 2; u++) {
+                            const uint32_t en = en2[u];
+                            const int t0 = (int)entry_sort_key(en) - 512;
+                            const int t1 = min(t0 + tpc1[u], t0 << 9);           // element 0 (t0 = 0) is row 0 only
+                            visit(en, __funnelshift_rc(GE, 0u, (unsigned)max(8 * t0 + cge, 0)) &
+                                      __funnelshift_rc(LE, 0u, (unsigned)max(cle - 8 * t1, 0)) & 0x1Cu);
+                        }
+                        if ((int)entry_sort_key(en2[1]) > 512 + post) break;
                     }
+                    const unsigned acc = acc_o >> 2 | acc_c << 1;            // bits 0-2: rows with another agent, 3-5: crossing
+                    if (dbg) cases |= (pt <= 1 ? 1u : 0u) | (pt == NPRED - 1 ? 2u : 0u) | (s1 - s0 > 16 ? 4u : 0u);
                     // treeobs.cpp:379-465: the first of the rows cur, pre, post that holds another agent decides, and it decides
                     // "conflict" when an entry of that row crosses the observer's direction (or belongs to a DONE agent):
                     // (acc & 1) ? (acc & 8) : (acc & 2) ? (acc & 16) : (acc & 4) ? (acc & 32) : false, as a 64-entry bit table
                     f_conf = (bool)((0xfe54ba10ee44aa00ull >> acc) & 1ull);
+                }
+                if (dbg) {
+                    // checks whose window starts at row 0 / ends at row 500, of buckets above 16 entries, that visited long-lived
+                    // entries, that met an entry of a train slower than 1/8 (the cases the tests of the conflict check must reach)
+                    for (int k = 0; k < 5; k++) {
+                        const unsigned m = __ballot_sync(0xFFFFFFFFu, (cases >> k) & 1u);
+                        if (lane == 0 && m) atomicAdd(reinterpret_cast<unsigned long long *>(&dbg[26 + k]), (unsigned long long)__popc(m));
+                    }
                 }
                 {
                     // A node keeps the FIRST conflict of its walk.  The queue holds cells in flat-list order (node after node,
