@@ -30,6 +30,7 @@ struct GemmArgs {
     const float *a2; long long lda2; int K2;
     const float *w; const float *bias; float *c; long long ldc;
     long long M; const int32_t *d_M; int N; int act;      // act: 0 none, 1 GELU(erf)
+    float *pre;                                           // when set: the value before the activation, at c's offsets (training forward)
 };
 
 __device__ __forceinline__ float gelu_erf(float x) { return x * 0.5f * (1.0f + erff(x * 0.70710678118654752440f)); }
@@ -81,6 +82,7 @@ __global__ void __launch_bounds__(256) k_gemm_f32(GemmArgs g) {
             const int n = n0 + tx * 4 + j;
             if (n >= g.N) continue;
             float v = acc[i][j] + (g.bias ? g.bias[n] : 0.0f);
+            if (g.pre) g.pre[m * g.ldc + n] = v;
             if (g.act == 1) v = gelu_erf(v);
             g.c[m * g.ldc + n] = v;
         }
@@ -194,8 +196,10 @@ __global__ void k_copy_cols(const float *__restrict__ src, long long lds, float 
 }
 
 // nn.MultiheadAttention over the agents of one environment (net_tree.py:20-32): one warp per (agent, head), 64 dims = 2 per
-// lane; softmax with the running maximum; qkv [T][768] = q | k | v, out [T][ldo] columns head*64..
-__global__ void k_attention(const float *__restrict__ qkv, float *__restrict__ out, long long ldo, long long n_env, int N) {
+// lane; softmax with the running maximum; qkv [T][768] = q | k | v, out [T][ldo] columns head*64..; lse (when set, training
+// forward): [T][4] log-sum-exp of the scores, from which the backward recomputes the probabilities
+__global__ void k_attention(const float *__restrict__ qkv, float *__restrict__ out, long long ldo, long long n_env, int N,
+                            float *__restrict__ lse) {
     const long long wid = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (wid >= n_env * N * 4) return;
@@ -219,6 +223,7 @@ __global__ void k_attention(const float *__restrict__ qkv, float *__restrict__ o
     }
     out[agent * ldo + head * 64 + lane] = o0 / den;
     out[agent * ldo + head * 64 + lane + 32] = o1 / den;
+    if (lse && lane == 0) lse[agent * 4 + head] = mx + logf(den);
 }
 
 // last layers: logits[a][0..4] = actor_net.4(y_actor[a]); value[env] = mean_a critic_net.4(y_critic[a])

@@ -1,0 +1,146 @@
+"""PolicyLearner — the PPO loss and its gradients for the reference network, computed on the device.
+
+Holds the fp32 master parameters of the reference `Network` (solution/nn/net_tree.py:33-72) as torch Parameters and fills
+their `.grad` with fl_policy_ppo_grad_f32 (include/flatland_policy_b200.h): a training forward in the fp32 path's arithmetic,
+the clipped-surrogate PPO loss and a deterministic backward pass, all CUDA kernels of the library.  The optimiser is the
+caller's: `torch.optim` and `torch.nn.utils.clip_grad_norm_` work on `parameters()` as on any module.
+"""
+import ctypes as C
+from collections import OrderedDict
+
+import torch
+
+from . import policy_weights as pw
+from ._lib import FlatlandB200Error
+from .policy import BatchedActor, FlPpoParams, _check, lib, weights_dict
+
+OBS_KEYS = (("agent_attr", torch.float32, (83,)), ("forest", torch.float32, (31, 12)), ("adjacency", torch.int32, (30, 3)),
+            ("node_order", torch.int32, (31,)))
+MB_KEYS = OBS_KEYS + (("valid_actions", torch.uint8, (5,)), ("actions", torch.uint8, ()), ("log_probs", torch.float32, ()))
+ROW_KEYS = (("advantages", torch.float32), ("returns", torch.float32), ("acted", torch.uint8))
+
+
+class PolicyLearner:
+    """The reference network's parameters, keyed by its state_dict names in weight_spec() order, as fp32 torch Parameters
+    on `device`.
+
+    weights: as BatchedActor — a reference checkpoint path (.pt state_dict or .npz), a state_dict-like dict, or None for
+    `init_weights(seed)`.
+
+    One update:
+        stats = learner.ppo_grad(rollout.minibatch(ids))   # writes every parameter's .grad
+        optimizer.step()                                   # e.g. torch.optim.Adam(learner.parameters())
+        rollout.actor = learner.actor()                    # acting with the new parameters
+    """
+
+    def __init__(self, weights=None, device="cuda:0", seed=0):
+        if not torch.cuda.is_available():
+            raise FlatlandB200Error("PolicyLearner needs a CUDA device (no CPU fallback on the policy path)")
+        self.lib = lib()
+        self.device = torch.device(device)
+        torch.cuda.set_device(self.device)
+        w = pw.check_weights(weights_dict(weights, seed))
+        self._params = OrderedDict((name, torch.nn.Parameter(torch.from_numpy(w[name].copy()).to(self.device)))
+                                   for name, _, _ in pw.weight_spec())
+        self._ws = None
+        self._out = None
+        self._stats = torch.zeros(8, dtype=torch.float32, device=self.device)
+
+    def parameters(self):
+        return iter(self._params.values())
+
+    def named_parameters(self):
+        return iter(self._params.items())
+
+    def state_dict(self):
+        """The parameters as CPU tensors under the reference's state_dict names (loadable by the reference `Network`)."""
+        return OrderedDict((k, v.detach().cpu().clone()) for k, v in self._params.items())
+
+    def actor(self, precision="bf16"):
+        """A BatchedActor with the current parameters.  It copies them to the host once and, for bf16, packs and casts them
+        there (pack_weights): a cost per update, not per minibatch."""
+        return BatchedActor(self.state_dict(), device=self.device, precision=precision)
+
+    def _stream(self):
+        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def _ptrs(self, tensors):
+        return (C.c_void_p * len(tensors))(*[t.data_ptr() for t in tensors])
+
+    def _weights(self):
+        ps = list(self._params.values())
+        for p in ps:
+            if p.device != self.device or p.dtype != torch.float32 or not p.is_contiguous():
+                raise ValueError("parameters must stay contiguous float32 tensors on %s" % self.device)
+        return self._ptrs([p.detach() for p in ps])
+
+    def _check_obs(self, d, keys):
+        a = d["agent_attr"]
+        if a.dim() != 3:
+            raise ValueError("agent_attr must be [E,N,83]")
+        E, N = int(a.shape[0]), int(a.shape[1])
+        for name, dt, tail in keys:
+            if name not in d:
+                raise KeyError("missing %s" % name)
+            t = d[name]
+            if t.device != self.device or t.dtype != dt or not t.is_contiguous():
+                raise ValueError("%s must be a contiguous %s tensor on %s" % (name, dt, self.device))
+            if tuple(t.shape) != (E, N) + tail:
+                raise ValueError("%s must have shape %s, got %s" % (name, (E, N) + tail, tuple(t.shape)))
+        return E, N
+
+    def _outputs(self, E, N):
+        if self._out is None or self._out[0].shape[:2] != (E, N):
+            self._out = (torch.empty((E, N, 5), dtype=torch.float32, device=self.device),
+                         torch.empty((E,), dtype=torch.float32, device=self.device))
+        return self._out
+
+    def forward(self, obs):
+        """Logits [E,N,5] and values [E] of the current parameters: fl_policy_forward_f32, whose bytes are those of the
+        training forward inside ppo_grad.  Device tensors, valid until the next call."""
+        E, N = self._check_obs(obs, OBS_KEYS)
+        need = int(self.lib.fl_policy_workspace_bytes_f32(E * N))
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        logits, value = self._outputs(E, N)
+        _check(self.lib.fl_policy_forward_f32(self._weights(), self._ws.data_ptr(), self._ws.numel(), E, N,
+                                              *(obs[k].data_ptr() for k, _, _ in OBS_KEYS), logits.data_ptr(), value.data_ptr(),
+                                              self._stream()), "fl_policy_forward_f32")
+        return logits, value
+
+    def ppo_grad(self, mb, clip_eps=0.2, vf_coef=0.5, ent_coef=0.01):
+        """PPO loss of a minibatch (Rollout.minibatch's dict: the observation tensors, valid_actions, actions, log_probs
+        [E,N,...], advantages, returns, acted [E]) and its gradient, written into every parameter's .grad (allocated when
+        missing, overwritten otherwise).  The loss is stated in include/flatland_policy_b200.h (fl_policy_ppo_grad_f32).
+
+        Returns the statistics as a float32 [8] device tensor (policy loss, value loss, entropy, approximate KL, clip
+        fraction, |S|, acted rows, total loss), reused by the next call.  The one host synchronisation is the fp32 path's
+        (per-level node counts)."""
+        E, N = self._check_obs(mb, MB_KEYS)
+        for name, dt in ROW_KEYS:
+            t = mb[name]
+            if t.device != self.device or t.dtype != dt or not t.is_contiguous() or tuple(t.shape) != (E,):
+                raise ValueError("%s must be a contiguous %s tensor of shape (%d,) on %s" % (name, dt, E, self.device))
+        if not clip_eps > 0:
+            raise ValueError("clip_eps must be positive")
+        need = int(self.lib.fl_policy_workspace_bytes_grad_f32(E * N))
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = None
+            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        grads = []
+        for p in self._params.values():
+            if p.grad is None or p.grad.shape != p.shape or p.grad.dtype != torch.float32 or p.grad.device != self.device \
+                    or not p.grad.is_contiguous():
+                p.grad = torch.empty_like(p, memory_format=torch.contiguous_format)
+            grads.append(p.grad)
+        logits, value = self._outputs(E, N)
+        params = FlPpoParams(float(clip_eps), float(vf_coef), float(ent_coef))
+        _check(self.lib.fl_policy_ppo_grad_f32(self._weights(), self._ws.data_ptr(), self._ws.numel(), E, N,
+                                               *(mb[k].data_ptr() for k, _, _ in MB_KEYS), *(mb[k].data_ptr() for k, _ in ROW_KEYS),
+                                               C.byref(params), self._ptrs(grads), logits.data_ptr(), value.data_ptr(),
+                                               self._stats.data_ptr(), self._stream()), "fl_policy_ppo_grad_f32")
+        return self._stats
+
+    def last_outputs(self):
+        """(logits [E,N,5], values [E]) of the last ppo_grad or forward call, device tensors."""
+        return self._out

@@ -19,7 +19,8 @@ LIB_PATH = os.path.join(HERE, "csrc", "policy", "libflatland_policy_b200.so")
 LAYERS = pw.N_TRANSFORMER
 
 EXPORTS = ["fl_policy_abi_version", "fl_policy_workspace_bytes", "fl_policy_forward", "fl_policy_workspace_bytes_f32",
-           "fl_policy_forward_f32", "fl_policy_choose_actions", "fl_policy_sample_actions", "fl_policy_gae",
+           "fl_policy_forward_f32", "fl_policy_workspace_bytes_grad_f32", "fl_policy_ppo_grad_f32", "fl_policy_choose_actions",
+           "fl_policy_sample_actions", "fl_policy_gae",
            "fl_policy_linear", "fl_policy_linear_debug", "fl_policy_debug_clocks", "fl_policy_launch_count"]
 
 
@@ -30,6 +31,11 @@ class FlPolicyWeights(C.Structure):
                 ("tf_wqkv", C.c_void_p * LAYERS), ("tf_bqkv", C.c_void_p * LAYERS), ("tf_wo", C.c_void_p * LAYERS),
                 ("tf_bo", C.c_void_p * LAYERS), ("tf_wm", C.c_void_p * LAYERS), ("tf_bm", C.c_void_p * LAYERS)] + \
                [(n, C.c_void_p) for n in ("head_w1", "head_b1", "head_w2a", "head_w2c", "head_b2", "head_w3", "head_b3")]
+
+
+class FlPpoParams(C.Structure):
+    """Mirror of `struct FlPpoParams` (include/flatland_policy_b200.h)."""
+    _fields_ = [("clip_eps", C.c_float), ("vf_coef", C.c_float), ("ent_coef", C.c_float)]
 
 
 _lib = None
@@ -54,6 +60,10 @@ def lib():
     L.fl_policy_workspace_bytes_f32.argtypes = [C.c_int64]
     L.fl_policy_forward_f32.restype = C.c_int
     L.fl_policy_forward_f32.argtypes = [P, P, C.c_size_t, C.c_int64, C.c_int64, P, P, P, P, P, P, P]
+    L.fl_policy_workspace_bytes_grad_f32.restype = C.c_size_t
+    L.fl_policy_workspace_bytes_grad_f32.argtypes = [C.c_int64]
+    L.fl_policy_ppo_grad_f32.restype = C.c_int
+    L.fl_policy_ppo_grad_f32.argtypes = [P, P, C.c_size_t, C.c_int64, C.c_int64] + [P] * 10 + [C.POINTER(FlPpoParams), P, P, P, P, P]
     L.fl_policy_choose_actions.restype = C.c_int
     L.fl_policy_choose_actions.argtypes = [P, P, P, C.c_int64, P]
     L.fl_policy_sample_actions.restype = C.c_int
@@ -125,6 +135,16 @@ def pack_weights(w):
     return {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in d.items()}
 
 
+def weights_dict(weights, seed=0):
+    """A weight source -> reference state_dict as numpy float32: a checkpoint path (.pt state_dict or .npz), a state_dict-like
+    dict of arrays or tensors, or None for `init_weights(seed)`."""
+    if weights is None:
+        return pw.init_weights(seed)
+    if isinstance(weights, (str, os.PathLike)):
+        return pw.load_weights(weights)
+    return {k: (v.detach().cpu().numpy() if hasattr(v, "detach") else np.asarray(v)).astype(np.float32) for k, v in weights.items()}
+
+
 _FP32_FIELDS = ("head_w3",)
 
 
@@ -146,13 +166,7 @@ class BatchedActor:
         self.lib = lib()
         self.device = torch.device(device)
         torch.cuda.set_device(self.device)
-        if weights is None:
-            weights = pw.init_weights(seed)
-        elif isinstance(weights, (str, os.PathLike)):
-            weights = pw.load_weights(weights)
-        else:
-            weights = {k: (v.detach().cpu().numpy() if hasattr(v, "detach") else np.asarray(v)).astype(np.float32) for k, v in weights.items()}
-        self.weights = weights
+        self.weights = weights = weights_dict(weights, seed)
         packed = pack_weights(weights)
         self.t = {}
         for k, v in packed.items():

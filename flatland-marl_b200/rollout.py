@@ -1,8 +1,8 @@
 """Rollout — PPO experience collected on the device, up to the learner's boundary.
 
 T lock-step steps of observation -> policy forward -> seeded sampling (fl_policy_sample_actions) -> step, with every row the
-batch returns copied into a trajectory buffer by one fl_copy_envs launch, and GAE advantages over that buffer
-(fl_policy_gae).  The learner itself (backward pass, PPO update, reward shaping) is the caller's.
+batch returns copied into a trajectory buffer by one fl_copy_envs launch, GAE advantages over that buffer (fl_policy_gae),
+and minibatches of its rows for the learner (PolicyLearner.ppo_grad, learner.py).
 """
 import ctypes as C
 
@@ -67,6 +67,7 @@ class Rollout:
         self.buffer["acted"] = torch.zeros((T, E), dtype=torch.uint8, device=dev)
         self._adv = torch.zeros((T, E), dtype=torch.float32, device=dev)
         self._ret = torch.zeros((T, E), dtype=torch.float32, device=dev)
+        self._have_adv = False
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.batch.device).cuda_stream)
@@ -97,6 +98,7 @@ class Rollout:
             self._copy_row(k + 1)
         self._forward(self.T)
         self.step += self.T
+        self._have_adv = False
         return buf
 
     def advantages(self, gamma=0.99, lam=0.95):
@@ -107,4 +109,28 @@ class Rollout:
         _check(self.actor.lib.fl_policy_gae(buf["rewards"].data_ptr(), buf["dones"].data_ptr(), buf["values"].data_ptr(),
                                             buf["acted"].data_ptr(), self.T, b.E, b.N, float(gamma), float(lam),
                                             self._adv.data_ptr(), self._ret.data_ptr(), self._stream()), "fl_policy_gae")
+        self._have_adv = True
         return self._adv, self._ret
+
+    MINIBATCH_KEYS = ("agent_attr", "forest", "adjacency", "node_order", "valid_actions", "actions", "log_probs")
+
+    def minibatch(self, row_ids):
+        """Rows k * E + e (step k < T, environment e) of the last collect(), gathered into the dict PolicyLearner.ppo_grad
+        takes: the observation tensors, valid_actions, actions and log_probs [M, N, ...] of those rows, advantages and returns
+        [M] of the last advantages() call, and acted [M].  row_ids: a sequence or tensor of ints; ids given on the host are
+        range-checked there, a device tensor is used as it is (no host synchronisation).  Plain torch gathers."""
+        if not self._have_adv:
+            raise ValueError("call advantages() after collect() before taking minibatches")
+        n = self.T * self.batch.E
+        if isinstance(row_ids, torch.Tensor) and row_ids.is_cuda:
+            ids = row_ids.to(device=self.batch.device, dtype=torch.int64)
+        else:
+            ids = torch.as_tensor(row_ids, dtype=torch.int64)
+            if ids.dim() != 1 or ids.numel() == 0 or int(ids.min()) < 0 or int(ids.max()) >= n:
+                raise ValueError("row_ids must be a non-empty list of ints in [0, T*E)")
+            ids = ids.to(self.batch.device)
+        buf = self.buffer
+        rows = lambda t: t[: self.T].reshape((n,) + tuple(t.shape[2:])).index_select(0, ids)
+        mb = {k: rows(buf[k]) for k in self.MINIBATCH_KEYS}
+        mb["advantages"], mb["returns"], mb["acted"] = rows(self._adv), rows(self._ret), rows(buf["acted"])
+        return mb

@@ -93,6 +93,42 @@ int fl_policy_forward_f32(const float *const *d_weights, void *d_workspace, size
                           const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
                           const int32_t *d_node_order, float *d_logits, float *d_value, void *stream);
 
+/* PPO loss and gradients of the fp32 network (csrc/policy/policy_f32_grad.cuh): one training forward with the arithmetic of
+ * fl_policy_forward_f32 (d_logits [E][N][5], d_value [E] bit-identical to it), the loss below, and its gradient with respect
+ * to every parameter, in fp32 on the CUDA cores.
+ *
+ * Inputs as fl_policy_forward_f32, plus per agent d_valid_actions [E][N][5] u8, d_actions [E][N] u8 (the actions taken,
+ * 0..4; a larger value is read as 4), d_old_log_probs [E][N] f32 (log pi_old, as fl_policy_sample_actions wrote it), and
+ * per row d_advantages, d_returns [E] f32, d_acted [E] u8.  With log pi_new(a) = (x_a - max) - log(sum of expf(x_j - max)) over the valid actions
+ * j in action order (the arithmetic of fl_policy_sample_actions), r = exp(log pi_new - log pi_old), A, R, V the row's
+ * advantage, return and critic value (mean over agents):
+ *   S      = the agents of rows with acted = 1 that have at least one valid action; rows = the rows with acted = 1
+ *   L_pol  = mean_S( -min(r A, clip(r, 1 - clip_eps, 1 + clip_eps) A) ), the gradient flowing through r A where
+ *            r A <= clip(r) A (ties included)
+ *   H      = entropy of the masked softmax
+ *   L      = L_pol - ent_coef mean_S(H) + vf_coef mean_rows((V - R)^2)
+ * An empty set contributes 0.  Agents with no valid action have log-probability 0 and no gradient.
+ * d_grads: FL_POLICY_F32_TENSORS device pointers, the shapes of d_weights (weight_spec order), overwritten with dL/dparameter.
+ * d_stats [8] f32: L_pol, mean_rows((V - R)^2), mean_S(H), approximate KL mean_S(log pi_old - log pi_new), clip fraction
+ * mean_S(|r - 1| > clip_eps), |S|, the number of acted rows, L.
+ * Deterministic: no floating-point atomics; weight gradients reduce over fixed row chunks, then in chunk order.  Two calls
+ * with the same inputs give the same bytes.  Synchronises `stream` once (per-level node counts), like the fp32 forward.
+ * d_workspace: fl_policy_workspace_bytes_grad_f32(E*N) bytes (about 250 KB per agent).  FL_ERR_BAD_ARG before any CUDA call
+ * for a NULL pointer (also among d_weights / d_grads), E or N <= 0, a workspace that is too small or clip_eps <= 0. */
+typedef struct FlPpoParams {
+    float clip_eps, vf_coef, ent_coef;
+} FlPpoParams;
+size_t fl_policy_workspace_bytes_grad_f32(int64_t n_agents_total);
+int fl_policy_ppo_grad_f32(const float *const *d_weights, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
+                           const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
+                           const int32_t *d_node_order, const uint8_t *d_valid_actions,
+                           const uint8_t *d_actions, const float *d_old_log_probs,
+                           const float *d_advantages, const float *d_returns,
+                           const uint8_t *d_acted,
+                           const FlPpoParams *params,
+                           float *const *d_grads,
+                           float *d_logits, float *d_value, float *d_stats, void *stream);
+
 /* Actor._choose_action in "soft" mode for every agent (plfActor.py:27-44): masked softmax over the valid actions,
  * then numpy's choice with the generator re-seeded to 42, i.e. the first action whose cumulative probability
  * exceeds 0.3745401188473625; no valid action -> 0.  d_valid_actions [n][5] u8, d_actions [n] u8. */

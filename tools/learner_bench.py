@@ -1,0 +1,143 @@
+"""Cost of one PPO minibatch update's loss and gradients on the device (PolicyLearner.ppo_grad, fl_policy_ppo_grad_f32), on a
+B200, against two yardsticks:
+  - the fp32 forward alone (fl_policy_forward_f32, what the training forward costs without keeping activations);
+  - torch autograd on the GPU over the test suite's torch restatement of the network and loss (tests/policy_grad_oracle.py,
+    fp32, TF32 off), forward + loss + backward.  Its tree index lists are built on the host per call, as the restatement does.
+The three are alternated call by call so that they see the same clocks and neighbours; the working sets (GBs of
+activations) are far larger than the 126 MB L2.
+
+Shapes: Test_03 x 1024 rows (51,200 agents) and a Test_02-shape minibatch of 8192 rows x 20 agents (163,840 agents).  The
+rows come from a Rollout collected with the bf16 actor, so the first pass also measures the spread of the PPO ratio r between
+the bf16 behaviour policy and the fp32 learner.  The card's name and power limit are read in the same run.
+
+    python tools/learner_bench.py --out profiles/learner_bench_b200.json [--calls 5]
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+
+import numpy as np
+import torch
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+
+import bench  # noqa: E402
+import flatland_marl_b200 as fb  # noqa: E402
+import policy_grad_oracle as pgo  # noqa: E402
+
+CASES = [("Test_03", 1024, 2), ("Test_02", 8192, 2)]      # config, rows per minibatch (= environments collected), T
+
+
+def timed(fn):
+    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    torch.cuda.synchronize()
+    a.record()
+    fn()
+    b.record()
+    b.synchronize()
+    return a.elapsed_time(b)
+
+
+def ratio_spread(mb, logits, eps=0.2):
+    """r = exp(log pi_new - log pi_old) over S (acted rows, agents with a valid action), in torch (measurement only)."""
+    valid = mb["valid_actions"].bool()
+    xm = torch.where(valid, logits, torch.full_like(logits, -1e30))
+    lp = (xm - torch.logsumexp(xm, -1, keepdim=True)).gather(-1, mb["actions"].long()[..., None])[..., 0]
+    S = valid.any(-1) & mb["acted"].bool()[:, None]
+    d = (lp - mb["log_probs"])[S].double()
+    r = d.exp()
+    q = torch.quantile((r - 1).abs().float(), torch.tensor([0.5, 0.9, 0.99], device=r.device)).tolist()
+    return dict(agents=int(S.sum()), abs_r_minus_1_p50=q[0], abs_r_minus_1_p90=q[1], abs_r_minus_1_p99=q[2],
+                abs_r_minus_1_max=float((r - 1).abs().max()), r_min=float(r.min()), r_max=float(r.max()),
+                approx_kl=float((-d).mean()), clip_fraction=float(((r - 1).abs() > eps).double().mean()))
+
+
+def run_case(config, E, T, calls):
+    learner = fb.PolicyLearner(None, seed=0)
+    batch = fb.BatchedRailEnv(bench.load_worlds(config, E), auto_reset=True)
+    batch.reset()
+    actor = learner.actor("bf16")
+    for _ in range(10):                                   # past the first steps' cold caches
+        batch.step(actor.get_actions(batch.obs))
+    ro = fb.Rollout(batch, actor, T=T, seed=1234)
+    ro.collect()
+    ro.advantages()
+    ids = list(range(E))                                  # one minibatch = the E rows of step 0
+    mb = ro.minibatch(ids)
+    N = batch.N
+    edge_order = ro.buffer["edge_order"][:T].reshape((T * E, N, 30))[:E].cpu().numpy()
+    obs_keys = ("agent_attr", "forest", "adjacency", "node_order")
+    stats = learner.ppo_grad(mb).cpu().numpy()
+    spread = ratio_spread(mb, learner.last_outputs()[0])
+    # torch yardstick: the restatement in fp32 on the GPU, TF32 off
+    torch.backends.cuda.matmul.allow_tf32 = False
+    torch.backends.cudnn.allow_tf32 = False
+    w = {k: v.detach().cpu().numpy() for k, v in learner.named_parameters()}
+    tp = pgo.params(w, requires_grad=True, dtype=torch.float32, device=learner.device)
+    host = {k: mb[k].cpu().numpy() for k in obs_keys + ("valid_actions", "actions", "log_probs", "advantages", "returns", "acted")}
+
+    def torch_step():
+        for p in tp.values():
+            p.grad = None
+        logits, value = pgo.forward(tp, host["agent_attr"], host["forest"], host["adjacency"], host["node_order"], edge_order)
+        L, _ = pgo.ppo_loss(logits, value, host["valid_actions"], host["actions"], host["log_probs"], host["advantages"],
+                            host["returns"], host["acted"], 0.2, 0.5, 0.01)
+        L.backward()
+    fwd = {k: mb[k] for k in obs_keys}
+    torch_ok = True
+    try:
+        torch_step()
+    except torch.cuda.OutOfMemoryError:
+        torch_ok = False
+        torch.cuda.empty_cache()
+    learner.ppo_grad(mb)
+    learner.forward(fwd)
+    ours, f32, tor = [], [], []
+    for _ in range(calls):
+        ours.append(timed(lambda: learner.ppo_grad(mb)))
+        f32.append(timed(lambda: learner.forward(fwd)))
+        if torch_ok:
+            tor.append(timed(torch_step))
+    med = lambda x: round(float(np.median(x)), 3) if x else None
+    r = dict(config=config, rows=E, agents_per_row=N, agents=E * N,
+             workspace_bytes=int(learner.lib.fl_policy_workspace_bytes_grad_f32(E * N)),
+             ppo_grad_ms=med(ours), fp32_forward_ms=med(f32), torch_autograd_fp32_ms=med(tor) if torch_ok else "out of memory",
+             ppo_grad_ms_calls=[round(x, 3) for x in ours], fp32_forward_ms_calls=[round(x, 3) for x in f32],
+             torch_autograd_fp32_ms_calls=[round(x, 3) for x in tor],
+             ppo_grad_over_forward=round(med(ours) / med(f32), 3),
+             first_pass_stats=dict(zip(("policy_loss", "value_loss", "entropy", "approx_kl", "clip_fraction", "S", "acted_rows",
+                                        "loss"), [float(x) for x in stats])),
+             ratio_bf16_behaviour_fp32_learner=spread)
+    print(json.dumps(r), flush=True)
+    del ro, batch, learner, tp
+    torch.cuda.empty_cache()
+    return r
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--calls", type=int, default=5, help="alternated timed calls per implementation")
+    ap.add_argument("--out", required=True, help="JSON file the results are written to (its directory is created)")
+    args = ap.parse_args()
+    if not torch.cuda.is_available():
+        raise SystemExit("learner_bench needs a CUDA device")
+    try:
+        power = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i", "0"],
+                               capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError):
+        power = "unknown"
+    out = dict(gpu=torch.cuda.get_device_name(0), power_limit=power, calls=args.calls)
+    print(json.dumps(out), flush=True)
+    out["cases"] = [run_case(config, E, T, args.calls) for config, E, T in CASES]
+    os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+    with open(args.out, "w") as f:
+        json.dump(out, f, indent=1)
+    print("wrote", args.out)
+
+
+if __name__ == "__main__":
+    main()
