@@ -1292,6 +1292,310 @@ Workspace carve(void *base, long long M) {
 
 #include "policy_f32.cuh"
 #include "policy_f32_grad.cuh"
+#include "policy_bf16_grad.cuh"
+
+// ---- the PPO graph (training forward, loss, backward), shared by the fp32 and the bf16 learner --------------------------
+// The two learners differ only in the launchers of the 20 large weight matrices' products (Lin::gemm, Lin::dx, Lin::dw):
+// F32Lin runs the fp32 CUDA-core kernels of policy_f32.cuh / policy_f32_grad.cuh, Bf16Lin the tensor-core kernel of
+// policy_bf16_grad.cuh.  Everything else (the 12-feature node terms, the heads' last layer, attention, the gates, the loss)
+// is launched here with the fp32 kernels in both.
+namespace ppograph {
+using namespace f32path;
+using namespace f32grad;
+
+struct F32Lin {
+    cudaStream_t st; float *part;
+    // C = act(A W^T + bias) as k_gemm_f32 (GemmArgs)
+    void gemm(const float *a1, const int32_t *idx1, long long lda1, int K1, const float *a2, long long lda2, int K2,
+              const float *w, const float *bias, float *c, long long ldc, long long M, int Nn, int act, float *pre) {
+        if (M <= 0) return;
+        GemmArgs g{a1, idx1, lda1, K1, a2, lda2, K2, w, bias, c, ldc, M, nullptr, Nn, act, pre};
+        k_gemm_f32<<<dim3((unsigned)((M + 63) / 64), (unsigned)((Nn + 63) / 64)), 256, 0, st>>>(g);
+        g_launches++;
+    }
+    // dX = dY W with the epilogue of k_gemm_dx
+    void dx(const float *a, long long lda, int Nn, const float *w, long long ldw, int K, float *c, const int32_t *cidx, long long ldc,
+            const float *add, long long ldadd, int accum, const float *pre, long long ldpre, long long M) {
+        if (M <= 0) return;
+        DxArgs g{a, lda, Nn, w, ldw, K, c, cidx, ldc, add, ldadd, accum, pre, ldpre, M};
+        k_gemm_dx<<<dim3((unsigned)((M + 63) / 64), (unsigned)((K + 63) / 64)), 256, 0, st>>>(g);
+        g_launches++;
+    }
+    // dW = dY^T X (and db when db != null) over M rows, fixed chunks, then summed in chunk order
+    void dw(const float *dy, long long ldy, int Nn, const float *x1, const int32_t *idx1, long long ldx1, int K1, const float *x2,
+            long long ldx2, int K2, long long M, float *dW, float *db) {
+        const int bias = db ? 1 : 0, Kp = K1 + K2 + bias;
+        int nch = n_chunks(M);
+        long long chunk = 0;
+        if (nch > 0) {
+            chunk = ((M + nch - 1) / nch + 15) & ~15LL;
+            nch = (int)((M + chunk - 1) / chunk);
+            DwArgs g{dy, ldy, Nn, x1, idx1, ldx1, K1, x2, ldx2, K2, bias, M, chunk, part};
+            k_gemm_dw<<<dim3((unsigned)((Nn + 63) / 64), (unsigned)((Kp + 63) / 64), (unsigned)nch), 256, 0, st>>>(g);
+            g_launches++;
+        }
+        k_dw_reduce<<<(unsigned)(((long long)Nn * Kp + 255) / 256), 256, 0, st>>>(part, nch, Nn, K1 + K2, bias, dW, db);
+        g_launches++;
+    }
+};
+
+struct Bf16Lin {
+    cudaStream_t st; float *part;
+    void gemm(const float *a1, const int32_t *idx1, long long lda1, int K1, const float *a2, long long lda2, int K2,
+              const float *w, const float *bias, float *c, long long ldc, long long M, int Nn, int act, float *pre) {
+        using namespace bf16grad;
+        if (M <= 0) return;
+        TcArgs g{};
+        g.a = make_src(a1, idx1, lda1, K1, a2, lda2, K2, M);
+        g.b = make_src(w, nullptr, K1 + K2, K1 + K2, nullptr, 0, 0, Nn);
+        g.red = K1 + K2;
+        g.e = no_epi();
+        g.e.c = c; g.e.ldc = ldc; g.e.rows = M; g.e.cols = Nn; g.e.bias = bias; g.e.pre = pre; g.e.act = act;
+        k_tc_gemm<TC_FWD><<<dim3((unsigned)((M + 127) / 128), (unsigned)((Nn + 127) / 128)), TC_THREADS, TC_SMEM, st>>>(g);
+        g_launches++;
+    }
+    void dx(const float *a, long long lda, int Nn, const float *w, long long ldw, int K, float *c, const int32_t *cidx, long long ldc,
+            const float *add, long long ldadd, int accum, const float *pre, long long ldpre, long long M) {
+        using namespace bf16grad;
+        if (M <= 0) return;
+        TcArgs g{};
+        g.a = make_src(a, nullptr, lda, Nn, nullptr, 0, 0, M);
+        g.b = make_src(w, nullptr, ldw, K, nullptr, 0, 0, Nn);
+        g.red = Nn;
+        g.e = no_epi();
+        g.e.c = c; g.e.cidx = cidx; g.e.ldc = ldc; g.e.rows = M; g.e.cols = K;
+        g.e.add = add; g.e.ldadd = ldadd; g.e.accum = accum; g.e.gpre = pre; g.e.ldgpre = ldpre;
+        k_tc_gemm<TC_DX><<<dim3((unsigned)((M + 127) / 128), (unsigned)((K + 127) / 128)), TC_THREADS, TC_SMEM, st>>>(g);
+        g_launches++;
+    }
+    void dw(const float *dy, long long ldy, int Nn, const float *x1, const int32_t *idx1, long long ldx1, int K1, const float *x2,
+            long long ldx2, int K2, long long M, float *dW, float *db) {
+        using namespace bf16grad;
+        const int bias = db ? 1 : 0, K = K1 + K2, Kp = K + bias;
+        int nch = 0;
+        const long long chunk = dw_chunk(M, &nch);
+        if (nch > 0) {
+            TcArgs g{};
+            g.a = make_src(dy, nullptr, ldy, Nn, nullptr, 0, 0, M);
+            g.b = make_src(x1, idx1, ldx1, K1, x2, ldx2, K2, M);
+            g.red = M; g.chunk = chunk;
+            g.e = no_epi();
+            g.e.c = part; g.e.ldc = Kp; g.e.rows = Nn; g.e.cols = K;
+            g.zstride = (long long)Nn * Kp;
+            k_tc_gemm<TC_DW><<<dim3((unsigned)((Nn + 127) / 128), (unsigned)((K + 127) / 128), (unsigned)nch), TC_THREADS, TC_SMEM, st>>>(g);
+            g_launches++;
+            if (bias) {
+                k_db_part<<<dim3((unsigned)((Nn + 127) / 128), (unsigned)nch), 128, 0, st>>>(dy, ldy, Nn, M, chunk, K, part);
+                g_launches++;
+            }
+        }
+        k_dw_reduce<<<(unsigned)(((long long)Nn * Kp + 255) / 256), 256, 0, st>>>(part, nch, Nn, K, bias, dW, db);
+        g_launches++;
+    }
+};
+
+// the dynamic shared-memory opt-in of k_tc_gemm, per device (as setup() for the inference kernels)
+unsigned long long g_tc_attr_mask = 0;
+int bf16_setup() {
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return (int)e;
+    if (dev < 64 && ((g_tc_attr_mask >> dev) & 1ull)) return 0;
+    using namespace bf16grad;
+    e = cudaFuncSetAttribute(k_tc_gemm<TC_FWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_tc_gemm<TC_DX>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_tc_gemm<TC_DW>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM);
+    if (e != cudaSuccess) return (int)e;
+    if (dev < 64) g_tc_attr_mask |= 1ull << dev;
+    return 0;
+}
+
+struct PpoIn {
+    const float *agent_attr, *forest; const int32_t *adjacency, *node_order;
+    const uint8_t *valid, *actions; const float *old_lp, *adv, *ret; const uint8_t *acted;
+    float eps, vf, ent;
+    float *const *grads; float *logits, *value, *stats;
+};
+
+// The training forward (fl_policy_forward_f32's arithmetic on F32Lin: every level and layer in its own slice of the
+// workspace) and, when `loss`, the PPO loss and the backward pass.  Arguments are checked by the caller.
+template <class Lin>
+int run(Lin &lin, const float *const *wts, Wg &ws, long long E, long long N, const PpoIn &in, bool loss, cudaStream_t st) {
+    F32Lin f32{st, ws.part};
+    const long long T = E * N;
+    auto copy_cols = [&](const float *src, long long lds, float *dst, long long ldd, long long rows, int cols) {
+        k_copy_cols<<<(unsigned)((rows * cols + 255) / 256), 256, 0, st>>>(src, lds, dst, ldd, rows, cols);
+        g_launches++;
+    };
+    auto gelu_bwd = [&](const float *src, long long lds, const float *pre, long long ldp, float *dst, long long ldd, long long rows, int cols) {
+        k_gelu_bwd<<<(unsigned)((rows * cols + 255) / 256), 256, 0, st>>>(src, lds, pre, ldp, dst, ldd, rows, cols);
+        g_launches++;
+    };
+    const float *W_iou = wts[0], *b_iou = wts[1], *U_iou = wts[2], *W_c = wts[3], *b_c = wts[4], *W_f = wts[5], *b_f = wts[6], *U_f = wts[7];
+    float *const *gr = in.grads;
+    const float *d_agent_attr = in.agent_attr, *d_forest = in.forest;
+
+    // ==== training forward: fl_policy_forward_f32's arithmetic, every level and layer in its own slice ====
+    const long long nodes = T * f32path::NODES;
+    cudaError_t err = cudaMemsetAsync(ws.h, 0, (size_t)nodes * T_H * 4, st);
+    if (err == cudaSuccess) err = cudaMemsetAsync(ws.c, 0, (size_t)nodes * T_H * 4, st);
+    if (err == cudaSuccess) err = cudaMemsetAsync(ws.counts, 0, 64 * 4, st);
+    if (err != cudaSuccess) return (int)err;
+    k_clean<<<(unsigned)((nodes * NF + 255) / 256), 256, 0, st>>>(d_forest, ws.xcl, nodes * NF);
+    k_tl_count<<<(unsigned)((T + 127) / 128), 128, 0, st>>>(in.adjacency, in.node_order, T, ws.child_base, ws.tcnt);
+    k_tl_scan<<<dim3((unsigned)ws.nblk, MAX_LEVELS), SCAN, 0, st>>>(ws.tcnt, T, ws.nblk, ws.tpos, ws.btot);
+    k_tl_tops<<<1, 32, 0, st>>>(ws.btot, ws.nblk, ws.counts);
+    k_tl_fill<<<(unsigned)((T + 127) / 128), 128, 0, st>>>(in.node_order, T, ws.nblk, ws.tpos, ws.btot, ws.counts, ws.lists);
+    k_tree_leaves<<<(unsigned)nodes, 128, 0, st>>>(d_forest, in.node_order, nodes, W_iou, b_iou, ws.h, ws.c);
+    g_launches += 6;
+    int32_t counts[MAX_LEVELS];
+    err = cudaMemcpyAsync(counts, ws.counts, sizeof(counts), cudaMemcpyDeviceToHost, st);
+    if (err == cudaSuccess) err = cudaStreamSynchronize(st);        // per-level sizes of the launches below; the only host sync
+    if (err != cudaSuccess) return (int)err;
+    long long loff[MAX_LEVELS + 1];                                  // list offset of every level (leaves first)
+    loff[0] = 0;
+    for (int lv = 0; lv < MAX_LEVELS; lv++) loff[lv + 1] = loff[lv] + counts[lv];
+    const long long n_leaf = counts[0], n_in = loff[MAX_LEVELS] - n_leaf;   // inner index i = list position - n_leaf
+    if (n_in > ws.cap) return -1;
+    for (int lv = 1; lv < MAX_LEVELS; lv++) {
+        const long long M = counts[lv], io = loff[lv] - n_leaf;
+        if (M <= 0) continue;
+        const int32_t *list = ws.lists + loff[lv], *dM = ws.counts + lv;
+        int32_t *mr = ws.merge_row + io, *cr = ws.child_row + 3 * io;
+        float *iou = ws.iou + io * 384, *fraw = ws.fraw + io * 384, *fc = ws.fc + io * 384;
+        k_level_rows<<<(unsigned)((M + 127) / 128), 128, 0, st>>>(list, dM, ws.child_base, mr, cr);
+        g_launches++;
+        lin.gemm(ws.h, mr, T_H, 3 * T_H, nullptr, 0, 0, U_iou, nullptr, iou, 3 * T_H, M, 3 * T_H, 0, nullptr);
+        lin.gemm(ws.h, cr, T_H, T_H, nullptr, 0, 0, U_f, nullptr, fraw, T_H, 3 * M, T_H, 0, nullptr);
+        k_forget<<<(unsigned)M, 384, 0, st>>>(fraw, list, cr, dM, d_forest, W_f, b_f, ws.c, fc);
+        lin.gemm(fc, nullptr, 3 * T_H, 3 * T_H, nullptr, 0, 0, W_c, nullptr, ws.craw, T_H, M, T_H, 0, nullptr);
+        k_inner<<<(unsigned)M, 128, 0, st>>>(iou, ws.craw, list, dM, d_forest, W_iou, b_iou, b_c, ws.h, ws.c);
+        g_launches += 2;
+    }
+    lin.gemm(d_agent_attr, nullptr, 83, 83, nullptr, 0, 0, wts[8], wts[9], ws.aa[0], 256, T, 256, 1, ws.ap[0]);
+    lin.gemm(ws.aa[0], nullptr, 256, 256, nullptr, 0, 0, wts[10], wts[11], ws.aa[1], 256, T, 256, 1, ws.ap[1]);
+    lin.gemm(ws.aa[1], nullptr, 256, 256, nullptr, 0, 0, wts[12], wts[13], ws.aa[2], 256, T, 256, 1, ws.ap[2]);
+    lin.gemm(ws.aa[2], nullptr, 256, 256, nullptr, 0, 0, wts[14], wts[15], ws.emb, 256, T, 128, 1, ws.ap[3]);
+    copy_cols(ws.h, (long long)f32path::NODES * T_H, ws.emb + 128, 256, T, 128);
+    const float *x = ws.emb;
+    for (int l = 0; l < 3; l++) {
+        const float *const *tw = wts + 16 + 6 * l;
+        lin.gemm(x, nullptr, 256, 256, nullptr, 0, 0, tw[0], tw[1], ws.qkv[l], 768, T, 768, 0, nullptr);
+        k_attention<<<(unsigned)((T * 4 * 32 + 255) / 256), 256, 0, st>>>(ws.qkv[l], ws.att[l], 256, E, (int)N, ws.lse[l]);
+        g_launches++;
+        lin.gemm(ws.att[l], nullptr, 256, 256, nullptr, 0, 0, tw[2], tw[3], ws.cat[l] + 256, 512, T, 256, 0, nullptr);
+        copy_cols(x, 256, ws.cat[l], 512, T, 256);
+        lin.gemm(ws.cat[l], nullptr, 512, 512, nullptr, 0, 0, tw[4], tw[5], ws.xs[l], 256, T, 256, 1, ws.mpre[l]);
+        x = ws.xs[l];
+    }
+    const float *const *aw = wts + 34, *const *cw = wts + 40;
+    for (int hd = 0; hd < 2; hd++) {
+        const float *const *hw = hd ? cw : aw;
+        lin.gemm(ws.emb, nullptr, 256, 256, x, 256, 256, hw[0], hw[1], ws.y1[hd], 256, T, 256, 1, ws.y1p[hd]);
+        lin.gemm(ws.y1[hd], nullptr, 256, 256, nullptr, 0, 0, hw[2], hw[3], ws.y2[hd], 128, T, 128, 1, ws.y2p[hd]);
+    }
+    k_heads_final<<<(unsigned)E, 256, (size_t)N * sizeof(float), st>>>(ws.y2[0], ws.y2[1], aw[4], aw[5], cw[4], cw[5], in.logits, in.value, (int)N);
+    g_launches++;
+    if (!loss) return (int)cudaGetLastError();
+
+    // ==== PPO loss: d loss / d logits, d loss / d critic output, statistics ====
+    PpoArgs pa{in.logits, in.value, in.old_lp, in.adv, in.ret, in.valid, in.actions, in.acted, E, (int)N, in.eps, in.vf, in.ent,
+               ws.counts + 32, ws.dlogits, ws.dcrit, ws.rowstats};
+    k_ppo_count<<<(unsigned)E, 128, 0, st>>>(pa);
+    k_ppo_loss<<<(unsigned)E, 128, 0, st>>>(pa);
+    k_ppo_stats<<<1, 256, 0, st>>>(ws.rowstats, E, ws.counts + 32, in.vf, in.ent, in.stats);
+    g_launches += 3;
+
+    // ==== backward: heads (net_tree.py:56-71, 100-110); the last layers (N = 5, 1) stay on F32Lin ====
+    f32.dx(ws.dlogits, 5, 5, aw[4], 128, 128, ws.dy2, nullptr, 128, nullptr, 0, 0, ws.y2p[0], 128, T);
+    f32.dw(ws.dlogits, 5, 5, ws.y2[0], nullptr, 128, 128, nullptr, 0, 0, T, gr[38], gr[39]);
+    lin.dx(ws.dy2, 128, 128, aw[2], 256, 256, ws.dy1, nullptr, 256, nullptr, 0, 0, ws.y1p[0], 256, T);
+    lin.dw(ws.dy2, 128, 128, ws.y1[0], nullptr, 256, 256, nullptr, 0, 0, T, gr[36], gr[37]);
+    lin.dx(ws.dy1, 256, 256, aw[0], 512, 512, ws.dz, nullptr, 512, nullptr, 0, 0, nullptr, 0, T);
+    lin.dw(ws.dy1, 256, 256, ws.emb, nullptr, 256, 256, x, 256, 256, T, gr[34], gr[35]);
+    f32.dx(ws.dcrit, 1, 1, cw[4], 128, 128, ws.dy2, nullptr, 128, nullptr, 0, 0, ws.y2p[1], 128, T);
+    f32.dw(ws.dcrit, 1, 1, ws.y2[1], nullptr, 128, 128, nullptr, 0, 0, T, gr[44], gr[45]);
+    lin.dx(ws.dy2, 128, 128, cw[2], 256, 256, ws.dy1, nullptr, 256, nullptr, 0, 0, ws.y1p[1], 256, T);
+    lin.dw(ws.dy2, 128, 128, ws.y1[1], nullptr, 256, 256, nullptr, 0, 0, T, gr[42], gr[43]);
+    lin.dx(ws.dy1, 256, 256, cw[0], 512, 512, ws.dz, nullptr, 512, nullptr, 0, 1, nullptr, 0, T);      // dz = d cat(emb, att)
+    lin.dw(ws.dy1, 256, 256, ws.emb, nullptr, 256, 256, x, 256, 256, T, gr[40], gr[41]);
+    // ==== three attention blocks (net_tree.py:20-32), last to first ====
+    int cur = 0;
+    gelu_bwd(ws.dz + 256, 512, ws.mpre[2], 256, ws.dx[cur], 256, T, 256);
+    for (int l = 2; l >= 0; l--) {
+        const float *const *tw = wts + 16 + 6 * l;
+        float *const *tg = gr + 16 + 6 * l;
+        const float *xin = l ? ws.xs[l - 1] : ws.emb;
+        const float *dpm = ws.dx[cur];
+        lin.dw(dpm, 256, 256, ws.cat[l], nullptr, 512, 512, nullptr, 0, 0, T, tg[4], tg[5]);                  // att_mlp.0
+        lin.dx(dpm, 256, 256, tw[4], 512, 512, ws.dcat, nullptr, 512, nullptr, 0, 0, nullptr, 0, T);
+        lin.dw(ws.dcat + 256, 512, 256, ws.att[l], nullptr, 256, 256, nullptr, 0, 0, T, tg[2], tg[3]);         // out_proj
+        lin.dx(ws.dcat + 256, 512, 256, tw[2], 256, 256, ws.datt, nullptr, 256, nullptr, 0, 0, nullptr, 0, T);
+        k_attn_bwd_q<<<(unsigned)((T * 4 * 32 + 255) / 256), 256, 0, st>>>(ws.qkv[l], ws.att[l], ws.datt, ws.lse[l], ws.dqkv, ws.Dq, E, (int)N);
+        k_attn_bwd_kv<<<(unsigned)((T * 4 * 32 + 255) / 256), 256, 0, st>>>(ws.qkv[l], ws.datt, ws.lse[l], ws.Dq, ws.dqkv, E, (int)N);
+        g_launches += 2;
+        lin.dw(ws.dqkv, 768, 768, xin, nullptr, 256, 256, nullptr, 0, 0, T, tg[0], tg[1]);                      // in_proj
+        if (l > 0) {   // d(block input) = d cat[:, :256] + dqkv W_in, through the previous block's GELU
+            lin.dx(ws.dqkv, 768, 768, tw[0], 256, 256, ws.dx[cur ^ 1], nullptr, 256, ws.dcat, 512, 0, ws.mpre[l - 1], 256, T);
+            cur ^= 1;
+        } else {       // d emb = dz[:, :256] (heads) + d cat[:, :256] + dqkv W_in, into dz[:, :256]
+            lin.dx(ws.dqkv, 768, 768, tw[0], 256, 256, ws.dz, nullptr, 512, ws.dcat, 512, 1, nullptr, 0, T);
+        }
+    }
+    // ==== attribute MLP (net_tree.py:41-50) on d emb[:, :128] ====
+    gelu_bwd(ws.dz, 512, ws.ap[3], 256, ws.dx[0], 256, T, 128);
+    lin.dw(ws.dx[0], 256, 128, ws.aa[2], nullptr, 256, 256, nullptr, 0, 0, T, gr[14], gr[15]);
+    lin.dx(ws.dx[0], 256, 128, wts[14], 256, 256, ws.dx[1], nullptr, 256, nullptr, 0, 0, ws.ap[2], 256, T);
+    lin.dw(ws.dx[1], 256, 256, ws.aa[1], nullptr, 256, 256, nullptr, 0, 0, T, gr[12], gr[13]);
+    lin.dx(ws.dx[1], 256, 256, wts[12], 256, 256, ws.dx[0], nullptr, 256, nullptr, 0, 0, ws.ap[1], 256, T);
+    lin.dw(ws.dx[0], 256, 256, ws.aa[0], nullptr, 256, 256, nullptr, 0, 0, T, gr[10], gr[11]);
+    lin.dx(ws.dx[0], 256, 256, wts[10], 256, 256, ws.dx[1], nullptr, 256, nullptr, 0, 0, ws.ap[0], 256, T);
+    lin.dw(ws.dx[1], 256, 256, d_agent_attr, nullptr, 83, 83, nullptr, 0, 0, T, gr[8], gr[9]);
+    // ==== Tree-LSTM (TreeLSTM.py:59-154), deepest level first; d h of the roots = d emb[:, 128:] ====
+    err = cudaMemsetAsync(ws.dh, 0, (size_t)nodes * T_H * 4, st);
+    if (err == cudaSuccess) err = cudaMemsetAsync(ws.dc, 0, (size_t)nodes * T_H * 4, st);
+    if (err != cudaSuccess) return (int)err;
+    copy_cols(ws.dz + 128, 512, ws.dh, (long long)f32path::NODES * T_H, T, 128);
+    for (int lv = MAX_LEVELS - 1; lv >= 1; lv--) {
+        const long long M = counts[lv], io = loff[lv] - n_leaf;
+        if (M <= 0) continue;
+        const int32_t *list = ws.lists + loff[lv], *mr = ws.merge_row + io, *cr = ws.child_row + 3 * io;
+        float *dG = ws.dG + loff[lv] * 384, *dC = ws.dC + io * 128, *dFC = ws.dFC + io * 384, *dF = ws.dF + io * 384, *dFs = ws.dFs + io * 128;
+        k_inner_bwd<<<(unsigned)M, 128, 0, st>>>(ws.iou + io * 384, list, ws.xcl, W_iou, b_iou, ws.c, ws.dh, ws.dc, dG, dC);
+        g_launches++;
+        lin.dx(dG, 384, 384, U_iou, 384, 384, ws.dh, mr, T_H, nullptr, 0, 0, nullptr, 0, M);            // children's h via U_iou (first write)
+        lin.dx(dC, 128, 128, W_c, 384, 384, dFC, nullptr, 384, nullptr, 0, 0, nullptr, 0, M);           // d(f * c_child)
+        k_forget_bwd<<<(unsigned)M, 384, 0, st>>>(ws.fraw + io * 384, list, cr, ws.xcl, W_f, b_f, ws.c, dFC, ws.dc, dF, dFs);
+        g_launches++;
+        lin.dx(dF, 128, 128, U_f, 128, 128, ws.dh, cr, T_H, nullptr, 0, 1, nullptr, 0, 3 * M);          // children's h via U_f (added)
+    }
+    if (n_leaf > 0) {
+        k_inner_bwd<<<(unsigned)n_leaf, 128, 0, st>>>(nullptr, ws.lists, ws.xcl, W_iou, b_iou, ws.c, ws.dh, ws.dc, ws.dG, nullptr);
+        g_launches++;
+    }
+    f32.dw(ws.dG, 384, 384, ws.xcl, ws.lists, NF, NF, nullptr, 0, 0, n_leaf + n_in, gr[0], gr[1]);                 // W_iou, b_iou
+    lin.dw(ws.dG + n_leaf * 384, 384, 384, ws.h, ws.merge_row, T_H, 3 * T_H, nullptr, 0, 0, n_in, gr[2], nullptr); // U_iou
+    lin.dw(ws.dC, 128, 128, ws.fc, nullptr, 384, 384, nullptr, 0, 0, n_in, gr[3], gr[4]);                          // W_c, b_c
+    f32.dw(ws.dFs, 128, 128, ws.xcl, ws.lists + n_leaf, NF, NF, nullptr, 0, 0, n_in, gr[5], gr[6]);                // W_f, b_f
+    lin.dw(ws.dF, 128, 128, ws.h, ws.child_row, T_H, T_H, nullptr, 0, 0, 3 * n_in, gr[7], nullptr);                // U_f
+    return (int)cudaGetLastError();
+}
+
+// the argument checks of fl_policy_ppo_grad_f32 (FL_ERR_BAD_ARG before any CUDA call)
+int check_args(const float *const *wts, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N, const PpoIn &in,
+               const FlPpoParams *params, Wg &ws) {
+    if (!wts || !in.grads || !params || !d_workspace || E <= 0 || N <= 0 || !in.agent_attr || !in.forest || !in.adjacency || !in.node_order ||
+        !in.valid || !in.actions || !in.old_lp || !in.adv || !in.ret || !in.acted || !in.logits || !in.value || !in.stats)
+        return -1;
+    if (N > (1ll << 31) / f32path::NODES || E > ((1ll << 31) / f32path::NODES) / N) return -1;      // node ids are 32-bit
+    if (!(params->clip_eps > 0.0f)) return -1;
+    for (int i = 0; i < FL_POLICY_F32_TENSORS; i++)
+        if (!wts[i] || !in.grads[i]) return -1;
+    if (carve(ws, (unsigned char *)d_workspace, E * N) > workspace_bytes) return -1;
+    return 0;
+}
+
+}  // namespace ppograph
 
 extern "C" {
 
@@ -1519,204 +1823,76 @@ int fl_policy_ppo_grad_f32(const float *const *wts, void *d_workspace, size_t wo
                            const float *d_old_log_probs, const float *d_advantages, const float *d_returns, const uint8_t *d_acted,
                            const FlPpoParams *params, float *const *d_grads, float *d_logits, float *d_value, float *d_stats,
                            void *stream) {
-    using namespace f32path;
-    using namespace f32grad;
-    if (!wts || !d_grads || !params || !d_workspace || E <= 0 || N <= 0 || !d_agent_attr || !d_forest || !d_adjacency || !d_node_order ||
-        !d_valid_actions || !d_actions || !d_old_log_probs || !d_advantages || !d_returns || !d_acted || !d_logits || !d_value || !d_stats)
-        return -1;
-    if (N > (1ll << 31) / f32path::NODES || E > ((1ll << 31) / f32path::NODES) / N) return -1;      // node ids are 32-bit
-    if (!(params->clip_eps > 0.0f)) return -1;
+    const ppograph::PpoIn in{d_agent_attr, d_forest, d_adjacency, d_node_order, d_valid_actions, d_actions, d_old_log_probs, d_advantages,
+                             d_returns, d_acted, params ? params->clip_eps : 0.0f, params ? params->vf_coef : 0.0f,
+                             params ? params->ent_coef : 0.0f, d_grads, d_logits, d_value, d_stats};
+    f32grad::Wg ws;
+    if (ppograph::check_args(wts, d_workspace, workspace_bytes, E, N, in, params, ws)) return -1;
+    ppograph::F32Lin lin{(cudaStream_t)stream, ws.part};
+    return ppograph::run(lin, wts, ws, E, N, in, true, (cudaStream_t)stream);
+}
+
+// ---- the same loss and gradients with the dense products on the tensor cores (policy_bf16_grad.cuh) --------------------
+size_t fl_policy_workspace_bytes_grad_bf16(int64_t n_agents_total) { return fl_policy_workspace_bytes_grad_f32(n_agents_total); }
+
+int fl_policy_ppo_grad_bf16(const float *const *wts, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
+                            const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
+                            const int32_t *d_node_order, const uint8_t *d_valid_actions, const uint8_t *d_actions,
+                            const float *d_old_log_probs, const float *d_advantages, const float *d_returns, const uint8_t *d_acted,
+                            const FlPpoParams *params, float *const *d_grads, float *d_logits, float *d_value, float *d_stats,
+                            void *stream) {
+    const ppograph::PpoIn in{d_agent_attr, d_forest, d_adjacency, d_node_order, d_valid_actions, d_actions, d_old_log_probs, d_advantages,
+                             d_returns, d_acted, params ? params->clip_eps : 0.0f, params ? params->vf_coef : 0.0f,
+                             params ? params->ent_coef : 0.0f, d_grads, d_logits, d_value, d_stats};
+    f32grad::Wg ws;
+    if (ppograph::check_args(wts, d_workspace, workspace_bytes, E, N, in, params, ws)) return -1;
+    const int rc = ppograph::bf16_setup();
+    if (rc) return rc;
+    ppograph::Bf16Lin lin{(cudaStream_t)stream, ws.part};
+    return ppograph::run(lin, wts, ws, E, N, in, true, (cudaStream_t)stream);
+}
+
+int fl_policy_forward_train_bf16(const float *const *wts, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
+                                 const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
+                                 const int32_t *d_node_order, float *d_logits, float *d_value, void *stream) {
+    if (!wts || !d_workspace || E <= 0 || N <= 0 || !d_agent_attr || !d_forest || !d_adjacency || !d_node_order || !d_logits || !d_value) return -1;
+    if (N > (1ll << 31) / f32path::NODES || E > ((1ll << 31) / f32path::NODES) / N) return -1;
     for (int i = 0; i < FL_POLICY_F32_TENSORS; i++)
-        if (!wts[i] || !d_grads[i]) return -1;
-    const long long T = E * N;
-    Wg ws;
-    if (carve(ws, (unsigned char *)d_workspace, T) > workspace_bytes) return -1;
-    cudaStream_t st = (cudaStream_t)stream;
-    const float eps = params->clip_eps, vf = params->vf_coef, ent = params->ent_coef;
-    auto gemm = [&](const float *a1, const int32_t *idx1, long long lda1, int K1, const float *a2, long long lda2, int K2,
-                    const float *w, const float *bias, float *c, long long ldc, long long M, int Nn, int act, float *pre) {
-        if (M <= 0) return;
-        GemmArgs g{a1, idx1, lda1, K1, a2, lda2, K2, w, bias, c, ldc, M, nullptr, Nn, act, pre};
-        k_gemm_f32<<<dim3((unsigned)((M + 63) / 64), (unsigned)((Nn + 63) / 64)), 256, 0, st>>>(g);
-        g_launches++;
-    };
-    // dX = dY W with the epilogue of k_gemm_dx
-    auto dx = [&](const float *a, long long lda, int Nn, const float *w, long long ldw, int K, float *c, const int32_t *cidx, long long ldc,
-                  const float *add, long long ldadd, int accum, const float *pre, long long ldpre, long long M) {
-        if (M <= 0) return;
-        DxArgs g{a, lda, Nn, w, ldw, K, c, cidx, ldc, add, ldadd, accum, pre, ldpre, M};
-        k_gemm_dx<<<dim3((unsigned)((M + 63) / 64), (unsigned)((K + 63) / 64)), 256, 0, st>>>(g);
-        g_launches++;
-    };
-    // dW = dY^T X (and db when db != null) over M rows, fixed chunks, then summed in chunk order
-    auto dw = [&](const float *dy, long long ldy, int Nn, const float *x1, const int32_t *idx1, long long ldx1, int K1, const float *x2,
-                  long long ldx2, int K2, long long M, float *dW, float *db) {
-        const int bias = db ? 1 : 0, Kp = K1 + K2 + bias;
-        int nch = n_chunks(M);
-        long long chunk = 0;
-        if (nch > 0) {
-            chunk = ((M + nch - 1) / nch + 15) & ~15LL;
-            nch = (int)((M + chunk - 1) / chunk);
-            DwArgs g{dy, ldy, Nn, x1, idx1, ldx1, K1, x2, ldx2, K2, bias, M, chunk, ws.part};
-            k_gemm_dw<<<dim3((unsigned)((Nn + 63) / 64), (unsigned)((Kp + 63) / 64), (unsigned)nch), 256, 0, st>>>(g);
-            g_launches++;
-        }
-        k_dw_reduce<<<(unsigned)(((long long)Nn * Kp + 255) / 256), 256, 0, st>>>(ws.part, nch, Nn, K1 + K2, bias, dW, db);
-        g_launches++;
-    };
-    auto copy_cols = [&](const float *src, long long lds, float *dst, long long ldd, long long rows, int cols) {
-        k_copy_cols<<<(unsigned)((rows * cols + 255) / 256), 256, 0, st>>>(src, lds, dst, ldd, rows, cols);
-        g_launches++;
-    };
-    auto gelu_bwd = [&](const float *src, long long lds, const float *pre, long long ldp, float *dst, long long ldd, long long rows, int cols) {
-        k_gelu_bwd<<<(unsigned)((rows * cols + 255) / 256), 256, 0, st>>>(src, lds, pre, ldp, dst, ldd, rows, cols);
-        g_launches++;
-    };
-    const float *W_iou = wts[0], *b_iou = wts[1], *U_iou = wts[2], *W_c = wts[3], *b_c = wts[4], *W_f = wts[5], *b_f = wts[6], *U_f = wts[7];
-    float *const *gr = d_grads;
+        if (!wts[i]) return -1;
+    f32grad::Wg ws;
+    if (f32grad::carve(ws, (unsigned char *)d_workspace, E * N) > workspace_bytes) return -1;
+    const int rc = ppograph::bf16_setup();
+    if (rc) return rc;
+    const ppograph::PpoIn in{d_agent_attr, d_forest, d_adjacency, d_node_order, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+                             0.0f, 0.0f, 0.0f, nullptr, d_logits, d_value, nullptr};
+    ppograph::Bf16Lin lin{(cudaStream_t)stream, ws.part};
+    return ppograph::run(lin, wts, ws, E, N, in, false, (cudaStream_t)stream);
+}
 
-    // ==== training forward: fl_policy_forward_f32's arithmetic, every level and layer in its own slice ====
-    const long long nodes = T * f32path::NODES;
-    cudaError_t err = cudaMemsetAsync(ws.h, 0, (size_t)nodes * T_H * 4, st);
-    if (err == cudaSuccess) err = cudaMemsetAsync(ws.c, 0, (size_t)nodes * T_H * 4, st);
-    if (err == cudaSuccess) err = cudaMemsetAsync(ws.counts, 0, 64 * 4, st);
-    if (err != cudaSuccess) return (int)err;
-    k_clean<<<(unsigned)((nodes * NF + 255) / 256), 256, 0, st>>>(d_forest, ws.xcl, nodes * NF);
-    k_tl_count<<<(unsigned)((T + 127) / 128), 128, 0, st>>>(d_adjacency, d_node_order, T, ws.child_base, ws.tcnt);
-    k_tl_scan<<<dim3((unsigned)ws.nblk, MAX_LEVELS), SCAN, 0, st>>>(ws.tcnt, T, ws.nblk, ws.tpos, ws.btot);
-    k_tl_tops<<<1, 32, 0, st>>>(ws.btot, ws.nblk, ws.counts);
-    k_tl_fill<<<(unsigned)((T + 127) / 128), 128, 0, st>>>(d_node_order, T, ws.nblk, ws.tpos, ws.btot, ws.counts, ws.lists);
-    k_tree_leaves<<<(unsigned)nodes, 128, 0, st>>>(d_forest, d_node_order, nodes, W_iou, b_iou, ws.h, ws.c);
-    g_launches += 6;
-    int32_t counts[MAX_LEVELS];
-    err = cudaMemcpyAsync(counts, ws.counts, sizeof(counts), cudaMemcpyDeviceToHost, st);
-    if (err == cudaSuccess) err = cudaStreamSynchronize(st);        // per-level sizes of the launches below; the only host sync
-    if (err != cudaSuccess) return (int)err;
-    long long loff[MAX_LEVELS + 1];                                  // list offset of every level (leaves first)
-    loff[0] = 0;
-    for (int lv = 0; lv < MAX_LEVELS; lv++) loff[lv + 1] = loff[lv] + counts[lv];
-    const long long n_leaf = counts[0], n_in = loff[MAX_LEVELS] - n_leaf;   // inner index i = list position - n_leaf
-    if (n_in > ws.cap) return -1;
-    for (int lv = 1; lv < MAX_LEVELS; lv++) {
-        const long long M = counts[lv], io = loff[lv] - n_leaf;
-        if (M <= 0) continue;
-        const int32_t *list = ws.lists + loff[lv], *dM = ws.counts + lv;
-        int32_t *mr = ws.merge_row + io, *cr = ws.child_row + 3 * io;
-        float *iou = ws.iou + io * 384, *fraw = ws.fraw + io * 384, *fc = ws.fc + io * 384;
-        k_level_rows<<<(unsigned)((M + 127) / 128), 128, 0, st>>>(list, dM, ws.child_base, mr, cr);
-        g_launches++;
-        gemm(ws.h, mr, T_H, 3 * T_H, nullptr, 0, 0, U_iou, nullptr, iou, 3 * T_H, M, 3 * T_H, 0, nullptr);
-        gemm(ws.h, cr, T_H, T_H, nullptr, 0, 0, U_f, nullptr, fraw, T_H, 3 * M, T_H, 0, nullptr);
-        k_forget<<<(unsigned)M, 384, 0, st>>>(fraw, list, cr, dM, d_forest, W_f, b_f, ws.c, fc);
-        gemm(fc, nullptr, 3 * T_H, 3 * T_H, nullptr, 0, 0, W_c, nullptr, ws.craw, T_H, M, T_H, 0, nullptr);
-        k_inner<<<(unsigned)M, 128, 0, st>>>(iou, ws.craw, list, dM, d_forest, W_iou, b_iou, b_c, ws.h, ws.c);
-        g_launches += 2;
+int fl_policy_tc_product_bf16(const FlTcProduct *p, void *d_workspace, size_t workspace_bytes, void *stream) {
+    if (!p || p->M < 0 || p->N <= 0 || p->K <= 0 || !p->c) return -1;
+    const bool xok = p->x1 && p->K1 >= 0 && p->K2 >= 0 && p->K1 + p->K2 == p->K && (!p->K2 || p->x2);
+    if (p->kind == FL_TC_FORWARD) {
+        if (!xok || !p->w) return -1;
+    } else if (p->kind == FL_TC_DX) {
+        if (!p->dy || !p->w || p->ldw < p->K) return -1;
+    } else if (p->kind == FL_TC_DW) {
+        if (!p->dy || !xok || !d_workspace) return -1;
+        int nch = 0;
+        bf16grad::dw_chunk(p->M, &nch);
+        if ((size_t)nch * p->N * (p->K + 1) * 4 > workspace_bytes) return -1;
+    } else {
+        return -1;
     }
-    gemm(d_agent_attr, nullptr, 83, 83, nullptr, 0, 0, wts[8], wts[9], ws.aa[0], 256, T, 256, 1, ws.ap[0]);
-    gemm(ws.aa[0], nullptr, 256, 256, nullptr, 0, 0, wts[10], wts[11], ws.aa[1], 256, T, 256, 1, ws.ap[1]);
-    gemm(ws.aa[1], nullptr, 256, 256, nullptr, 0, 0, wts[12], wts[13], ws.aa[2], 256, T, 256, 1, ws.ap[2]);
-    gemm(ws.aa[2], nullptr, 256, 256, nullptr, 0, 0, wts[14], wts[15], ws.emb, 256, T, 128, 1, ws.ap[3]);
-    copy_cols(ws.h, (long long)f32path::NODES * T_H, ws.emb + 128, 256, T, 128);
-    const float *x = ws.emb;
-    for (int l = 0; l < 3; l++) {
-        const float *const *tw = wts + 16 + 6 * l;
-        gemm(x, nullptr, 256, 256, nullptr, 0, 0, tw[0], tw[1], ws.qkv[l], 768, T, 768, 0, nullptr);
-        k_attention<<<(unsigned)((T * 4 * 32 + 255) / 256), 256, 0, st>>>(ws.qkv[l], ws.att[l], 256, E, (int)N, ws.lse[l]);
-        g_launches++;
-        gemm(ws.att[l], nullptr, 256, 256, nullptr, 0, 0, tw[2], tw[3], ws.cat[l] + 256, 512, T, 256, 0, nullptr);
-        copy_cols(x, 256, ws.cat[l], 512, T, 256);
-        gemm(ws.cat[l], nullptr, 512, 512, nullptr, 0, 0, tw[4], tw[5], ws.xs[l], 256, T, 256, 1, ws.mpre[l]);
-        x = ws.xs[l];
-    }
-    const float *const *aw = wts + 34, *const *cw = wts + 40;
-    for (int hd = 0; hd < 2; hd++) {
-        const float *const *hw = hd ? cw : aw;
-        gemm(ws.emb, nullptr, 256, 256, x, 256, 256, hw[0], hw[1], ws.y1[hd], 256, T, 256, 1, ws.y1p[hd]);
-        gemm(ws.y1[hd], nullptr, 256, 256, nullptr, 0, 0, hw[2], hw[3], ws.y2[hd], 128, T, 128, 1, ws.y2p[hd]);
-    }
-    k_heads_final<<<(unsigned)E, 256, (size_t)N * sizeof(float), st>>>(ws.y2[0], ws.y2[1], aw[4], aw[5], cw[4], cw[5], d_logits, d_value, (int)N);
-    g_launches++;
-
-    // ==== PPO loss: d loss / d logits, d loss / d critic output, statistics ====
-    PpoArgs pa{d_logits, d_value, d_old_log_probs, d_advantages, d_returns, d_valid_actions, d_actions, d_acted, E, (int)N, eps, vf, ent,
-               ws.counts + 32, ws.dlogits, ws.dcrit, ws.rowstats};
-    k_ppo_count<<<(unsigned)E, 128, 0, st>>>(pa);
-    k_ppo_loss<<<(unsigned)E, 128, 0, st>>>(pa);
-    k_ppo_stats<<<1, 256, 0, st>>>(ws.rowstats, E, ws.counts + 32, vf, ent, d_stats);
-    g_launches += 3;
-
-    // ==== backward: heads (net_tree.py:56-71, 100-110) ====
-    dx(ws.dlogits, 5, 5, aw[4], 128, 128, ws.dy2, nullptr, 128, nullptr, 0, 0, ws.y2p[0], 128, T);
-    dw(ws.dlogits, 5, 5, ws.y2[0], nullptr, 128, 128, nullptr, 0, 0, T, gr[38], gr[39]);
-    dx(ws.dy2, 128, 128, aw[2], 256, 256, ws.dy1, nullptr, 256, nullptr, 0, 0, ws.y1p[0], 256, T);
-    dw(ws.dy2, 128, 128, ws.y1[0], nullptr, 256, 256, nullptr, 0, 0, T, gr[36], gr[37]);
-    dx(ws.dy1, 256, 256, aw[0], 512, 512, ws.dz, nullptr, 512, nullptr, 0, 0, nullptr, 0, T);
-    dw(ws.dy1, 256, 256, ws.emb, nullptr, 256, 256, x, 256, 256, T, gr[34], gr[35]);
-    dx(ws.dcrit, 1, 1, cw[4], 128, 128, ws.dy2, nullptr, 128, nullptr, 0, 0, ws.y2p[1], 128, T);
-    dw(ws.dcrit, 1, 1, ws.y2[1], nullptr, 128, 128, nullptr, 0, 0, T, gr[44], gr[45]);
-    dx(ws.dy2, 128, 128, cw[2], 256, 256, ws.dy1, nullptr, 256, nullptr, 0, 0, ws.y1p[1], 256, T);
-    dw(ws.dy2, 128, 128, ws.y1[1], nullptr, 256, 256, nullptr, 0, 0, T, gr[42], gr[43]);
-    dx(ws.dy1, 256, 256, cw[0], 512, 512, ws.dz, nullptr, 512, nullptr, 0, 1, nullptr, 0, T);      // dz = d cat(emb, att)
-    dw(ws.dy1, 256, 256, ws.emb, nullptr, 256, 256, x, 256, 256, T, gr[40], gr[41]);
-    // ==== three attention blocks (net_tree.py:20-32), last to first ====
-    int cur = 0;
-    gelu_bwd(ws.dz + 256, 512, ws.mpre[2], 256, ws.dx[cur], 256, T, 256);
-    for (int l = 2; l >= 0; l--) {
-        const float *const *tw = wts + 16 + 6 * l;
-        float *const *tg = gr + 16 + 6 * l;
-        const float *xin = l ? ws.xs[l - 1] : ws.emb;
-        const float *dpm = ws.dx[cur];
-        dw(dpm, 256, 256, ws.cat[l], nullptr, 512, 512, nullptr, 0, 0, T, tg[4], tg[5]);                  // att_mlp.0
-        dx(dpm, 256, 256, tw[4], 512, 512, ws.dcat, nullptr, 512, nullptr, 0, 0, nullptr, 0, T);
-        dw(ws.dcat + 256, 512, 256, ws.att[l], nullptr, 256, 256, nullptr, 0, 0, T, tg[2], tg[3]);         // out_proj
-        dx(ws.dcat + 256, 512, 256, tw[2], 256, 256, ws.datt, nullptr, 256, nullptr, 0, 0, nullptr, 0, T);
-        k_attn_bwd_q<<<(unsigned)((T * 4 * 32 + 255) / 256), 256, 0, st>>>(ws.qkv[l], ws.att[l], ws.datt, ws.lse[l], ws.dqkv, ws.Dq, E, (int)N);
-        k_attn_bwd_kv<<<(unsigned)((T * 4 * 32 + 255) / 256), 256, 0, st>>>(ws.qkv[l], ws.datt, ws.lse[l], ws.Dq, ws.dqkv, E, (int)N);
-        g_launches += 2;
-        dw(ws.dqkv, 768, 768, xin, nullptr, 256, 256, nullptr, 0, 0, T, tg[0], tg[1]);                      // in_proj
-        if (l > 0) {   // d(block input) = d cat[:, :256] + dqkv W_in, through the previous block's GELU
-            dx(ws.dqkv, 768, 768, tw[0], 256, 256, ws.dx[cur ^ 1], nullptr, 256, ws.dcat, 512, 0, ws.mpre[l - 1], 256, T);
-            cur ^= 1;
-        } else {       // d emb = dz[:, :256] (heads) + d cat[:, :256] + dqkv W_in, into dz[:, :256]
-            dx(ws.dqkv, 768, 768, tw[0], 256, 256, ws.dz, nullptr, 512, ws.dcat, 512, 1, nullptr, 0, T);
-        }
-    }
-    // ==== attribute MLP (net_tree.py:41-50) on d emb[:, :128] ====
-    gelu_bwd(ws.dz, 512, ws.ap[3], 256, ws.dx[0], 256, T, 128);
-    dw(ws.dx[0], 256, 128, ws.aa[2], nullptr, 256, 256, nullptr, 0, 0, T, gr[14], gr[15]);
-    dx(ws.dx[0], 256, 128, wts[14], 256, 256, ws.dx[1], nullptr, 256, nullptr, 0, 0, ws.ap[2], 256, T);
-    dw(ws.dx[1], 256, 256, ws.aa[1], nullptr, 256, 256, nullptr, 0, 0, T, gr[12], gr[13]);
-    dx(ws.dx[1], 256, 256, wts[12], 256, 256, ws.dx[0], nullptr, 256, nullptr, 0, 0, ws.ap[1], 256, T);
-    dw(ws.dx[0], 256, 256, ws.aa[0], nullptr, 256, 256, nullptr, 0, 0, T, gr[10], gr[11]);
-    dx(ws.dx[0], 256, 256, wts[10], 256, 256, ws.dx[1], nullptr, 256, nullptr, 0, 0, ws.ap[0], 256, T);
-    dw(ws.dx[1], 256, 256, d_agent_attr, nullptr, 83, 83, nullptr, 0, 0, T, gr[8], gr[9]);
-    // ==== Tree-LSTM (TreeLSTM.py:59-154), deepest level first; d h of the roots = d emb[:, 128:] ====
-    err = cudaMemsetAsync(ws.dh, 0, (size_t)nodes * T_H * 4, st);
-    if (err == cudaSuccess) err = cudaMemsetAsync(ws.dc, 0, (size_t)nodes * T_H * 4, st);
-    if (err != cudaSuccess) return (int)err;
-    copy_cols(ws.dz + 128, 512, ws.dh, (long long)f32path::NODES * T_H, T, 128);
-    for (int lv = MAX_LEVELS - 1; lv >= 1; lv--) {
-        const long long M = counts[lv], io = loff[lv] - n_leaf;
-        if (M <= 0) continue;
-        const int32_t *list = ws.lists + loff[lv], *mr = ws.merge_row + io, *cr = ws.child_row + 3 * io;
-        float *dG = ws.dG + loff[lv] * 384, *dC = ws.dC + io * 128, *dFC = ws.dFC + io * 384, *dF = ws.dF + io * 384, *dFs = ws.dFs + io * 128;
-        k_inner_bwd<<<(unsigned)M, 128, 0, st>>>(ws.iou + io * 384, list, ws.xcl, W_iou, b_iou, ws.c, ws.dh, ws.dc, dG, dC);
-        g_launches++;
-        dx(dG, 384, 384, U_iou, 384, 384, ws.dh, mr, T_H, nullptr, 0, 0, nullptr, 0, M);            // children's h via U_iou (first write)
-        dx(dC, 128, 128, W_c, 384, 384, dFC, nullptr, 384, nullptr, 0, 0, nullptr, 0, M);           // d(f * c_child)
-        k_forget_bwd<<<(unsigned)M, 384, 0, st>>>(ws.fraw + io * 384, list, cr, ws.xcl, W_f, b_f, ws.c, dFC, ws.dc, dF, dFs);
-        g_launches++;
-        dx(dF, 128, 128, U_f, 128, 128, ws.dh, cr, T_H, nullptr, 0, 1, nullptr, 0, 3 * M);          // children's h via U_f (added)
-    }
-    if (n_leaf > 0) {
-        k_inner_bwd<<<(unsigned)n_leaf, 128, 0, st>>>(nullptr, ws.lists, ws.xcl, W_iou, b_iou, ws.c, ws.dh, ws.dc, ws.dG, nullptr);
-        g_launches++;
-    }
-    dw(ws.dG, 384, 384, ws.xcl, ws.lists, NF, NF, nullptr, 0, 0, n_leaf + n_in, gr[0], gr[1]);                 // W_iou, b_iou
-    dw(ws.dG + n_leaf * 384, 384, 384, ws.h, ws.merge_row, T_H, 3 * T_H, nullptr, 0, 0, n_in, gr[2], nullptr); // U_iou
-    dw(ws.dC, 128, 128, ws.fc, nullptr, 384, 384, nullptr, 0, 0, n_in, gr[3], gr[4]);                          // W_c, b_c
-    dw(ws.dFs, 128, 128, ws.xcl, ws.lists + n_leaf, NF, NF, nullptr, 0, 0, n_in, gr[5], gr[6]);                // W_f, b_f
-    dw(ws.dF, 128, 128, ws.h, ws.child_row, T_H, T_H, nullptr, 0, 0, 3 * n_in, gr[7], nullptr);                // U_f
+    const int rc = ppograph::bf16_setup();
+    if (rc) return rc;
+    ppograph::Bf16Lin lin{(cudaStream_t)stream, (float *)d_workspace};
+    if (p->kind == FL_TC_FORWARD)
+        lin.gemm(p->x1, p->idx, p->ldx1, p->K1, p->x2, p->ldx2, p->K2, p->w, p->bias, p->c, p->ldc, p->M, p->N, p->act, p->pre);
+    else if (p->kind == FL_TC_DX)
+        lin.dx(p->dy, p->lddy, p->N, p->w, p->ldw, p->K, p->c, p->cidx, p->ldc, p->add, p->ldadd, p->accum, p->gpre, p->ldgpre, p->M);
+    else
+        lin.dw(p->dy, p->lddy, p->N, p->x1, p->idx, p->ldx1, p->K1, p->x2, p->ldx2, p->K2, p->M, p->c, p->db);
     return (int)cudaGetLastError();
 }
 

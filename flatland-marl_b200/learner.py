@@ -4,6 +4,10 @@ Holds the fp32 master parameters of the reference `Network` (solution/nn/net_tre
 their `.grad` with fl_policy_ppo_grad_f32 (include/flatland_policy_b200.h): a training forward in the fp32 path's arithmetic,
 the clipped-surrogate PPO loss and a deterministic backward pass, all CUDA kernels of the library.  The optimiser is the
 caller's: `torch.optim` and `torch.nn.utils.clip_grad_norm_` work on `parameters()` as on any module.
+
+precision="bf16" computes the same loss through the same graph with the dense products of the 20 large weight matrices on
+the tensor cores (fl_policy_ppo_grad_bf16: bf16 operands, fp32 accumulation, fp32 master weights and gradients); see
+DESIGN.md §4.8 for what the two learners trade.
 """
 import ctypes as C
 from collections import OrderedDict
@@ -33,10 +37,13 @@ class PolicyLearner:
         rollout.actor = learner.actor()                    # acting with the new parameters
     """
 
-    def __init__(self, weights=None, device="cuda:0", seed=0):
+    def __init__(self, weights=None, device="cuda:0", seed=0, precision="fp32"):
+        if precision not in ("fp32", "bf16"):
+            raise ValueError("precision must be 'fp32' or 'bf16'")
         if not torch.cuda.is_available():
             raise FlatlandB200Error("PolicyLearner needs a CUDA device (no CPU fallback on the policy path)")
         self.lib = lib()
+        self.precision = precision
         self.device = torch.device(device)
         torch.cuda.set_device(self.device)
         w = pw.check_weights(weights_dict(weights, seed))
@@ -96,16 +103,20 @@ class PolicyLearner:
         return self._out
 
     def forward(self, obs):
-        """Logits [E,N,5] and values [E] of the current parameters: fl_policy_forward_f32, whose bytes are those of the
-        training forward inside ppo_grad.  Device tensors, valid until the next call."""
+        """Logits [E,N,5] and values [E] of the current parameters: fl_policy_forward_f32 (fl_policy_forward_train_bf16 for
+        precision="bf16"), whose bytes are those of the training forward inside ppo_grad.  Device tensors, valid until the next
+        call."""
         E, N = self._check_obs(obs, OBS_KEYS)
-        need = int(self.lib.fl_policy_workspace_bytes_f32(E * N))
+        bf16 = self.precision == "bf16"
+        need = int(self.lib.fl_policy_workspace_bytes_grad_bf16(E * N) if bf16 else self.lib.fl_policy_workspace_bytes_f32(E * N))
         if self._ws is None or self._ws.numel() < need:
+            self._ws = None
             self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
         logits, value = self._outputs(E, N)
-        _check(self.lib.fl_policy_forward_f32(self._weights(), self._ws.data_ptr(), self._ws.numel(), E, N,
-                                              *(obs[k].data_ptr() for k, _, _ in OBS_KEYS), logits.data_ptr(), value.data_ptr(),
-                                              self._stream()), "fl_policy_forward_f32")
+        fn, name = (self.lib.fl_policy_forward_train_bf16, "fl_policy_forward_train_bf16") if bf16 else \
+            (self.lib.fl_policy_forward_f32, "fl_policy_forward_f32")
+        _check(fn(self._weights(), self._ws.data_ptr(), self._ws.numel(), E, N, *(obs[k].data_ptr() for k, _, _ in OBS_KEYS),
+                  logits.data_ptr(), value.data_ptr(), self._stream()), name)
         return logits, value
 
     def ppo_grad(self, mb, clip_eps=0.2, vf_coef=0.5, ent_coef=0.01):
@@ -115,7 +126,7 @@ class PolicyLearner:
 
         Returns the statistics as a float32 [8] device tensor (policy loss, value loss, entropy, approximate KL, clip
         fraction, |S|, acted rows, total loss), reused by the next call.  The one host synchronisation is the fp32 path's
-        (per-level node counts)."""
+        (per-level node counts), in both precisions."""
         E, N = self._check_obs(mb, MB_KEYS)
         for name, dt in ROW_KEYS:
             t = mb[name]
@@ -123,7 +134,8 @@ class PolicyLearner:
                 raise ValueError("%s must be a contiguous %s tensor of shape (%d,) on %s" % (name, dt, E, self.device))
         if not clip_eps > 0:
             raise ValueError("clip_eps must be positive")
-        need = int(self.lib.fl_policy_workspace_bytes_grad_f32(E * N))
+        bf16 = self.precision == "bf16"
+        need = int(self.lib.fl_policy_workspace_bytes_grad_bf16(E * N) if bf16 else self.lib.fl_policy_workspace_bytes_grad_f32(E * N))
         if self._ws is None or self._ws.numel() < need:
             self._ws = None
             self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
@@ -135,10 +147,12 @@ class PolicyLearner:
             grads.append(p.grad)
         logits, value = self._outputs(E, N)
         params = FlPpoParams(float(clip_eps), float(vf_coef), float(ent_coef))
-        _check(self.lib.fl_policy_ppo_grad_f32(self._weights(), self._ws.data_ptr(), self._ws.numel(), E, N,
-                                               *(mb[k].data_ptr() for k, _, _ in MB_KEYS), *(mb[k].data_ptr() for k, _ in ROW_KEYS),
-                                               C.byref(params), self._ptrs(grads), logits.data_ptr(), value.data_ptr(),
-                                               self._stats.data_ptr(), self._stream()), "fl_policy_ppo_grad_f32")
+        fn, name = (self.lib.fl_policy_ppo_grad_bf16, "fl_policy_ppo_grad_bf16") if bf16 else \
+            (self.lib.fl_policy_ppo_grad_f32, "fl_policy_ppo_grad_f32")
+        _check(fn(self._weights(), self._ws.data_ptr(), self._ws.numel(), E, N,
+                  *(mb[k].data_ptr() for k, _, _ in MB_KEYS), *(mb[k].data_ptr() for k, _ in ROW_KEYS),
+                  C.byref(params), self._ptrs(grads), logits.data_ptr(), value.data_ptr(),
+                  self._stats.data_ptr(), self._stream()), name)
         return self._stats
 
     def last_outputs(self):

@@ -19,7 +19,8 @@ LIB_PATH = os.path.join(HERE, "csrc", "policy", "libflatland_policy_b200.so")
 LAYERS = pw.N_TRANSFORMER
 
 EXPORTS = ["fl_policy_abi_version", "fl_policy_workspace_bytes", "fl_policy_forward", "fl_policy_workspace_bytes_f32",
-           "fl_policy_forward_f32", "fl_policy_workspace_bytes_grad_f32", "fl_policy_ppo_grad_f32", "fl_policy_choose_actions",
+           "fl_policy_forward_f32", "fl_policy_workspace_bytes_grad_f32", "fl_policy_ppo_grad_f32", "fl_policy_workspace_bytes_grad_bf16",
+           "fl_policy_ppo_grad_bf16", "fl_policy_forward_train_bf16", "fl_policy_tc_product_bf16", "fl_policy_choose_actions",
            "fl_policy_sample_actions", "fl_policy_gae",
            "fl_policy_linear", "fl_policy_linear_debug", "fl_policy_debug_clocks", "fl_policy_launch_count"]
 
@@ -36,6 +37,20 @@ class FlPolicyWeights(C.Structure):
 class FlPpoParams(C.Structure):
     """Mirror of `struct FlPpoParams` (include/flatland_policy_b200.h)."""
     _fields_ = [("clip_eps", C.c_float), ("vf_coef", C.c_float), ("ent_coef", C.c_float)]
+
+
+class FlTcProduct(C.Structure):
+    """Mirror of `struct FlTcProduct` (include/flatland_policy_b200.h): one tensor-core product of the bf16 learner."""
+    _fields_ = [("kind", C.c_int32), ("M", C.c_int64), ("N", C.c_int32), ("K", C.c_int32),
+                ("x1", C.c_void_p), ("idx", C.c_void_p), ("ldx1", C.c_int64), ("K1", C.c_int32),
+                ("x2", C.c_void_p), ("ldx2", C.c_int64), ("K2", C.c_int32),
+                ("dy", C.c_void_p), ("lddy", C.c_int64),
+                ("w", C.c_void_p), ("ldw", C.c_int64), ("bias", C.c_void_p),
+                ("c", C.c_void_p), ("cidx", C.c_void_p), ("ldc", C.c_int64),
+                ("add", C.c_void_p), ("ldadd", C.c_int64), ("accum", C.c_int32),
+                ("pre", C.c_void_p), ("act", C.c_int32),
+                ("gpre", C.c_void_p), ("ldgpre", C.c_int64),
+                ("db", C.c_void_p)]
 
 
 _lib = None
@@ -64,6 +79,14 @@ def lib():
     L.fl_policy_workspace_bytes_grad_f32.argtypes = [C.c_int64]
     L.fl_policy_ppo_grad_f32.restype = C.c_int
     L.fl_policy_ppo_grad_f32.argtypes = [P, P, C.c_size_t, C.c_int64, C.c_int64] + [P] * 10 + [C.POINTER(FlPpoParams), P, P, P, P, P]
+    L.fl_policy_workspace_bytes_grad_bf16.restype = C.c_size_t
+    L.fl_policy_workspace_bytes_grad_bf16.argtypes = [C.c_int64]
+    L.fl_policy_ppo_grad_bf16.restype = C.c_int
+    L.fl_policy_ppo_grad_bf16.argtypes = [P, P, C.c_size_t, C.c_int64, C.c_int64] + [P] * 10 + [C.POINTER(FlPpoParams), P, P, P, P, P]
+    L.fl_policy_forward_train_bf16.restype = C.c_int
+    L.fl_policy_forward_train_bf16.argtypes = [P, P, C.c_size_t, C.c_int64, C.c_int64, P, P, P, P, P, P, P]
+    L.fl_policy_tc_product_bf16.restype = C.c_int
+    L.fl_policy_tc_product_bf16.argtypes = [C.POINTER(FlTcProduct), P, C.c_size_t, P]
     L.fl_policy_choose_actions.restype = C.c_int
     L.fl_policy_choose_actions.argtypes = [P, P, P, C.c_int64, P]
     L.fl_policy_sample_actions.restype = C.c_int

@@ -129,6 +129,62 @@ int fl_policy_ppo_grad_f32(const float *const *d_weights, void *d_workspace, siz
                            float *const *d_grads,
                            float *d_logits, float *d_value, float *d_stats, void *stream);
 
+/* The same loss, statistics and outputs through the same graph, with the dense products on the tensor cores
+ * (csrc/policy/policy_bf16_grad.cuh).  Arguments, workspace, argument errors, determinism and the one host synchronisation
+ * are those of fl_policy_ppo_grad_f32; the arithmetic differs in one place only:
+ *   - The tensor-core layers: the weights U_iou, U_f, W_c (Tree-LSTM), attr_embedding.{0,2,4,6}, per transformer layer
+ *     in_proj, out_proj and att_mlp.0, actor_net.{0,2} and critic_net.{0,2}.  For each of them the forward X W^T, the input
+ *     gradient dY W and the weight gradient dY^T X run as tcgen05.mma kind::f16: both operands are the fp32 values rounded
+ *     to bf16 (round to nearest even), the products accumulate in fp32.  The bias gradient is the fp32 sum over rows of the
+ *     unrounded dY, over fixed row chunks and then in chunk order.
+ *   - Everything else is the fp32 path's arithmetic in its kernels: the 12-feature node terms W_iou x, W_f x and their weight
+ *     gradients, actor_net.4 and critic_net.4 (forward, dX, dW), attention and its backward, the Tree-LSTM gates, GELU and
+ *     GELU', the loss and the statistics.  Activations and gradients are stored in fp32; the bf16 values exist only as
+ *     operands inside the products.
+ * fl_policy_forward_train_bf16 is the training forward alone (signature of fl_policy_forward_f32, this workspace): its
+ * logits and values are bit-identical to those fl_policy_ppo_grad_bf16 writes for the same weights and observations. */
+size_t fl_policy_workspace_bytes_grad_bf16(int64_t n_agents_total);
+int fl_policy_ppo_grad_bf16(const float *const *d_weights, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
+                            const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
+                            const int32_t *d_node_order, const uint8_t *d_valid_actions,
+                            const uint8_t *d_actions, const float *d_old_log_probs,
+                            const float *d_advantages, const float *d_returns,
+                            const uint8_t *d_acted,
+                            const FlPpoParams *params,
+                            float *const *d_grads,
+                            float *d_logits, float *d_value, float *d_stats, void *stream);
+int fl_policy_forward_train_bf16(const float *const *d_weights, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
+                                 const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
+                                 const int32_t *d_node_order, float *d_logits, float *d_value, void *stream);
+
+/* One tensor-core product of fl_policy_ppo_grad_bf16, exposed for tests.  bf16-rounded operands, fp32 accumulation; every
+ * other term in fp32.  X(m, k) = x1[row(m) ldx1 + k] (k < K1), x2[m ldx2 + k - K1] (K1 <= k < K = K1 + K2); row(m) = idx ?
+ * idx[m] : m.  Row strides in floats.
+ *   FL_TC_FORWARD  c[m][n] (ldc) = act(sum_k X(m, k) w[n][k] + bias[n]), m < M, n < N; w is [N][K]; pre (optional) gets
+ *                  the value before the activation at c's offsets; act 0 none, 1 GELU(erf).
+ *   FL_TC_DX       c[r(m)][k] = (sum_n dy[m][n] w[n][k] + add[m][k] + accum c[r(m)][k]) * gelu'(gpre[m][k]), k < K, n < N;
+ *                  w is [N][ldw]; r(m) = cidx ? cidx[m] : m; add, gpre optional.
+ *   FL_TC_DW       c[n][k] (row stride K) = sum over m < M of dy[m][n] X(m, k), db[n] (optional) = sum of dy[m][n]; over
+ *                  fixed row chunks into d_workspace (at least 512 rows each, at most 128 chunks: 4 nch N (K + 1) bytes).
+ * FL_ERR_BAD_ARG for a NULL operand or inconsistent sizes. */
+#define FL_TC_FORWARD 0
+#define FL_TC_DX 1
+#define FL_TC_DW 2
+typedef struct FlTcProduct {
+    int32_t kind;
+    int64_t M; int32_t N, K;
+    const float *x1; const int32_t *idx; int64_t ldx1; int32_t K1;
+    const float *x2; int64_t ldx2; int32_t K2;
+    const float *dy; int64_t lddy;
+    const float *w; int64_t ldw; const float *bias;
+    float *c; const int32_t *cidx; int64_t ldc;
+    const float *add; int64_t ldadd; int32_t accum;
+    float *pre; int32_t act;
+    const float *gpre; int64_t ldgpre;
+    float *db;
+} FlTcProduct;
+int fl_policy_tc_product_bf16(const FlTcProduct *p, void *d_workspace, size_t workspace_bytes, void *stream);
+
 /* Actor._choose_action in "soft" mode for every agent (plfActor.py:27-44): masked softmax over the valid actions,
  * then numpy's choice with the generator re-seeded to 42, i.e. the first action whose cumulative probability
  * exceeds 0.3745401188473625; no valid action -> 0.  d_valid_actions [n][5] u8, d_actions [n] u8. */

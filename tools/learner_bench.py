@@ -1,16 +1,22 @@
-"""Cost of one PPO minibatch update's loss and gradients on the device (PolicyLearner.ppo_grad, fl_policy_ppo_grad_f32), on a
-B200, against two yardsticks:
+"""Cost of one PPO minibatch update's loss and gradients on the device (PolicyLearner.ppo_grad, fl_policy_ppo_grad_f32 and,
+with --bf16, fl_policy_ppo_grad_bf16: the dense products on the tensor cores), on a B200, against two yardsticks:
   - the fp32 forward alone (fl_policy_forward_f32, what the training forward costs without keeping activations);
   - torch autograd on the GPU over the test suite's torch restatement of the network and loss (tests/policy_grad_oracle.py,
     fp32, TF32 off), forward + loss + backward.  Its tree index lists are built on the host per call, as the restatement does.
-The three are alternated call by call so that they see the same clocks and neighbours; the working sets (GBs of
+All are alternated call by call so that they see the same clocks and neighbours; the working sets (GBs of
 activations) are far larger than the 126 MB L2.
+
+With --bf16 the bf16 learner (same parameters) joins the alternation, and the report adds its workspace, the PPO-ratio
+spread of the bf16 behaviour policy against the bf16 learner, a per-kernel time table of both learners from a separate
+torch.profiler run (two calls each, after the timed ones), and the achieved rate of the tensor-core products: their FLOPs,
+counted from the layer shapes and the minibatch's actual per-level node counts, over the profiled time of k_tc_gemm.
 
 Shapes: Test_03 x 1024 rows (51,200 agents) and a Test_02-shape minibatch of 8192 rows x 20 agents (163,840 agents).  The
 rows come from a Rollout collected with the bf16 actor, so the first pass also measures the spread of the PPO ratio r between
 the bf16 behaviour policy and the fp32 learner.  The card's name and power limit are read in the same run.
 
     python tools/learner_bench.py --out profiles/learner_bench_b200.json [--calls 5]
+    python tools/learner_bench.py --bf16 --out profiles/learner_bench_bf16_b200.json
 """
 import argparse
 import json
@@ -56,7 +62,38 @@ def ratio_spread(mb, logits, eps=0.2):
                 approx_kl=float((-d).mean()), clip_fraction=float(((r - 1).abs() > eps).double().mean()))
 
 
-def run_case(config, E, T, calls):
+def tc_flops(node_order, T):
+    """FLOPs (2 per multiply-add) of the tensor-core products of one fl_policy_ppo_grad_bf16 call: forward, dW for the 20
+    matrices, dX for all but attr_embedding.0 (its input is the observation).  node_order [T][31] (host): inner nodes are
+    those with node_order >= 1; each costs U_iou (384 x 384), U_f (3 x 128 x 128) and W_c (128 x 384) per product."""
+    n_in = int((node_order >= 1).sum())
+    tree = n_in * (384 * 384 + 3 * 128 * 128 + 128 * 384)
+    attr0 = T * 83 * 256
+    rest = T * (256 * 256 * 2 + 256 * 128 + 3 * (256 * 768 + 256 * 256 + 512 * 256) + 2 * (512 * 256 + 256 * 128))
+    fwd = tree + attr0 + rest
+    return 2 * (fwd + fwd + (fwd - attr0)), n_in
+
+
+def kernel_table(fn, calls=2):
+    """{kernel name: mean device ms per call} of fn over `calls` calls, from torch.profiler."""
+    from torch.profiler import ProfilerActivity, profile
+    fn()
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(calls):
+            fn()
+        torch.cuda.synchronize()
+    out = {}
+    for e in prof.key_averages():
+        t = getattr(e, "self_device_time_total", 0) or 0
+        if t <= 0:
+            continue
+        name = e.key.replace("void ", "").split("(")[0]
+        out[name] = out.get(name, 0.0) + t / 1000.0 / calls
+    return dict(sorted(((k, round(v, 4)) for k, v in out.items()), key=lambda kv: -kv[1]))
+
+
+def run_case(config, E, T, calls, with_bf16=False):
     learner = fb.PolicyLearner(None, seed=0)
     batch = fb.BatchedRailEnv(bench.load_worlds(config, E), auto_reset=True)
     batch.reset()
@@ -96,9 +133,17 @@ def run_case(config, E, T, calls):
         torch.cuda.empty_cache()
     learner.ppo_grad(mb)
     learner.forward(fwd)
-    ours, f32, tor = [], [], []
+    lb = None
+    if with_bf16:
+        lb = fb.PolicyLearner(learner.state_dict(), seed=0, precision="bf16")
+        lb.ppo_grad(mb)
+        spread_bf16 = ratio_spread(mb, lb.last_outputs()[0])
+        stats_bf16 = lb.ppo_grad(mb).cpu().numpy()
+    ours, f32, tor, bf = [], [], [], []
     for _ in range(calls):
         ours.append(timed(lambda: learner.ppo_grad(mb)))
+        if lb is not None:
+            bf.append(timed(lambda: lb.ppo_grad(mb)))
         f32.append(timed(lambda: learner.forward(fwd)))
         if torch_ok:
             tor.append(timed(torch_step))
@@ -112,8 +157,22 @@ def run_case(config, E, T, calls):
              first_pass_stats=dict(zip(("policy_loss", "value_loss", "entropy", "approx_kl", "clip_fraction", "S", "acted_rows",
                                         "loss"), [float(x) for x in stats])),
              ratio_bf16_behaviour_fp32_learner=spread)
+    if lb is not None:
+        flops, n_in = tc_flops(host["node_order"], E * N)
+        tab32 = kernel_table(lambda: learner.ppo_grad(mb))
+        tab16 = kernel_table(lambda: lb.ppo_grad(mb))
+        tc_ms = sum(v for k, v in tab16.items() if "k_tc_gemm" in k)
+        r.update(bf16_ppo_grad_ms=med(bf), bf16_ppo_grad_ms_calls=[round(x, 3) for x in bf],
+                 bf16_speedup_over_fp32=round(med(ours) / med(bf), 2),
+                 bf16_workspace_bytes=int(lb.lib.fl_policy_workspace_bytes_grad_bf16(E * N)),
+                 bf16_first_pass_stats=dict(zip(("policy_loss", "value_loss", "entropy", "approx_kl", "clip_fraction", "S",
+                                                 "acted_rows", "loss"), [float(x) for x in stats_bf16])),
+                 ratio_bf16_behaviour_bf16_learner=spread_bf16,
+                 inner_nodes=n_in, tc_product_gflop=round(flops / 1e9, 2), tc_kernel_ms=round(tc_ms, 3),
+                 tc_achieved_tflops=round(flops / (tc_ms * 1e-3) / 1e12, 1) if tc_ms > 0 else None,
+                 kernels_fp32_ms_per_call=tab32, kernels_bf16_ms_per_call=tab16)
     print(json.dumps(r), flush=True)
-    del ro, batch, learner, tp
+    del ro, batch, learner, tp, lb
     torch.cuda.empty_cache()
     return r
 
@@ -121,6 +180,7 @@ def run_case(config, E, T, calls):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--calls", type=int, default=5, help="alternated timed calls per implementation")
+    ap.add_argument("--bf16", action="store_true", help="also time the bf16 learner and profile both")
     ap.add_argument("--out", required=True, help="JSON file the results are written to (its directory is created)")
     args = ap.parse_args()
     if not torch.cuda.is_available():
@@ -132,7 +192,7 @@ def main():
         power = "unknown"
     out = dict(gpu=torch.cuda.get_device_name(0), power_limit=power, calls=args.calls)
     print(json.dumps(out), flush=True)
-    out["cases"] = [run_case(config, E, T, args.calls) for config, E, T in CASES]
+    out["cases"] = [run_case(config, E, T, args.calls, args.bf16) for config, E, T in CASES]
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, "w") as f:
         json.dump(out, f, indent=1)
