@@ -1415,6 +1415,7 @@ struct PpoIn {
     const uint8_t *valid, *actions; const float *old_lp, *adv, *ret; const uint8_t *acted;
     float eps, vf, ent;
     float *const *grads; float *logits, *value, *stats;
+    const long long *gcnt;   // the loss's denominators [|S|, acted rows] over the whole minibatch; null: these rows' own counts
 };
 
 // The training forward (fl_policy_forward_f32's arithmetic on F32Lin: every level and layer in its own slice of the
@@ -1499,11 +1500,14 @@ int run(Lin &lin, const float *const *wts, Wg &ws, long long E, long long N, con
     if (!loss) return (int)cudaGetLastError();
 
     // ==== PPO loss: d loss / d logits, d loss / d critic output, statistics ====
+    // these rows' counts go to words 32..35 of ws.counts (zeroed above); one shard of a minibatch divides by the minibatch's
+    unsigned long long *cnt = reinterpret_cast<unsigned long long *>(ws.counts + 32);
+    const long long *gcnt = in.gcnt ? in.gcnt : reinterpret_cast<const long long *>(cnt);
     PpoArgs pa{in.logits, in.value, in.old_lp, in.adv, in.ret, in.valid, in.actions, in.acted, E, (int)N, in.eps, in.vf, in.ent,
-               ws.counts + 32, ws.dlogits, ws.dcrit, ws.rowstats};
+               cnt, ws.dlogits, ws.dcrit, ws.rowstats, gcnt};
     k_ppo_count<<<(unsigned)E, 128, 0, st>>>(pa);
     k_ppo_loss<<<(unsigned)E, 128, 0, st>>>(pa);
-    k_ppo_stats<<<1, 256, 0, st>>>(ws.rowstats, E, ws.counts + 32, in.vf, in.ent, in.stats);
+    k_ppo_stats<<<1, 256, 0, st>>>(ws.rowstats, E, cnt, gcnt, in.vf, in.ent, in.stats);
     g_launches += 3;
 
     // ==== backward: heads (net_tree.py:56-71, 100-110); the last layers (N = 5, 1) stay on F32Lin ====
@@ -1817,19 +1821,38 @@ size_t fl_policy_workspace_bytes_grad_f32(int64_t n_agents_total) {
     return f32grad::carve(w, nullptr, n_agents_total);
 }
 
+// fl_policy_ppo_grad_{f32,bf16} are the shard path fed from the workspace's own count (gcnt null)
+static int ppo_grad(bool bf16, const int64_t *gcnt, const float *const *wts, void *d_workspace, size_t workspace_bytes,
+                    int64_t E, int64_t N, const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
+                    const int32_t *d_node_order, const uint8_t *d_valid_actions, const uint8_t *d_actions,
+                    const float *d_old_log_probs, const float *d_advantages, const float *d_returns, const uint8_t *d_acted,
+                    const FlPpoParams *params, float *const *d_grads, float *d_logits, float *d_value, float *d_stats,
+                    void *stream) {
+    const ppograph::PpoIn in{d_agent_attr, d_forest, d_adjacency, d_node_order, d_valid_actions, d_actions, d_old_log_probs, d_advantages,
+                             d_returns, d_acted, params ? params->clip_eps : 0.0f, params ? params->vf_coef : 0.0f,
+                             params ? params->ent_coef : 0.0f, d_grads, d_logits, d_value, d_stats,
+                             reinterpret_cast<const long long *>(gcnt)};
+    f32grad::Wg ws;
+    if (ppograph::check_args(wts, d_workspace, workspace_bytes, E, N, in, params, ws)) return -1;
+    if (!bf16) {
+        ppograph::F32Lin lin{(cudaStream_t)stream, ws.part};
+        return ppograph::run(lin, wts, ws, E, N, in, true, (cudaStream_t)stream);
+    }
+    const int rc = ppograph::bf16_setup();
+    if (rc) return rc;
+    ppograph::Bf16Lin lin{(cudaStream_t)stream, ws.part};
+    return ppograph::run(lin, wts, ws, E, N, in, true, (cudaStream_t)stream);
+}
+
 int fl_policy_ppo_grad_f32(const float *const *wts, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
                            const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
                            const int32_t *d_node_order, const uint8_t *d_valid_actions, const uint8_t *d_actions,
                            const float *d_old_log_probs, const float *d_advantages, const float *d_returns, const uint8_t *d_acted,
                            const FlPpoParams *params, float *const *d_grads, float *d_logits, float *d_value, float *d_stats,
                            void *stream) {
-    const ppograph::PpoIn in{d_agent_attr, d_forest, d_adjacency, d_node_order, d_valid_actions, d_actions, d_old_log_probs, d_advantages,
-                             d_returns, d_acted, params ? params->clip_eps : 0.0f, params ? params->vf_coef : 0.0f,
-                             params ? params->ent_coef : 0.0f, d_grads, d_logits, d_value, d_stats};
-    f32grad::Wg ws;
-    if (ppograph::check_args(wts, d_workspace, workspace_bytes, E, N, in, params, ws)) return -1;
-    ppograph::F32Lin lin{(cudaStream_t)stream, ws.part};
-    return ppograph::run(lin, wts, ws, E, N, in, true, (cudaStream_t)stream);
+    return ppo_grad(false, nullptr, wts, d_workspace, workspace_bytes, E, N, d_agent_attr, d_forest, d_adjacency, d_node_order,
+                    d_valid_actions, d_actions, d_old_log_probs, d_advantages, d_returns, d_acted, params, d_grads, d_logits, d_value,
+                    d_stats, stream);
 }
 
 // ---- the same loss and gradients with the dense products on the tensor cores (policy_bf16_grad.cuh) --------------------
@@ -1841,15 +1864,54 @@ int fl_policy_ppo_grad_bf16(const float *const *wts, void *d_workspace, size_t w
                             const float *d_old_log_probs, const float *d_advantages, const float *d_returns, const uint8_t *d_acted,
                             const FlPpoParams *params, float *const *d_grads, float *d_logits, float *d_value, float *d_stats,
                             void *stream) {
-    const ppograph::PpoIn in{d_agent_attr, d_forest, d_adjacency, d_node_order, d_valid_actions, d_actions, d_old_log_probs, d_advantages,
-                             d_returns, d_acted, params ? params->clip_eps : 0.0f, params ? params->vf_coef : 0.0f,
-                             params ? params->ent_coef : 0.0f, d_grads, d_logits, d_value, d_stats};
-    f32grad::Wg ws;
-    if (ppograph::check_args(wts, d_workspace, workspace_bytes, E, N, in, params, ws)) return -1;
-    const int rc = ppograph::bf16_setup();
-    if (rc) return rc;
-    ppograph::Bf16Lin lin{(cudaStream_t)stream, ws.part};
-    return ppograph::run(lin, wts, ws, E, N, in, true, (cudaStream_t)stream);
+    return ppo_grad(true, nullptr, wts, d_workspace, workspace_bytes, E, N, d_agent_attr, d_forest, d_adjacency, d_node_order,
+                    d_valid_actions, d_actions, d_old_log_probs, d_advantages, d_returns, d_acted, params, d_grads, d_logits, d_value,
+                    d_stats, stream);
+}
+
+// ---- one shard of a data-parallel minibatch: the counts of its rows, and the loss divided by the minibatch's counts ------
+int fl_policy_ppo_counts(int64_t E, int64_t N, const uint8_t *d_valid_actions, const uint8_t *d_acted, int64_t *d_counts,
+                         void *stream) {
+    if (E <= 0 || N <= 0 || !d_valid_actions || !d_acted || !d_counts) return -1;
+    if (N > (1ll << 31) / f32path::NODES || E > ((1ll << 31) / f32path::NODES) / N) return -1;      // as fl_policy_ppo_grad_f32
+    const cudaStream_t st = (cudaStream_t)stream;
+    const cudaError_t err = cudaMemsetAsync(d_counts, 0, 2 * sizeof(int64_t), st);
+    if (err != cudaSuccess) return (int)err;
+    f32grad::PpoArgs pa{};
+    pa.valid = d_valid_actions;
+    pa.acted = d_acted;
+    pa.E = E;
+    pa.N = (int)N;
+    pa.cnt = reinterpret_cast<unsigned long long *>(d_counts);
+    f32grad::k_ppo_count<<<(unsigned)E, 128, 0, st>>>(pa);
+    g_launches++;
+    return (int)cudaGetLastError();
+}
+
+int fl_policy_ppo_grad_shard_f32(const float *const *wts, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
+                                 const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
+                                 const int32_t *d_node_order, const uint8_t *d_valid_actions, const uint8_t *d_actions,
+                                 const float *d_old_log_probs, const float *d_advantages, const float *d_returns, const uint8_t *d_acted,
+                                 const int64_t *d_global_counts,
+                                 const FlPpoParams *params, float *const *d_grads, float *d_logits, float *d_value, float *d_stats,
+                                 void *stream) {
+    if (!d_global_counts) return -1;
+    return ppo_grad(false, d_global_counts, wts, d_workspace, workspace_bytes, E, N, d_agent_attr, d_forest, d_adjacency, d_node_order,
+                    d_valid_actions, d_actions, d_old_log_probs, d_advantages, d_returns, d_acted, params, d_grads, d_logits, d_value,
+                    d_stats, stream);
+}
+
+int fl_policy_ppo_grad_shard_bf16(const float *const *wts, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
+                                  const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
+                                  const int32_t *d_node_order, const uint8_t *d_valid_actions, const uint8_t *d_actions,
+                                  const float *d_old_log_probs, const float *d_advantages, const float *d_returns, const uint8_t *d_acted,
+                                  const int64_t *d_global_counts,
+                                  const FlPpoParams *params, float *const *d_grads, float *d_logits, float *d_value, float *d_stats,
+                                  void *stream) {
+    if (!d_global_counts) return -1;
+    return ppo_grad(true, d_global_counts, wts, d_workspace, workspace_bytes, E, N, d_agent_attr, d_forest, d_adjacency, d_node_order,
+                    d_valid_actions, d_actions, d_old_log_probs, d_advantages, d_returns, d_acted, params, d_grads, d_logits, d_value,
+                    d_stats, stream);
 }
 
 int fl_policy_forward_train_bf16(const float *const *wts, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
@@ -1864,7 +1926,7 @@ int fl_policy_forward_train_bf16(const float *const *wts, void *d_workspace, siz
     const int rc = ppograph::bf16_setup();
     if (rc) return rc;
     const ppograph::PpoIn in{d_agent_attr, d_forest, d_adjacency, d_node_order, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
-                             0.0f, 0.0f, 0.0f, nullptr, d_logits, d_value, nullptr};
+                             0.0f, 0.0f, 0.0f, nullptr, d_logits, d_value, nullptr, nullptr};
     ppograph::Bf16Lin lin{(cudaStream_t)stream, ws.part};
     return ppograph::run(lin, wts, ws, E, N, in, false, (cudaStream_t)stream);
 }

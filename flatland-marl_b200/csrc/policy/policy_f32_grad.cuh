@@ -6,9 +6,11 @@
 // pre-activations (GemmArgs::pre), attention its log-sum-exp per (agent, head).  The level lists are built in a fixed order
 // (tree order, then node order; k_tl_*) instead of by atomics, because the weight gradients reduce over their rows.
 //
-// Loss: k_ppo_count (|S| and the number of acted rows; integer atomics, exact in any order), k_ppo_loss (one CTA per
-// environment row: log pi with masked_choice's arithmetic, clipped surrogate, entropy, value term, d loss / d logits and
-// d loss / d critic output), k_ppo_stats (one CTA, fixed-order reduction of the per-row sums).
+// Loss: k_ppo_count (|S| and the number of acted rows; int64 integer atomics, exact in any order and across shards),
+// k_ppo_loss (one CTA per environment row: log pi with masked_choice's arithmetic, clipped surrogate, entropy, value term,
+// d loss / d logits and d loss / d critic output), k_ppo_stats (one CTA, fixed-order reduction of the per-row sums).  The
+// loss and the statistics divide by the denominators in PpoArgs::gcnt: the call's own counts, or the counts of the whole
+// minibatch when the rows are one shard of it (fl_policy_ppo_grad_shard_*).
 //
 // Backward: k_gemm_dx (dX = dY W, optional gathered output rows, added term, accumulation and GELU' epilogue), k_gemm_dw +
 // k_dw_reduce (dW = dY^T X and db over fixed row chunks into partial buffers, then summed in chunk order), k_attn_bwd_q /
@@ -391,8 +393,9 @@ struct PpoArgs {
     const uint8_t *valid, *actions, *acted;
     long long E; int N;
     float eps, vf, ent;
-    int32_t *cnt;                       // [0] |S|, [1] acted rows
+    unsigned long long *cnt;            // [0] |S|, [1] acted rows of these rows (k_ppo_count; zeroed before it)
     float *dlogits, *dcrit, *rowstats;  // [T][5], [T], [E][5]
+    const long long *gcnt;              // the denominators: [0] |S|, [1] acted rows of the whole minibatch (cnt for one shard)
 };
 
 __device__ __forceinline__ int block_sum_i(int v, int *sh) {
@@ -416,8 +419,8 @@ __global__ void k_ppo_count(PpoArgs p) {
     }
     n = block_sum_i(n, sh);
     if (threadIdx.x == 0) {
-        if (n) atomicAdd(&p.cnt[0], n);
-        atomicAdd(&p.cnt[1], 1);
+        if (n) atomicAdd(&p.cnt[0], (unsigned long long)n);
+        atomicAdd(&p.cnt[1], 1ull);
     }
 }
 
@@ -426,7 +429,7 @@ __global__ void k_ppo_count(PpoArgs p) {
 __global__ void __launch_bounds__(128) k_ppo_loss(PpoArgs p) {
     __shared__ float sh[4][128];
     const long long e = blockIdx.x;
-    const int nS = p.cnt[0], nR = p.cnt[1];
+    const long long nS = p.gcnt[0], nR = p.gcnt[1];
     const bool acted = p.acted[e] != 0;
     const float invS = nS > 0 ? 1.0f / (float)nS : 0.0f;
     const float A = p.adv[e], dV = (acted && nR > 0) ? p.vf * 2.0f * (p.value[e] - p.ret[e]) / (float)nR : 0.0f;
@@ -477,8 +480,10 @@ __global__ void __launch_bounds__(128) k_ppo_loss(PpoArgs p) {
     }
 }
 
-// one CTA of 256 threads: stats = (policy, value, entropy, approx KL, clip fraction, |S|, acted rows, total loss)
-__global__ void __launch_bounds__(256) k_ppo_stats(const float *__restrict__ rowstats, long long E, const int32_t *__restrict__ cnt,
+// one CTA of 256 threads: stats = (policy, value, entropy, approx KL, clip fraction, |S|, acted rows, total loss); the sums
+// over these rows divided by the minibatch's counts gcnt, and the counts cnt of these rows
+__global__ void __launch_bounds__(256) k_ppo_stats(const float *__restrict__ rowstats, long long E,
+                                                   const unsigned long long *__restrict__ cnt, const long long *__restrict__ gcnt,
                                                    float vf, float ent, float *__restrict__ stats) {
     __shared__ float sh[5][256];
     float acc[5] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f};
@@ -492,16 +497,17 @@ __global__ void __launch_bounds__(256) k_ppo_stats(const float *__restrict__ row
         __syncthreads();
     }
     if (threadIdx.x == 0) {
-        const float nS = (float)cnt[0], nR = (float)cnt[1];
-        const float pol = cnt[0] ? sh[0][0] / nS : 0.0f, entm = cnt[0] ? sh[1][0] / nS : 0.0f;
-        const float val = cnt[1] ? sh[4][0] / nR : 0.0f;
+        const bool hS = gcnt[0] > 0, hR = gcnt[1] > 0;
+        const float nS = (float)gcnt[0], nR = (float)gcnt[1];
+        const float pol = hS ? sh[0][0] / nS : 0.0f, entm = hS ? sh[1][0] / nS : 0.0f;
+        const float val = hR ? sh[4][0] / nR : 0.0f;
         stats[0] = pol;
         stats[1] = val;
         stats[2] = entm;
-        stats[3] = cnt[0] ? sh[2][0] / nS : 0.0f;
-        stats[4] = cnt[0] ? sh[3][0] / nS : 0.0f;
-        stats[5] = nS;
-        stats[6] = nR;
+        stats[3] = hS ? sh[2][0] / nS : 0.0f;
+        stats[4] = hS ? sh[3][0] / nS : 0.0f;
+        stats[5] = (float)cnt[0];
+        stats[6] = (float)cnt[1];
         stats[7] = pol - ent * entm + vf * val;
     }
 }

@@ -8,11 +8,16 @@ caller's: `torch.optim` and `torch.nn.utils.clip_grad_norm_` work on `parameters
 precision="bf16" computes the same loss through the same graph with the dense products of the 20 large weight matrices on
 the tensor cores (fl_policy_ppo_grad_bf16: bf16 operands, fp32 accumulation, fp32 master weights and gradients); see
 DESIGN.md §4.8 for what the two learners trade.
+
+group= (a torch.distributed process group, NCCL on GPUs) makes the learner data-parallel: every rank passes its own share of
+one minibatch, and ppo_grad leaves on every rank the gradient and the statistics of the whole minibatch (DESIGN.md §4.9,
+INTEGRATION.md §7b).
 """
 import ctypes as C
 from collections import OrderedDict
 
 import torch
+import torch.distributed as dist
 
 from . import policy_weights as pw
 from ._lib import FlatlandB200Error
@@ -35,9 +40,15 @@ class PolicyLearner:
         stats = learner.ppo_grad(rollout.minibatch(ids))   # writes every parameter's .grad
         optimizer.step()                                   # e.g. torch.optim.Adam(learner.parameters())
         rollout.actor = learner.actor()                    # acting with the new parameters
+
+    group: None, or a torch.distributed process group over which each minibatch is split by rows.  Construction is then a
+    collective: the parameters are broadcast from the group's first rank, so every rank starts from the same bytes.  The 46
+    .grad tensors and the statistics are views of one flat fp32 buffer, so that ppo_grad ends in a single all-reduce; views
+    dropped by the caller (zero_grad(set_to_none=True)) are reattached by the next call.  Every rank must make the same
+    sequence of ppo_grad calls, a rank with no rows in a minibatch included (pass it the empty minibatch).
     """
 
-    def __init__(self, weights=None, device="cuda:0", seed=0, precision="fp32"):
+    def __init__(self, weights=None, device="cuda:0", seed=0, precision="fp32", group=None):
         if precision not in ("fp32", "bf16"):
             raise ValueError("precision must be 'fp32' or 'bf16'")
         if not torch.cuda.is_available():
@@ -52,6 +63,29 @@ class PolicyLearner:
         self._ws = None
         self._out = None
         self._stats = torch.zeros(8, dtype=torch.float32, device=self.device)
+        self.group = group
+        if group is not None:
+            self._init_group()
+
+    def _init_group(self):
+        """The flat buffer [all parameters' gradients in weight_spec order | 8 statistics], its views, the int64 counts, and
+        the parameters broadcast from the group's first rank."""
+        ps = list(self._params.values())
+        n = sum(p.numel() for p in ps)
+        self._flat = torch.zeros(n + 8, dtype=torch.float32, device=self.device)
+        self._grad_views, off = [], 0
+        for p in ps:
+            self._grad_views.append(self._flat[off:off + p.numel()].view(p.shape))
+            off += p.numel()
+        self._stats = self._flat[n:]
+        self._counts = torch.zeros(2, dtype=torch.int64, device=self.device)
+        with torch.no_grad():
+            w = torch.cat([p.detach().reshape(-1) for p in ps])
+            dist.broadcast(w, src=dist.get_global_rank(self.group, 0), group=self.group)
+            off = 0
+            for p in ps:
+                p.copy_(w[off:off + p.numel()].view(p.shape))
+                off += p.numel()
 
     def parameters(self):
         return iter(self._params.values())
@@ -126,7 +160,12 @@ class PolicyLearner:
 
         Returns the statistics as a float32 [8] device tensor (policy loss, value loss, entropy, approximate KL, clip
         fraction, |S|, acted rows, total loss), reused by the next call.  The one host synchronisation is the fp32 path's
-        (per-level node counts), in both precisions."""
+        (per-level node counts), in both precisions.
+
+        With a group, mb is this rank's share of the minibatch (it may have no rows), and all of this is enqueued on the
+        current stream with no torch-side host synchronisation: fl_policy_ppo_counts of the share, all_reduce of the counts,
+        fl_policy_ppo_grad_shard_* with those counts, all_reduce of the flat gradient and statistics buffer.  Every rank then
+        holds the gradient and the statistics of the whole minibatch, byte-identical across ranks."""
         E, N = self._check_obs(mb, MB_KEYS)
         for name, dt in ROW_KEYS:
             t = mb[name]
@@ -134,11 +173,9 @@ class PolicyLearner:
                 raise ValueError("%s must be a contiguous %s tensor of shape (%d,) on %s" % (name, dt, E, self.device))
         if not clip_eps > 0:
             raise ValueError("clip_eps must be positive")
-        bf16 = self.precision == "bf16"
-        need = int(self.lib.fl_policy_workspace_bytes_grad_bf16(E * N) if bf16 else self.lib.fl_policy_workspace_bytes_grad_f32(E * N))
-        if self._ws is None or self._ws.numel() < need:
-            self._ws = None
-            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        if self.group is not None:
+            return self._ppo_grad_shard(mb, E, N, clip_eps, vf_coef, ent_coef)
+        self._workspace(E, N)
         grads = []
         for p in self._params.values():
             if p.grad is None or p.grad.shape != p.shape or p.grad.dtype != torch.float32 or p.grad.device != self.device \
@@ -147,12 +184,47 @@ class PolicyLearner:
             grads.append(p.grad)
         logits, value = self._outputs(E, N)
         params = FlPpoParams(float(clip_eps), float(vf_coef), float(ent_coef))
-        fn, name = (self.lib.fl_policy_ppo_grad_bf16, "fl_policy_ppo_grad_bf16") if bf16 else \
+        fn, name = (self.lib.fl_policy_ppo_grad_bf16, "fl_policy_ppo_grad_bf16") if self.precision == "bf16" else \
             (self.lib.fl_policy_ppo_grad_f32, "fl_policy_ppo_grad_f32")
         _check(fn(self._weights(), self._ws.data_ptr(), self._ws.numel(), E, N,
                   *(mb[k].data_ptr() for k, _, _ in MB_KEYS), *(mb[k].data_ptr() for k, _ in ROW_KEYS),
                   C.byref(params), self._ptrs(grads), logits.data_ptr(), value.data_ptr(),
                   self._stats.data_ptr(), self._stream()), name)
+        return self._stats
+
+    def _workspace(self, E, N):
+        bf16 = self.precision == "bf16"
+        need = int(self.lib.fl_policy_workspace_bytes_grad_bf16(E * N) if bf16 else self.lib.fl_policy_workspace_bytes_grad_f32(E * N))
+        if self._ws is None or self._ws.numel() < need:
+            self._ws = None
+            self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+
+    def _ppo_grad_shard(self, mb, E, N, clip_eps, vf_coef, ent_coef):
+        """ppo_grad of one rank's share: this rank's contribution computed with the minibatch's counts, then summed over the
+        group.  A share with no rows contributes zero counts, gradients and statistics and joins the same collectives."""
+        for p, v in zip(self._params.values(), self._grad_views):
+            if p.grad is None or p.grad.data_ptr() != v.data_ptr() or p.grad.shape != v.shape or p.grad.stride() != v.stride():
+                p.grad = v
+        stream = self._stream()
+        if E > 0:
+            _check(self.lib.fl_policy_ppo_counts(E, N, mb["valid_actions"].data_ptr(), mb["acted"].data_ptr(),
+                                                 self._counts.data_ptr(), stream), "fl_policy_ppo_counts")
+        else:
+            self._counts.zero_()
+        dist.all_reduce(self._counts, group=self.group)
+        logits, value = self._outputs(E, N)
+        if E > 0:
+            self._workspace(E, N)
+            params = FlPpoParams(float(clip_eps), float(vf_coef), float(ent_coef))
+            fn, name = (self.lib.fl_policy_ppo_grad_shard_bf16, "fl_policy_ppo_grad_shard_bf16") if self.precision == "bf16" \
+                else (self.lib.fl_policy_ppo_grad_shard_f32, "fl_policy_ppo_grad_shard_f32")
+            _check(fn(self._weights(), self._ws.data_ptr(), self._ws.numel(), E, N,
+                      *(mb[k].data_ptr() for k, _, _ in MB_KEYS), *(mb[k].data_ptr() for k, _ in ROW_KEYS),
+                      self._counts.data_ptr(), C.byref(params), self._ptrs(self._grad_views), logits.data_ptr(),
+                      value.data_ptr(), self._stats.data_ptr(), stream), name)
+        else:
+            self._flat.zero_()
+        dist.all_reduce(self._flat, group=self.group)
         return self._stats
 
     def last_outputs(self):

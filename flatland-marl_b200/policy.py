@@ -20,7 +20,8 @@ LAYERS = pw.N_TRANSFORMER
 
 EXPORTS = ["fl_policy_abi_version", "fl_policy_workspace_bytes", "fl_policy_forward", "fl_policy_workspace_bytes_f32",
            "fl_policy_forward_f32", "fl_policy_workspace_bytes_grad_f32", "fl_policy_ppo_grad_f32", "fl_policy_workspace_bytes_grad_bf16",
-           "fl_policy_ppo_grad_bf16", "fl_policy_forward_train_bf16", "fl_policy_tc_product_bf16", "fl_policy_choose_actions",
+           "fl_policy_ppo_grad_bf16", "fl_policy_forward_train_bf16", "fl_policy_tc_product_bf16", "fl_policy_ppo_counts",
+           "fl_policy_ppo_grad_shard_f32", "fl_policy_ppo_grad_shard_bf16", "fl_policy_choose_actions",
            "fl_policy_sample_actions", "fl_policy_gae",
            "fl_policy_linear", "fl_policy_linear_debug", "fl_policy_debug_clocks", "fl_policy_launch_count"]
 
@@ -85,6 +86,11 @@ def lib():
     L.fl_policy_ppo_grad_bf16.argtypes = [P, P, C.c_size_t, C.c_int64, C.c_int64] + [P] * 10 + [C.POINTER(FlPpoParams), P, P, P, P, P]
     L.fl_policy_forward_train_bf16.restype = C.c_int
     L.fl_policy_forward_train_bf16.argtypes = [P, P, C.c_size_t, C.c_int64, C.c_int64, P, P, P, P, P, P, P]
+    L.fl_policy_ppo_counts.restype = C.c_int
+    L.fl_policy_ppo_counts.argtypes = [C.c_int64, C.c_int64, P, P, P, P]
+    for name in ("fl_policy_ppo_grad_shard_f32", "fl_policy_ppo_grad_shard_bf16"):
+        getattr(L, name).restype = C.c_int
+        getattr(L, name).argtypes = [P, P, C.c_size_t, C.c_int64, C.c_int64] + [P] * 11 + [C.POINTER(FlPpoParams), P, P, P, P, P]
     L.fl_policy_tc_product_bf16.restype = C.c_int
     L.fl_policy_tc_product_bf16.argtypes = [C.POINTER(FlTcProduct), P, C.c_size_t, P]
     L.fl_policy_choose_actions.restype = C.c_int

@@ -157,6 +157,51 @@ int fl_policy_forward_train_bf16(const float *const *d_weights, void *d_workspac
                                  const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
                                  const int32_t *d_node_order, float *d_logits, float *d_value, void *stream);
 
+/* Data-parallel learning: one minibatch split by rows into shards (one per GPU), each shard's loss divided by the counts of
+ * the whole minibatch, so that the shard gradients sum to the minibatch's gradient.
+ *
+ * fl_policy_ppo_counts writes d_counts [2] i64 = [|S|, acted rows] of these E rows (S and rows as in the loss statement of
+ * fl_policy_ppo_grad_f32), computed from d_valid_actions [E][N][5] u8 and d_acted [E] u8 alone.  Integer counts: their sum
+ * over shards, in any order, is the minibatch's count.  One memset and one kernel on `stream`, no host synchronisation.
+ *
+ * fl_policy_ppo_grad_shard_f32 / _bf16 take the arguments of fl_policy_ppo_grad_f32 / _bf16 and d_global_counts, a device
+ * pointer to [|S_g|, rows_g] i64: |S| and the acted rows of the whole minibatch (the sum over its shards of
+ * fl_policy_ppo_counts), read on the device.  With S, rows the sets of this shard, the shard's loss is
+ *   L_shard = sum_S( -min(r A, clip(r, 1 - clip_eps, 1 + clip_eps) A) ) / |S_g| - ent_coef sum_S(H) / |S_g|
+ *             + vf_coef sum_rows((V - R)^2) / rows_g,
+ * a term with a zero denominator contributing 0; every symbol, the tie rule and the arithmetic are those of
+ * fl_policy_ppo_grad_f32 / _bf16.  The sum over the shards of L_shard is L of the whole minibatch, so:
+ *   - d_grads: dL_shard / dparameter, this shard's contribution; the sum over shards is dL/dparameter of the minibatch.
+ *   - d_stats [8]: entries 0..4 and 7 are this shard's sums over S (over rows for entry 1) divided by |S_g| (rows_g), so
+ *     their sum over shards is the minibatch's statistic; entries 5 and 6 are |S| and the acted rows of this shard, so
+ *     their sum is the minibatch's count.
+ *   - d_logits, d_value: as fl_policy_ppo_grad_f32 / _bf16; they do not depend on the counts.
+ * Given d_global_counts = fl_policy_ppo_counts of its own rows, a shard call writes the bytes fl_policy_ppo_grad_f32 / _bf16
+ * write (those calls are this path with the counts taken from the workspace).  The training forward, the backward, the
+ * determinism and the one host synchronisation are those calls'.  FL_ERR_BAD_ARG before any CUDA call for the argument
+ * errors of fl_policy_ppo_grad_f32 and for a NULL d_global_counts; for fl_policy_ppo_counts, for a NULL pointer, E <= 0,
+ * N <= 0, or E N above the 32-bit node-id bound of fl_policy_ppo_grad_f32. */
+int fl_policy_ppo_counts(int64_t E, int64_t N, const uint8_t *d_valid_actions, const uint8_t *d_acted, int64_t *d_counts,
+                         void *stream);
+int fl_policy_ppo_grad_shard_f32(const float *const *d_weights, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
+                                 const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
+                                 const int32_t *d_node_order, const uint8_t *d_valid_actions,
+                                 const uint8_t *d_actions, const float *d_old_log_probs,
+                                 const float *d_advantages, const float *d_returns,
+                                 const uint8_t *d_acted, const int64_t *d_global_counts,
+                                 const FlPpoParams *params,
+                                 float *const *d_grads,
+                                 float *d_logits, float *d_value, float *d_stats, void *stream);
+int fl_policy_ppo_grad_shard_bf16(const float *const *d_weights, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
+                                  const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
+                                  const int32_t *d_node_order, const uint8_t *d_valid_actions,
+                                  const uint8_t *d_actions, const float *d_old_log_probs,
+                                  const float *d_advantages, const float *d_returns,
+                                  const uint8_t *d_acted, const int64_t *d_global_counts,
+                                  const FlPpoParams *params,
+                                  float *const *d_grads,
+                                  float *d_logits, float *d_value, float *d_stats, void *stream);
+
 /* One tensor-core product of fl_policy_ppo_grad_bf16, exposed for tests.  bf16-rounded operands, fp32 accumulation; every
  * other term in fp32.  X(m, k) = x1[row(m) ldx1 + k] (k < K1), x2[m ldx2 + k - K1] (K1 <= k < K = K1 + K2); row(m) = idx ?
  * idx[m] : m.  Row strides in floats.
