@@ -61,7 +61,7 @@ struct LinArgs {
     const uint32_t *entries;    // MODE_TREE_F: level list (tree | node << 22 | first child << 27)
     const bf16 *cstate;         //              c of every node [tree][32][128]
     bf16 *fc;                   //              f * c_child     [tree][32][128]
-    const uint8_t *eflags;      //              per list entry: bit j = child j of the node is a null node (shared h / c row)
+    const uint8_t *eflags;      //              per list entry: bit j = child j of the node is a null leaf (shared h / c row)
     uint32_t null_off;          //              element offset of that shared row in h / c
 };
 
@@ -585,7 +585,7 @@ struct TreeArgs {
     int emb_ld;
     const bf16 *uiou, *wiou, *wc;
     const float *b_iou, *b_c;
-    const uint8_t *eflags;     // per list entry: bit j = child j of the node is a null node: its h is a shared row at null_off
+    const uint8_t *eflags;     // per list entry: bit j = child j of the node is a null leaf: its h is a shared row at null_off
     uint32_t null_off;
 };
 
@@ -647,7 +647,7 @@ __global__ void __launch_bounds__(416, 1) k_tree_p(const TreeArgs p, const __gri
                     entry_decode(ent[i], t, v, ch0);
                     offc[i] = (t * NODES + ch0) * 128u;
                     offx[i] = (t * NODES + v) * 16u;
-                    nul[i] = efl[i];                                   // which of the three children are null nodes
+                    nul[i] = efl[i];                                   // which of the three children are null leaves
                     offn[i] = p.null_off + (t & (NULL_COPIES - 1)) * (NODES * 128u);
                 }
             }
@@ -870,7 +870,7 @@ __global__ void k_tree_plan(const int32_t *__restrict__ adjacency, const int32_t
     unsigned char child0[32];
     unsigned short pos[31];
     signed char lvl[31];
-    uint32_t nm = 0;
+    uint32_t shared = 0;   // bit v: node v is a null leaf, whose h / c its parent reads from the shared null row
     if (t < M) {
 #pragma unroll 1
         for (int v = 0; v < 32; v++) child0[v] = 0;
@@ -879,12 +879,14 @@ __global__ void k_tree_plan(const int32_t *__restrict__ adjacency, const int32_t
             const int par = adjacency[(t * 30 + 3 * g) * 3];
             if (par >= 0 && par < 31) child0[par] = (unsigned char)(3 * g + 1);
         }
-        nm = nullmask[t];
+        const uint32_t nm = nullmask[t];
 #pragma unroll 1
         for (int v = 0; v < 31; v++) {
             int o = node_order[t * 31 + v];
             if (o >= FL_POLICY_MAX_LEVELS) o = -1;
-            if (o == 0 && ((nm >> v) & 1u)) o = -1;       // a null leaf: its h / c is the shared row, nothing to compute
+            // a null leaf: its h / c is the shared row, nothing to compute.  A null-featured node with children is not
+            // shared: its state depends on its subtree, so it is computed in its own row and its parent reads that row.
+            if (o == 0 && ((nm >> v) & 1u)) { o = -1; shared |= 1u << v; }
             lvl[v] = (signed char)o;
             if (o >= 0) pos[v] = (unsigned short)atomicAdd(&cnt[o], 1);
         }
@@ -905,7 +907,7 @@ __global__ void k_tree_plan(const int32_t *__restrict__ adjacency, const int32_t
             if (o < 0) continue;
             const size_t off = o == 0 ? 0 : (size_t)21 * M + NULL_COPIES + (size_t)(o - 1) * 10 * M;
             lists[off + base[o] + pos[v]] = (uint32_t)t | ((uint32_t)v << 22) | ((uint32_t)child0[v] << 27);
-            eflags[off + base[o] + pos[v]] = (uint8_t)(o > 0 ? (nm >> child0[v]) & 7u : 0u);
+            eflags[off + base[o] + pos[v]] = (uint8_t)(o > 0 ? (shared >> child0[v]) & 7u : 0u);
         }
     }
 }
