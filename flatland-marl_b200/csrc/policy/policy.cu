@@ -1420,8 +1420,9 @@ struct PpoIn {
     const long long *gcnt;   // the loss's denominators [|S|, acted rows] over the whole minibatch; null: these rows' own counts
 };
 
-// The training forward (fl_policy_forward_f32's arithmetic on F32Lin: every level and layer in its own slice of the
-// workspace) and, when `loss`, the PPO loss and the backward pass.  Arguments are checked by the caller.
+// The forward pass and, when `loss`, the PPO loss and the backward pass.  On F32Lin with the forward-only layout
+// (carve(..., false)) this is fl_policy_forward_f32; with the training layout every level and layer keeps its own slice of
+// the workspace for the backward.  Both layouts give the same logits and values.  Arguments are checked by the caller.
 template <class Lin>
 int run(Lin &lin, const float *const *wts, Wg &ws, long long E, long long N, const PpoIn &in, bool loss, cudaStream_t st) {
     F32Lin f32{st, ws.part};
@@ -1438,19 +1439,22 @@ int run(Lin &lin, const float *const *wts, Wg &ws, long long E, long long N, con
     float *const *gr = in.grads;
     const float *d_agent_attr = in.agent_attr, *d_forest = in.forest;
 
-    // ==== training forward: fl_policy_forward_f32's arithmetic, every level and layer in its own slice ====
+    // ==== forward: Tree-LSTM (TreeLSTM.py:34-154), leaves, then one level at a time ====
     const long long nodes = T * f32path::NODES;
     cudaError_t err = cudaMemsetAsync(ws.h, 0, (size_t)nodes * T_H * 4, st);
     if (err == cudaSuccess) err = cudaMemsetAsync(ws.c, 0, (size_t)nodes * T_H * 4, st);
     if (err == cudaSuccess) err = cudaMemsetAsync(ws.counts, 0, 64 * 4, st);
     if (err != cudaSuccess) return (int)err;
-    k_clean<<<(unsigned)((nodes * NF + 255) / 256), 256, 0, st>>>(d_forest, ws.xcl, nodes * NF);
+    if (ws.xcl) {   // only the backward reads the cleaned features
+        k_clean<<<(unsigned)((nodes * NF + 255) / 256), 256, 0, st>>>(d_forest, ws.xcl, nodes * NF);
+        g_launches++;
+    }
     k_tl_count<<<(unsigned)((T + 127) / 128), 128, 0, st>>>(in.adjacency, in.node_order, T, ws.child_base, ws.tcnt);
     k_tl_scan<<<dim3((unsigned)ws.nblk, MAX_LEVELS), SCAN, 0, st>>>(ws.tcnt, T, ws.nblk, ws.tpos, ws.btot);
     k_tl_tops<<<1, 32, 0, st>>>(ws.btot, ws.nblk, ws.counts);
     k_tl_fill<<<(unsigned)((T + 127) / 128), 128, 0, st>>>(in.node_order, T, ws.nblk, ws.tpos, ws.btot, ws.counts, ws.lists);
     k_tree_leaves<<<(unsigned)nodes, 128, 0, st>>>(d_forest, in.node_order, nodes, W_iou, b_iou, ws.h, ws.c);
-    g_launches += 6;
+    g_launches += 5;
     int32_t counts[MAX_LEVELS];
     err = cudaMemcpyAsync(counts, ws.counts, sizeof(counts), cudaMemcpyDeviceToHost, st);
     if (err == cudaSuccess) err = cudaStreamSynchronize(st);        // per-level sizes of the launches below; the only host sync
@@ -1475,13 +1479,14 @@ int run(Lin &lin, const float *const *wts, Wg &ws, long long E, long long N, con
         k_inner<<<(unsigned)M, 128, 0, st>>>(iou, ws.craw, list, dM, d_forest, W_iou, b_iou, b_c, ws.h, ws.c);
         g_launches += 2;
     }
+    // attribute MLP (net_tree.py:41-50), emb = cat(attr embedding, h of the root)
     lin.gemm(d_agent_attr, nullptr, 83, 83, nullptr, 0, 0, wts[8], wts[9], ws.aa[0], 256, T, 256, 1, ws.ap[0]);
     lin.gemm(ws.aa[0], nullptr, 256, 256, nullptr, 0, 0, wts[10], wts[11], ws.aa[1], 256, T, 256, 1, ws.ap[1]);
     lin.gemm(ws.aa[1], nullptr, 256, 256, nullptr, 0, 0, wts[12], wts[13], ws.aa[2], 256, T, 256, 1, ws.ap[2]);
     lin.gemm(ws.aa[2], nullptr, 256, 256, nullptr, 0, 0, wts[14], wts[15], ws.emb, 256, T, 128, 1, ws.ap[3]);
     copy_cols(ws.h, (long long)f32path::NODES * T_H, ws.emb + 128, 256, T, 128);
     const float *x = ws.emb;
-    for (int l = 0; l < 3; l++) {
+    for (int l = 0; l < 3; l++) {   // three attention blocks (net_tree.py:20-32)
         const float *const *tw = wts + 16 + 6 * l;
         lin.gemm(x, nullptr, 256, 256, nullptr, 0, 0, tw[0], tw[1], ws.qkv[l], 768, T, 768, 0, nullptr);
         k_attention<<<(unsigned)((T * 4 * 32 + 255) / 256), 256, 0, st>>>(ws.qkv[l], ws.att[l], 256, E, (int)N, ws.lse[l]);
@@ -1492,7 +1497,7 @@ int run(Lin &lin, const float *const *wts, Wg &ws, long long E, long long N, con
         x = ws.xs[l];
     }
     const float *const *aw = wts + 34, *const *cw = wts + 40;
-    for (int hd = 0; hd < 2; hd++) {
+    for (int hd = 0; hd < 2; hd++) {   // heads on cat(emb, att) (net_tree.py:56-71, 100-110)
         const float *const *hw = hd ? cw : aw;
         lin.gemm(ws.emb, nullptr, 256, 256, x, 256, 256, hw[0], hw[1], ws.y1[hd], 256, T, 256, 1, ws.y1p[hd]);
         lin.gemm(ws.y1[hd], nullptr, 256, 256, nullptr, 0, 0, hw[2], hw[3], ws.y2[hd], 128, T, 128, 1, ws.y2p[hd]);
@@ -1587,18 +1592,31 @@ int run(Lin &lin, const float *const *wts, Wg &ws, long long E, long long N, con
     return (int)cudaGetLastError();
 }
 
-// the argument checks of fl_policy_ppo_grad_f32 (FL_ERR_BAD_ARG before any CUDA call)
+// E, N > 0 and E * N * 31 < 2^31: node ids are 32-bit
+bool bad_shape(int64_t E, int64_t N) {
+    return E <= 0 || N <= 0 || N > (1ll << 31) / f32path::NODES || E > ((1ll << 31) / f32path::NODES) / N;
+}
+
+// the observation-side argument checks of every entry point of the fp32 network (FL_ERR_BAD_ARG before any CUDA call);
+// carves `ws` out of d_workspace in the training layout when `train`, else in the forward-only one
+int check_obs(const float *const *wts, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N, const PpoIn &in,
+              Wg &ws, bool train) {
+    if (!wts || !d_workspace || !in.agent_attr || !in.forest || !in.adjacency || !in.node_order || !in.logits || !in.value)
+        return -1;
+    if (bad_shape(E, N)) return -1;
+    for (int i = 0; i < FL_POLICY_F32_TENSORS; i++)
+        if (!wts[i]) return -1;
+    return carve(ws, (unsigned char *)d_workspace, E * N, train) > workspace_bytes ? -1 : 0;
+}
+
+// the argument checks of fl_policy_ppo_grad_f32: the observation side and the loss's inputs
 int check_args(const float *const *wts, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N, const PpoIn &in,
                const FlPpoParams *params, Wg &ws) {
-    if (!wts || !in.grads || !params || !d_workspace || E <= 0 || N <= 0 || !in.agent_attr || !in.forest || !in.adjacency || !in.node_order ||
-        !in.valid || !in.actions || !in.old_lp || !in.adv || !in.ret || !in.acted || !in.logits || !in.value || !in.stats)
-        return -1;
-    if (N > (1ll << 31) / f32path::NODES || E > ((1ll << 31) / f32path::NODES) / N) return -1;      // node ids are 32-bit
+    if (!in.grads || !params || !in.valid || !in.actions || !in.old_lp || !in.adv || !in.ret || !in.acted || !in.stats) return -1;
     if (!(params->clip_eps > 0.0f)) return -1;
     for (int i = 0; i < FL_POLICY_F32_TENSORS; i++)
-        if (!wts[i] || !in.grads[i]) return -1;
-    if (carve(ws, (unsigned char *)d_workspace, E * N) > workspace_bytes) return -1;
-    return 0;
+        if (!in.grads[i]) return -1;
+    return check_obs(wts, d_workspace, workspace_bytes, E, N, in, ws, true);
 }
 
 }  // namespace ppograph
@@ -1733,94 +1751,29 @@ int fl_policy_forward(const FlPolicyWeights *w, void *d_workspace, size_t worksp
     return (int)cudaGetLastError();
 }
 
-// ---- the same forward pass in fp32 on the CUDA cores (policy_f32.cuh) --------------------------------------------------
+// ---- the same forward pass in fp32 on the CUDA cores (policy_f32.cuh): the training graph's forward, forward-only layout
 size_t fl_policy_workspace_bytes_f32(int64_t n_agents_total) {
     if (n_agents_total <= 0) return 0;
-    f32path::Ws w;
-    return f32path::carve(w, nullptr, n_agents_total);
+    f32grad::Wg w;
+    return f32grad::carve(w, nullptr, n_agents_total, false);
 }
 
 int fl_policy_forward_f32(const float *const *wts, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
                           const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
                           const int32_t *d_node_order, float *d_logits, float *d_value, void *stream) {
-    using namespace f32path;
-    if (!wts || !d_workspace || E <= 0 || N <= 0 || !d_agent_attr || !d_forest || !d_adjacency || !d_node_order || !d_logits || !d_value) return -1;
-    const long long T = E * N;
-    Ws ws;
-    if (carve(ws, (unsigned char *)d_workspace, T) > workspace_bytes) return -1;
-    cudaStream_t st = (cudaStream_t)stream;
-    auto gemm = [&](const float *a1, const int32_t *idx1, long long lda1, int K1, const float *a2, long long lda2, int K2,
-                    const float *w, const float *bias, float *c, long long ldc, long long M, int Nn, int act) {
-        if (M <= 0) return;
-        GemmArgs g{a1, idx1, lda1, K1, a2, lda2, K2, w, bias, c, ldc, M, nullptr, Nn, act};
-        k_gemm_f32<<<dim3((unsigned)((M + 63) / 64), (unsigned)((Nn + 63) / 64)), 256, 0, st>>>(g);
-        g_launches++;
-    };
-    // reference state_dict order (policy_weights.weight_spec)
-    const float *W_iou = wts[0], *b_iou = wts[1], *U_iou = wts[2], *W_c = wts[3], *b_c = wts[4], *W_f = wts[5], *b_f = wts[6], *U_f = wts[7];
-    // ---- Tree-LSTM (TreeLSTM.py:34-154) ----
-    const long long nodes = T * f32path::NODES;
-    cudaMemsetAsync(ws.h, 0, (size_t)nodes * T_H * 4, st);
-    cudaMemsetAsync(ws.c, 0, (size_t)nodes * T_H * 4, st);
-    cudaMemsetAsync(ws.counts, 0, 64 * 4, st);
-    k_tree_lists<<<(unsigned)((T + 127) / 128), 128, 0, st>>>(d_adjacency, d_node_order, T, ws.child_base, ws.lists, ws.counts, ws.cap);
-    k_tree_leaves<<<(unsigned)nodes, 128, 0, st>>>(d_forest, d_node_order, nodes, W_iou, b_iou, ws.h, ws.c);
-    g_launches += 2;
-    int32_t counts[MAX_LEVELS];
-    cudaError_t err = cudaMemcpyAsync(counts, ws.counts, sizeof(counts), cudaMemcpyDeviceToHost, st);
-    if (err == cudaSuccess) err = cudaStreamSynchronize(st);        // per-level sizes of the launches below (the fp32 path is not the fast path)
-    if (err != cudaSuccess) return (int)err;
-    for (int lv = 1; lv < MAX_LEVELS; lv++) {
-        const long long M = counts[lv];
-        if (M <= 0) continue;
-        if (M > ws.cap) return -1;
-        const int32_t *list = ws.lists + (long long)lv * ws.cap, *dM = ws.counts + lv;
-        k_level_rows<<<(unsigned)((M + 127) / 128), 128, 0, st>>>(list, dM, ws.child_base, ws.merge_row, ws.child_row);
-        g_launches++;
-        gemm(ws.h, ws.merge_row, T_H, 3 * T_H, nullptr, 0, 0, U_iou, nullptr, ws.iou, 3 * T_H, M, 3 * T_H, 0);          // U_iou [h_c0 | h_c1 | h_c2]
-        gemm(ws.h, ws.child_row, T_H, T_H, nullptr, 0, 0, U_f, nullptr, ws.fraw, T_H, 3 * M, T_H, 0);                    // U_f h_child
-        k_forget<<<(unsigned)M, 384, 0, st>>>(ws.fraw, list, ws.child_row, dM, d_forest, W_f, b_f, ws.c, ws.fc);
-        gemm(ws.fc, nullptr, 3 * T_H, 3 * T_H, nullptr, 0, 0, W_c, nullptr, ws.craw, T_H, M, T_H, 0);                    // W_c [f c]_merge
-        k_inner<<<(unsigned)M, 128, 0, st>>>(ws.iou, ws.craw, list, dM, d_forest, W_iou, b_iou, b_c, ws.h, ws.c);
-        g_launches += 2;
-    }
-    // ---- attribute MLP (net_tree.py:41-50), emb = cat(attr embedding, h of the root) ----
-    gemm(d_agent_attr, nullptr, 83, 83, nullptr, 0, 0, wts[8], wts[9], ws.a0, 256, T, 256, 1);
-    gemm(ws.a0, nullptr, 256, 256, nullptr, 0, 0, wts[10], wts[11], ws.a1, 256, T, 256, 1);
-    gemm(ws.a1, nullptr, 256, 256, nullptr, 0, 0, wts[12], wts[13], ws.a0, 256, T, 256, 1);
-    gemm(ws.a0, nullptr, 256, 256, nullptr, 0, 0, wts[14], wts[15], ws.emb, 256, T, 128, 1);
-    k_copy_cols<<<(unsigned)((T * 128 + 255) / 256), 256, 0, st>>>(ws.h, (long long)f32path::NODES * T_H, ws.emb + 128, 256, T, 128);
-    g_launches++;
-    // ---- three attention blocks (net_tree.py:20-32) ----
-    const float *x = ws.emb;
-    float *outs[3] = {ws.x0, ws.x1, ws.x0};
-    for (int l = 0; l < 3; l++) {
-        const float *const *tw = wts + 16 + 6 * l;
-        gemm(x, nullptr, 256, 256, nullptr, 0, 0, tw[0], tw[1], ws.qkv, 768, T, 768, 0);
-        k_attention<<<(unsigned)((T * 4 * 32 + 255) / 256), 256, 0, st>>>(ws.qkv, ws.y1, 256, E, (int)N, nullptr);              // heads -> y1 [T][256]
-        g_launches++;
-        gemm(ws.y1, nullptr, 256, 256, nullptr, 0, 0, tw[2], tw[3], ws.cat + 256, 512, T, 256, 0);                         // out_proj -> cat[:, 256:]
-        k_copy_cols<<<(unsigned)((T * 256 + 255) / 256), 256, 0, st>>>(x, 256, ws.cat, 512, T, 256);                   // cat[:, :256] = input
-        g_launches++;
-        gemm(ws.cat, nullptr, 512, 512, nullptr, 0, 0, tw[4], tw[5], outs[l], 256, T, 256, 1);
-        x = outs[l];
-    }
-    // ---- heads on cat(emb, att) (net_tree.py:56-71, 100-110) ----
-    const float *const *aw = wts + 34, *const *cw = wts + 40;
-    gemm(ws.emb, nullptr, 256, 256, x, 256, 256, aw[0], aw[1], ws.y1, 256, T, 256, 1);
-    gemm(ws.y1, nullptr, 256, 256, nullptr, 0, 0, aw[2], aw[3], ws.y2a, 128, T, 128, 1);
-    gemm(ws.emb, nullptr, 256, 256, x, 256, 256, cw[0], cw[1], ws.y1, 256, T, 256, 1);
-    gemm(ws.y1, nullptr, 256, 256, nullptr, 0, 0, cw[2], cw[3], ws.y2c, 128, T, 128, 1);
-    k_heads_final<<<(unsigned)E, 256, (size_t)N * sizeof(float), st>>>(ws.y2a, ws.y2c, aw[4], aw[5], cw[4], cw[5], d_logits, d_value, (int)N);
-    g_launches++;
-    return (int)cudaGetLastError();
+    const ppograph::PpoIn in{d_agent_attr, d_forest, d_adjacency, d_node_order, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+                             0.0f, 0.0f, 0.0f, nullptr, d_logits, d_value, nullptr, nullptr};
+    f32grad::Wg ws;
+    if (ppograph::check_obs(wts, d_workspace, workspace_bytes, E, N, in, ws, false)) return -1;
+    ppograph::F32Lin lin{(cudaStream_t)stream, ws.part};
+    return ppograph::run(lin, wts, ws, E, N, in, false, (cudaStream_t)stream);
 }
 
 // ---- PPO loss and gradients of the fp32 network (policy_f32_grad.cuh) ------------------------------------------------
 size_t fl_policy_workspace_bytes_grad_f32(int64_t n_agents_total) {
     if (n_agents_total <= 0) return 0;
     f32grad::Wg w;
-    return f32grad::carve(w, nullptr, n_agents_total);
+    return f32grad::carve(w, nullptr, n_agents_total, true);
 }
 
 // fl_policy_ppo_grad_{f32,bf16} are the shard path fed from the workspace's own count (gcnt null)
@@ -1874,8 +1827,7 @@ int fl_policy_ppo_grad_bf16(const float *const *wts, void *d_workspace, size_t w
 // ---- one shard of a data-parallel minibatch: the counts of its rows, and the loss divided by the minibatch's counts ------
 int fl_policy_ppo_counts(int64_t E, int64_t N, const uint8_t *d_valid_actions, const uint8_t *d_acted, int64_t *d_counts,
                          void *stream) {
-    if (E <= 0 || N <= 0 || !d_valid_actions || !d_acted || !d_counts) return -1;
-    if (N > (1ll << 31) / f32path::NODES || E > ((1ll << 31) / f32path::NODES) / N) return -1;      // as fl_policy_ppo_grad_f32
+    if (ppograph::bad_shape(E, N) || !d_valid_actions || !d_acted || !d_counts) return -1;      // as fl_policy_ppo_grad_f32
     const cudaStream_t st = (cudaStream_t)stream;
     const cudaError_t err = cudaMemsetAsync(d_counts, 0, 2 * sizeof(int64_t), st);
     if (err != cudaSuccess) return (int)err;
@@ -1919,16 +1871,12 @@ int fl_policy_ppo_grad_shard_bf16(const float *const *wts, void *d_workspace, si
 int fl_policy_forward_train_bf16(const float *const *wts, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
                                  const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
                                  const int32_t *d_node_order, float *d_logits, float *d_value, void *stream) {
-    if (!wts || !d_workspace || E <= 0 || N <= 0 || !d_agent_attr || !d_forest || !d_adjacency || !d_node_order || !d_logits || !d_value) return -1;
-    if (N > (1ll << 31) / f32path::NODES || E > ((1ll << 31) / f32path::NODES) / N) return -1;
-    for (int i = 0; i < FL_POLICY_F32_TENSORS; i++)
-        if (!wts[i]) return -1;
-    f32grad::Wg ws;
-    if (f32grad::carve(ws, (unsigned char *)d_workspace, E * N) > workspace_bytes) return -1;
-    const int rc = ppograph::bf16_setup();
-    if (rc) return rc;
     const ppograph::PpoIn in{d_agent_attr, d_forest, d_adjacency, d_node_order, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
                              0.0f, 0.0f, 0.0f, nullptr, d_logits, d_value, nullptr, nullptr};
+    f32grad::Wg ws;      // the training layout: the header gives this call fl_policy_workspace_bytes_grad_bf16's workspace
+    if (ppograph::check_obs(wts, d_workspace, workspace_bytes, E, N, in, ws, true)) return -1;
+    const int rc = ppograph::bf16_setup();
+    if (rc) return rc;
     ppograph::Bf16Lin lin{(cudaStream_t)stream, ws.part};
     return ppograph::run(lin, wts, ws, E, N, in, false, (cudaStream_t)stream);
 }

@@ -9,8 +9,10 @@
 // callers that need the reference's numbers, and as the yardstick of the bf16 path.
 //
 // Structure: one tiled SGEMM kernel (64 x 64 x 16 tiles, 4 x 4 outputs per thread, gathered rows, two concatenated A
-// sources) for every matrix product; the Tree-LSTM runs level by level over per-level node lists built on the device,
-// with small element-wise kernels for the gates (TreeLSTM.py:59-154); attention is one warp per (query, head).
+// sources) for every matrix product; the Tree-LSTM runs level by level over per-level node lists built on the device
+// (k_tl_*, policy_f32_grad.cuh), with small element-wise kernels for the gates (TreeLSTM.py:59-154); attention is one warp
+// per (query, head).  The kernels are launched by ppograph::run (policy.cu), the one launch sequence of this forward and of
+// the training forward.
 #pragma once
 #include <cuda_runtime.h>
 #include <math.h>
@@ -91,28 +93,6 @@ __global__ void __launch_bounds__(256) k_gemm_f32(GemmArgs g) {
 
 // ---- Tree-LSTM --------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ float clean(float f) { return (isinf(f) && f > 0.0f) ? -1.0f : f; }   // eval_env.py:76
-
-// per tree: index of the first child of every node (adjacency rows of one parent are consecutive, child of row r is r + 1:
-// TreeLSTM.py:118-119), and the per-level lists of inner nodes (node_order >= 1)
-__global__ void k_tree_lists(const int32_t *__restrict__ adj, const int32_t *__restrict__ node_order, long long n_trees,
-                             int8_t *__restrict__ child_base, int32_t *__restrict__ lists, int32_t *__restrict__ counts, long long cap) {
-    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= n_trees) return;
-    int8_t cb[NODES];
-    for (int n = 0; n < NODES; n++) cb[n] = -1;
-    for (int r = NODES - 2; r >= 0; r--) {
-        const int p = adj[(t * (NODES - 1) + r) * 3];
-        if (p >= 0 && p < NODES) cb[p] = (int8_t)(r + 1);    // descending r: ends on the first row of the parent
-    }
-    for (int n = 0; n < NODES; n++) {
-        child_base[t * NODES + n] = cb[n];
-        const int lv = node_order[t * NODES + n];
-        if (lv >= 1 && lv < MAX_LEVELS) {
-            const int pos = atomicAdd(&counts[lv], 1);
-            if (pos < cap) lists[(long long)lv * cap + pos] = (int32_t)(t * NODES + n);
-        }
-    }
-}
 
 // leaves (node_order == 0): iou = W_iou x + b; c = sigmoid(i) tanh(u); h = sigmoid(o) tanh(c)   (TreeLSTM.py:96-111 with no children)
 __global__ void k_tree_leaves(const float *__restrict__ forest, const int32_t *__restrict__ node_order, long long n_nodes,
@@ -254,27 +234,6 @@ __global__ void k_heads_final(const float *__restrict__ ya, const float *__restr
         for (int a = 0; a < N; a++) s += sv[a];
         value[env] = s / (float)N;
     }
-}
-
-struct Ws {   // carved out of the caller's workspace
-    float *h, *c, *iou, *fraw, *fc, *craw, *a0, *a1, *emb, *qkv, *cat, *x0, *x1, *y1, *y2a, *y2c, *zc;
-    int8_t *child_base; int32_t *lists, *counts, *merge_row, *child_row;
-    long long cap;
-};
-
-inline size_t carve(Ws &w, unsigned char *base, long long T) {
-    size_t off = 0;
-    auto take = [&](size_t bytes) { unsigned char *p = base ? base + off : nullptr; off = (off + bytes + 255) & ~(size_t)255; return p; };
-    const long long nodes = T * NODES, cap = T * 10;          // at most 10 inner nodes per 31-node ternary tree
-    w.cap = cap;
-    w.h = (float *)take(nodes * T_H * 4); w.c = (float *)take(nodes * T_H * 4);
-    w.iou = (float *)take(cap * 384 * 4); w.fraw = (float *)take(cap * 384 * 4); w.fc = (float *)take(cap * 384 * 4); w.craw = (float *)take(cap * 128 * 4);
-    w.a0 = (float *)take(T * 256 * 4); w.a1 = (float *)take(T * 256 * 4); w.emb = (float *)take(T * 256 * 4);
-    w.qkv = (float *)take(T * 768 * 4); w.cat = (float *)take(T * 512 * 4); w.x0 = (float *)take(T * 256 * 4); w.x1 = (float *)take(T * 256 * 4);
-    w.y1 = (float *)take(T * 256 * 4); w.y2a = (float *)take(T * 128 * 4); w.y2c = (float *)take(T * 128 * 4); w.zc = (float *)take(T * 512 * 4);
-    w.child_base = (int8_t *)take(nodes); w.lists = (int32_t *)take(MAX_LEVELS * cap * 4); w.counts = (int32_t *)take(64 * 4);
-    w.merge_row = (int32_t *)take(cap * 4); w.child_row = (int32_t *)take(cap * 3 * 4);
-    return off;
 }
 
 }  // namespace f32path

@@ -1,10 +1,11 @@
 // policy_f32_grad.cuh — the PPO loss of the fp32 network and its gradients with respect to every parameter
 // (fl_policy_ppo_grad_f32, include/flatland_policy_b200.h).  Everything runs in fp32 on the CUDA cores.
 //
-// Training forward: the kernels of policy_f32.cuh with the arithmetic of fl_policy_forward_f32, so that logits and values
-// are bit-identical to it, but every level and layer writes its own slice of the workspace and the GEMMs also store their
-// pre-activations (GemmArgs::pre), attention its log-sum-exp per (agent, head).  The level lists are built in a fixed order
-// (tree order, then node order; k_tl_*) instead of by atomics, because the weight gradients reduce over their rows.
+// Training forward: the kernels of policy_f32.cuh launched by ppograph::run (policy.cu), which is also fl_policy_forward_f32,
+// so logits and values are bit-identical to it.  For training every level and layer writes its own slice of the workspace,
+// the GEMMs also store their pre-activations (GemmArgs::pre) and attention its log-sum-exp per (agent, head); the forward
+// alone carves a smaller layout without them (carve, train = false).  The level lists are built in a fixed order (tree
+// order, then node order; k_tl_*) with no atomics, because the weight gradients reduce over their rows.
 //
 // Loss: k_ppo_count (|S| and the number of acted rows; int64 integer atomics, exact in any order and across shards),
 // k_ppo_loss (one CTA per environment row: log pi with masked_choice's arithmetic, clipped surrogate, entropy, value term,
@@ -33,7 +34,8 @@ __device__ __forceinline__ float gelu_grad(float x) {
 }
 
 // ---- level lists in a fixed order --------------------------------------------------------------------------------------
-// per tree: first child of every node (as k_tree_lists) and the number of nodes of every level 0..10 -> tcnt[lv][t]
+// per tree: first child of every node (adjacency rows of one parent are consecutive, child of row r is r + 1:
+// TreeLSTM.py:118-119) and the number of nodes of every level 0..10 -> tcnt[lv][t]
 __global__ void k_tl_count(const int32_t *__restrict__ adj, const int32_t *__restrict__ node_order, long long T,
                            int8_t *__restrict__ child_base, int32_t *__restrict__ tcnt) {
     const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -42,7 +44,7 @@ __global__ void k_tl_count(const int32_t *__restrict__ adj, const int32_t *__res
     for (int n = 0; n < f32path::NODES; n++) cb[n] = -1;
     for (int r = f32path::NODES - 2; r >= 0; r--) {
         const int p = adj[(t * (f32path::NODES - 1) + r) * 3];
-        if (p >= 0 && p < f32path::NODES) cb[p] = (int8_t)(r + 1);
+        if (p >= 0 && p < f32path::NODES) cb[p] = (int8_t)(r + 1);    // descending r: ends on the first row of the parent
     }
     int cnt[MAX_LEVELS];
     for (int l = 0; l < MAX_LEVELS; l++) cnt[l] = 0;
@@ -529,27 +531,43 @@ inline int n_chunks(long long M) {
     return (int)(n < MAX_CHUNKS ? n : MAX_CHUNKS);
 }
 
-inline size_t carve(Wg &w, unsigned char *base, long long T) {
+// train: the training forward, the loss and the backward.  Otherwise the forward alone (fl_policy_forward_f32): the
+// pointers only the backward reads (xcl, ap, mpre, lse, y1p, y2p, d*, part) stay null, and a dense buffer is shared once
+// the forward has read it for the last time (aa[2] = aa[0]; one qkv, att and cat for the three layers; xs ping-pongs; one
+// y1 for both heads; y2 stays per head, k_heads_final reads both).
+inline size_t carve(Wg &w, unsigned char *base, long long T, bool train) {
+    w = Wg{};
     size_t off = 0;
     auto take = [&](size_t bytes) { unsigned char *p = base ? base + off : nullptr; off = (off + bytes + 255) & ~(size_t)255; return p; };
     auto f = [&](long long n) { return (float *)take((size_t)n * 4); };
-    const long long nodes = T * f32path::NODES, cap = T * 10;
+    const long long nodes = T * f32path::NODES, cap = T * 10;     // at most 10 inner nodes per 31-node ternary tree
     w.cap = cap;
     w.nblk = (int)((T + SCAN - 1) / SCAN);
-    w.h = f(nodes * T_H); w.c = f(nodes * T_H); w.xcl = f(nodes * NF);
+    w.h = f(nodes * T_H); w.c = f(nodes * T_H);
+    if (train) w.xcl = f(nodes * NF);
     w.iou = f(cap * 384); w.fraw = f(cap * 384); w.fc = f(cap * 384); w.craw = f(cap * 128);
     w.child_base = (int8_t *)take(nodes);
     w.tcnt = (int32_t *)take(MAX_LEVELS * T * 4); w.tpos = (int32_t *)take(MAX_LEVELS * T * 4);
     w.btot = (int32_t *)take((size_t)MAX_LEVELS * w.nblk * 4); w.counts = (int32_t *)take(64 * 4);
     w.lists = (int32_t *)take(nodes * 4); w.merge_row = (int32_t *)take(cap * 4); w.child_row = (int32_t *)take(cap * 3 * 4);
-    for (int i = 0; i < 4; i++) w.ap[i] = f(T * 256);
-    for (int i = 0; i < 3; i++) w.aa[i] = f(T * 256);
+    if (train)
+        for (int i = 0; i < 4; i++) w.ap[i] = f(T * 256);
+    for (int i = 0; i < 3; i++) w.aa[i] = train || i < 2 ? f(T * 256) : w.aa[0];
     w.emb = f(T * 256);
     for (int l = 0; l < 3; l++) {
-        w.qkv[l] = f(T * 768); w.att[l] = f(T * 256); w.cat[l] = f(T * 512); w.mpre[l] = f(T * 256); w.xs[l] = f(T * 256);
-        w.lse[l] = f(T * 4);
+        const bool own = train || l == 0;
+        w.qkv[l] = own ? f(T * 768) : w.qkv[0]; w.att[l] = own ? f(T * 256) : w.att[0]; w.cat[l] = own ? f(T * 512) : w.cat[0];
+        if (train) w.mpre[l] = f(T * 256);
+        w.xs[l] = train || l < 2 ? f(T * 256) : w.xs[0];
+        if (train) w.lse[l] = f(T * 4);
     }
-    for (int h = 0; h < 2; h++) { w.y1p[h] = f(T * 256); w.y1[h] = f(T * 256); w.y2p[h] = f(T * 128); w.y2[h] = f(T * 128); }
+    for (int h = 0; h < 2; h++) {
+        if (train) w.y1p[h] = f(T * 256);
+        w.y1[h] = train || h == 0 ? f(T * 256) : w.y1[0];
+        if (train) w.y2p[h] = f(T * 128);
+        w.y2[h] = f(T * 128);
+    }
+    if (!train) return off;
     w.dlogits = f(T * 5); w.dcrit = f(T); w.rowstats = f(T * 5);                    // E <= T rows
     w.dz = f(T * 512); w.dy1 = f(T * 256); w.dy2 = f(T * 128); w.dcat = f(T * 512); w.datt = f(T * 256); w.dqkv = f(T * 768);
     w.dx[0] = f(T * 256); w.dx[1] = f(T * 256); w.Dq = f(T * 4);

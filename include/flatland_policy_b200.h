@@ -86,7 +86,10 @@ int fl_policy_forward(const FlPolicyWeights *w, void *d_workspace, size_t worksp
  * pointers to the fp32 tensors of the reference state_dict in its registration order (solution/nn/net_tree.py:33-72,
  * TreeLSTM.py:12-32; flatland-marl_b200/policy_weights.py:weight_spec lists names and shapes).  Logits and values agree with
  * the reference network to summation-order rounding (tests: 1e-4 absolute); about ten times slower than the tensor-core
- * path.  Synchronises `stream` once (per-level node counts). */
+ * path.  It is the training forward of fl_policy_ppo_grad_f32 run on a smaller workspace that keeps no activations for a
+ * backward pass.  Synchronises `stream` once (per-level node counts).  d_workspace: fl_policy_workspace_bytes_f32(E*N)
+ * bytes (0 for n_agents_total <= 0).  FL_ERR_BAD_ARG before any CUDA call for a NULL pointer (also among d_weights), E or
+ * N <= 0, E*N*31 >= 2^31 (node ids are 32-bit) or a workspace that is too small. */
 #define FL_POLICY_F32_TENSORS 46
 size_t fl_policy_workspace_bytes_f32(int64_t n_agents_total);
 int fl_policy_forward_f32(const float *const *d_weights, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
