@@ -19,6 +19,7 @@
 //   k_tree_leaf   leaves of the Tree-LSTM (K = 12: one MMA k-step), two 192-column accumulators, 16 epilogue warps.
 //   k_prep / k_tree_plan / k_head_final / k_choose: casts, level lists, final 128->5/1 layers, action choice.
 //   rollout.cuh: seeded sampling with log-probabilities (k_sample) and GAE (k_gae) for PPO rollouts.
+#include <cmath>
 #include <cstdlib>
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -1418,6 +1419,9 @@ struct PpoIn {
     float eps, vf, ent;
     float *const *grads; float *logits, *value, *stats;
     const long long *gcnt;   // the loss's denominators [|S|, acted rows] over the whole minibatch; null: these rows' own counts
+    // FlPpoOptions (all off by default); gmom: [sum_S A, sum_S A^2] of the whole minibatch, null: these rows' own moments
+    const float *old_values = nullptr; const double *gmom = nullptr;
+    float vf_clip = 0.0f, adv_eps = 0.0f; int norm_adv = 0;
 };
 
 // The forward pass and, when `loss`, the PPO loss and the backward pass.  On F32Lin with the forward-only layout
@@ -1507,13 +1511,21 @@ int run(Lin &lin, const float *const *wts, Wg &ws, long long E, long long N, con
     if (!loss) return (int)cudaGetLastError();
 
     // ==== PPO loss: d loss / d logits, d loss / d critic output, statistics ====
-    // these rows' counts go to words 32..35 of ws.counts (zeroed above); one shard of a minibatch divides by the minibatch's
+    // these rows' counts go to words 32..35 of ws.counts (zeroed above), their advantage moments to words 36..39; one shard
+    // of a minibatch divides by the minibatch's counts and normalises by its moments
     unsigned long long *cnt = reinterpret_cast<unsigned long long *>(ws.counts + 32);
+    double *mom = reinterpret_cast<double *>(ws.counts + 36);
     const long long *gcnt = in.gcnt ? in.gcnt : reinterpret_cast<const long long *>(cnt);
     PpoArgs pa{in.logits, in.value, in.old_lp, in.adv, in.ret, in.valid, in.actions, in.acted, E, (int)N, in.eps, in.vf, in.ent,
-               cnt, ws.dlogits, ws.dcrit, ws.rowstats, gcnt};
+               cnt, ws.dlogits, ws.dcrit, ws.rowstats, gcnt, in.old_values, in.gmom ? in.gmom : mom, in.vf_clip, in.adv_eps,
+               in.norm_adv};
     k_ppo_count<<<(unsigned)E, 128, 0, st>>>(pa);
-    k_ppo_loss<<<(unsigned)E, 128, 0, st>>>(pa);
+    if (in.norm_adv && !in.gmom) {
+        k_ppo_moments<<<1, 1024, 0, st>>>(pa, mom);
+        g_launches++;
+    }
+    if (in.norm_adv || in.vf_clip > 0.0f) k_ppo_loss<true><<<(unsigned)E, 128, 0, st>>>(pa);
+    else k_ppo_loss<false><<<(unsigned)E, 128, 0, st>>>(pa);
     k_ppo_stats<<<1, 256, 0, st>>>(ws.rowstats, E, cnt, gcnt, in.vf, in.ent, in.stats);
     g_launches += 3;
 
@@ -1614,6 +1626,8 @@ int check_args(const float *const *wts, void *d_workspace, size_t workspace_byte
                const FlPpoParams *params, Wg &ws) {
     if (!in.grads || !params || !in.valid || !in.actions || !in.old_lp || !in.adv || !in.ret || !in.acted || !in.stats) return -1;
     if (!(params->clip_eps > 0.0f)) return -1;
+    if (!(in.vf_clip >= 0.0f) || (in.norm_adv != 0 && in.norm_adv != 1) || !(in.adv_eps >= 0.0f) || !std::isfinite(in.adv_eps)) return -1;
+    if ((in.vf_clip > 0.0f && !in.old_values) || (in.gmom && !in.gcnt)) return -1;
     for (int i = 0; i < FL_POLICY_F32_TENSORS; i++)
         if (!in.grads[i]) return -1;
     return check_obs(wts, d_workspace, workspace_bytes, E, N, in, ws, true);
@@ -1776,17 +1790,26 @@ size_t fl_policy_workspace_bytes_grad_f32(int64_t n_agents_total) {
     return f32grad::carve(w, nullptr, n_agents_total, true);
 }
 
-// fl_policy_ppo_grad_{f32,bf16} are the shard path fed from the workspace's own count (gcnt null)
+// The one PPO path: fl_policy_ppo_grad_{f32,bf16} are it with the counts taken from the workspace (gcnt null) and the
+// options off, fl_policy_ppo_grad_shard_* with the options off, fl_policy_ppo_grad_ex_* as given
 static int ppo_grad(bool bf16, const int64_t *gcnt, const float *const *wts, void *d_workspace, size_t workspace_bytes,
                     int64_t E, int64_t N, const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
                     const int32_t *d_node_order, const uint8_t *d_valid_actions, const uint8_t *d_actions,
                     const float *d_old_log_probs, const float *d_advantages, const float *d_returns, const uint8_t *d_acted,
                     const FlPpoParams *params, float *const *d_grads, float *d_logits, float *d_value, float *d_stats,
-                    void *stream) {
-    const ppograph::PpoIn in{d_agent_attr, d_forest, d_adjacency, d_node_order, d_valid_actions, d_actions, d_old_log_probs, d_advantages,
-                             d_returns, d_acted, params ? params->clip_eps : 0.0f, params ? params->vf_coef : 0.0f,
-                             params ? params->ent_coef : 0.0f, d_grads, d_logits, d_value, d_stats,
-                             reinterpret_cast<const long long *>(gcnt)};
+                    void *stream, const float *d_old_values = nullptr, const double *gmom = nullptr,
+                    const FlPpoOptions *opts = nullptr) {
+    ppograph::PpoIn in{d_agent_attr, d_forest, d_adjacency, d_node_order, d_valid_actions, d_actions, d_old_log_probs, d_advantages,
+                       d_returns, d_acted, params ? params->clip_eps : 0.0f, params ? params->vf_coef : 0.0f,
+                       params ? params->ent_coef : 0.0f, d_grads, d_logits, d_value, d_stats,
+                       reinterpret_cast<const long long *>(gcnt)};
+    in.old_values = d_old_values;
+    in.gmom = gmom;
+    if (opts) {
+        in.vf_clip = opts->vf_clip;
+        in.norm_adv = opts->norm_adv;
+        in.adv_eps = opts->adv_eps;
+    }
     f32grad::Wg ws;
     if (ppograph::check_args(wts, d_workspace, workspace_bytes, E, N, in, params, ws)) return -1;
     if (!bf16) {
@@ -1866,6 +1889,47 @@ int fl_policy_ppo_grad_shard_bf16(const float *const *wts, void *d_workspace, si
     return ppo_grad(true, d_global_counts, wts, d_workspace, workspace_bytes, E, N, d_agent_attr, d_forest, d_adjacency, d_node_order,
                     d_valid_actions, d_actions, d_old_log_probs, d_advantages, d_returns, d_acted, params, d_grads, d_logits, d_value,
                     d_stats, stream);
+}
+
+// ---- options of the loss: the minibatch's advantage moments, and the PPO path with clipped value loss / normalisation ----
+int fl_policy_ppo_moments(int64_t E, int64_t N, const uint8_t *d_valid_actions, const uint8_t *d_acted, const float *d_advantages,
+                          double *d_moments, void *stream) {
+    if (ppograph::bad_shape(E, N) || !d_valid_actions || !d_acted || !d_advantages || !d_moments) return -1;
+    f32grad::PpoArgs pa{};
+    pa.valid = d_valid_actions;
+    pa.acted = d_acted;
+    pa.adv = d_advantages;
+    pa.E = E;
+    pa.N = (int)N;
+    f32grad::k_ppo_moments<<<1, 1024, 0, (cudaStream_t)stream>>>(pa, d_moments);
+    g_launches++;
+    return (int)cudaGetLastError();
+}
+
+int fl_policy_ppo_grad_ex_f32(const float *const *wts, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
+                              const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
+                              const int32_t *d_node_order, const uint8_t *d_valid_actions, const uint8_t *d_actions,
+                              const float *d_old_log_probs, const float *d_advantages, const float *d_returns, const uint8_t *d_acted,
+                              const int64_t *d_global_counts,
+                              const FlPpoParams *params, float *const *d_grads, float *d_logits, float *d_value, float *d_stats,
+                              void *stream, const float *d_old_values, const double *d_global_moments, const FlPpoOptions *opts) {
+    if (!opts) return -1;
+    return ppo_grad(false, d_global_counts, wts, d_workspace, workspace_bytes, E, N, d_agent_attr, d_forest, d_adjacency, d_node_order,
+                    d_valid_actions, d_actions, d_old_log_probs, d_advantages, d_returns, d_acted, params, d_grads, d_logits, d_value,
+                    d_stats, stream, d_old_values, d_global_moments, opts);
+}
+
+int fl_policy_ppo_grad_ex_bf16(const float *const *wts, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
+                               const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
+                               const int32_t *d_node_order, const uint8_t *d_valid_actions, const uint8_t *d_actions,
+                               const float *d_old_log_probs, const float *d_advantages, const float *d_returns, const uint8_t *d_acted,
+                               const int64_t *d_global_counts,
+                               const FlPpoParams *params, float *const *d_grads, float *d_logits, float *d_value, float *d_stats,
+                               void *stream, const float *d_old_values, const double *d_global_moments, const FlPpoOptions *opts) {
+    if (!opts) return -1;
+    return ppo_grad(true, d_global_counts, wts, d_workspace, workspace_bytes, E, N, d_agent_attr, d_forest, d_adjacency, d_node_order,
+                    d_valid_actions, d_actions, d_old_log_probs, d_advantages, d_returns, d_acted, params, d_grads, d_logits, d_value,
+                    d_stats, stream, d_old_values, d_global_moments, opts);
 }
 
 int fl_policy_forward_train_bf16(const float *const *wts, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,

@@ -11,7 +11,10 @@
 // k_ppo_loss (one CTA per environment row: log pi with masked_choice's arithmetic, clipped surrogate, entropy, value term,
 // d loss / d logits and d loss / d critic output), k_ppo_stats (one CTA, fixed-order reduction of the per-row sums).  The
 // loss and the statistics divide by the denominators in PpoArgs::gcnt: the call's own counts, or the counts of the whole
-// minibatch when the rows are one shard of it (fl_policy_ppo_grad_shard_*).
+// minibatch when the rows are one shard of it (fl_policy_ppo_grad_shard_*).  The loss options (FlPpoOptions,
+// fl_policy_ppo_grad_ex_*) run in k_ppo_loss<true>: advantages normalised by the float64 moments in PpoArgs::gmom (the
+// minibatch's, or these rows' from k_ppo_moments, one CTA in a fixed order) and the clipped value term; k_ppo_loss<false> is
+// the plain loss.
 //
 // Backward: k_gemm_dx (dX = dY W, optional gathered output rows, added term, accumulation and GELU' epilogue), k_gemm_dw +
 // k_dw_reduce (dW = dY^T X and db over fixed row chunks into partial buffers, then summed in chunk order), k_attn_bwd_q /
@@ -398,6 +401,10 @@ struct PpoArgs {
     unsigned long long *cnt;            // [0] |S|, [1] acted rows of these rows (k_ppo_count; zeroed before it)
     float *dlogits, *dcrit, *rowstats;  // [T][5], [T], [E][5]
     const long long *gcnt;              // the denominators: [0] |S|, [1] acted rows of the whole minibatch (cnt for one shard)
+    // options (k_ppo_loss<true> only): vf_clip > 0 clips the value term around old_values [E]; norm_adv normalises A by the
+    // minibatch moments gmom = [sum_S A, sum_S A^2] (float64) with the denominator sigma + adv_eps
+    const float *old_values; const double *gmom;
+    float vf_clip, adv_eps; int norm_adv;
 };
 
 __device__ __forceinline__ int block_sum_i(int v, int *sh) {
@@ -426,15 +433,63 @@ __global__ void k_ppo_count(PpoArgs p) {
     }
 }
 
+// one CTA (1024 threads): out = [sum_S A, sum_S A^2] in float64, each acted row's A counted once per agent of S.  Warp w takes
+// rows w, w + 32, ... in order (|S| of a row: an integer warp sum), then thread 0 adds the 32 warp sums in warp order: the
+// same bytes for the same inputs.
+__global__ void __launch_bounds__(1024) k_ppo_moments(PpoArgs p, double *__restrict__ out) {
+    __shared__ double sh[2][32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    double s1 = 0.0, s2 = 0.0;
+    for (long long e = warp; e < p.E; e += 32) {
+        if (!p.acted[e]) continue;
+        int n = 0;
+        for (int i = lane; i < p.N; i += 32) {
+            const uint8_t *v = p.valid + (e * p.N + i) * 5;
+            n += (v[0] | v[1] | v[2] | v[3] | v[4]) ? 1 : 0;
+        }
+        for (int d = 16; d > 0; d >>= 1) n += __shfl_xor_sync(0xFFFFFFFFu, n, d);
+        const double a = (double)p.adv[e];
+        s1 += (double)n * a;
+        s2 += (double)n * (a * a);
+    }
+    if (lane == 0) { sh[0][warp] = s1; sh[1][warp] = s2; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double t1 = 0.0, t2 = 0.0;
+        for (int w = 0; w < 32; w++) { t1 += sh[0][w]; t2 += sh[1][w]; }
+        out[0] = t1;
+        out[1] = t2;
+    }
+}
+
 // one CTA (128 threads) per environment row; rowstats[e] = sums over the row's agents in S of (policy term, entropy,
-// logp_old - logp_new, |r - 1| > eps) and the value term (V - R)^2 (0 for rows with acted = 0)
+// logp_old - logp_new, |r - 1| > eps) and the value term (V - R)^2 (0 for rows with acted = 0).  OPT (PpoArgs options):
+// A is normalised by the minibatch moments and the value term is max((V - R)^2, (V_clip - R)^2); without it the kernel is
+// the plain loss, arithmetic unchanged.
+template <bool OPT>
 __global__ void __launch_bounds__(128) k_ppo_loss(PpoArgs p) {
     __shared__ float sh[4][128];
     const long long e = blockIdx.x;
     const long long nS = p.gcnt[0], nR = p.gcnt[1];
     const bool acted = p.acted[e] != 0;
     const float invS = nS > 0 ? 1.0f / (float)nS : 0.0f;
-    const float A = p.adv[e], dV = (acted && nR > 0) ? p.vf * 2.0f * (p.value[e] - p.ret[e]) / (float)nR : 0.0f;
+    float A = p.adv[e], dV = (acted && nR > 0) ? p.vf * 2.0f * (p.value[e] - p.ret[e]) / (float)nR : 0.0f;
+    float vterm = (p.value[e] - p.ret[e]) * (p.value[e] - p.ret[e]);
+    if (OPT) {
+        if (p.norm_adv) {   // (A - mu) / (sigma + adv_eps) in float64, sigma the unbiased deviation over S; 0 when that is 0
+            const double n = (double)nS, s = p.gmom[0], q = p.gmom[1];
+            const double mu = nS > 0 ? s / n : 0.0;
+            const double var = nS > 1 ? fmax(0.0, (q - s * s / n) / (n - 1.0)) : 0.0;
+            const double den = sqrt(var) + (double)p.adv_eps;
+            A = den > 0.0 ? (float)(((double)A - mu) / den) : 0.0f;
+        }
+        if (p.vf_clip > 0.0f) {   // V_clip = V_old + clip(V - V_old, -c, c); the unclipped square wins ties (dV as above)
+            const float V = p.value[e], R = p.ret[e], Vo = p.old_values[e], c = p.vf_clip, dvo = V - Vo;
+            const float Vc = dvo > c ? Vo + c : (dvo < -c ? Vo - c : V);
+            const float uc = (Vc - R) * (Vc - R);
+            if (uc > vterm) { vterm = uc; dV = 0.0f; }
+        }
+    }
     float acc[4] = {0.0f, 0.0f, 0.0f, 0.0f};
     for (int i = threadIdx.x; i < p.N; i += blockDim.x) {
         const long long t = e * p.N + i;
@@ -477,8 +532,7 @@ __global__ void __launch_bounds__(128) k_ppo_loss(PpoArgs p) {
     }
     if (threadIdx.x == 0) {
         for (int q = 0; q < 4; q++) p.rowstats[e * 5 + q] = sh[q][0];
-        const float dv = p.value[e] - p.ret[e];
-        p.rowstats[e * 5 + 4] = acted ? dv * dv : 0.0f;
+        p.rowstats[e * 5 + 4] = acted ? vterm : 0.0f;
     }
 }
 

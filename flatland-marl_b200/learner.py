@@ -12,8 +12,12 @@ DESIGN.md §4.8 for what the two learners trade.
 group= (a torch.distributed process group, NCCL on GPUs) makes the learner data-parallel: every rank passes its own share of
 one minibatch, and ppo_grad leaves on every rank the gradient and the statistics of the whole minibatch (DESIGN.md §4.9,
 INTEGRATION.md §7b).
+
+ppo_grad's vf_clip and norm_adv are the clipped value loss and the advantage normalisation of common PPO implementations,
+computed inside the same call (fl_policy_ppo_grad_ex_*; with a group, over the whole minibatch).
 """
 import ctypes as C
+import math
 from collections import OrderedDict
 
 import torch
@@ -21,7 +25,7 @@ import torch.distributed as dist
 
 from . import policy_weights as pw
 from ._lib import FlatlandB200Error
-from .policy import BatchedActor, FlPpoParams, _check, lib, weights_dict
+from .policy import BatchedActor, FlPpoOptions, FlPpoParams, _check, lib, weights_dict
 
 OBS_KEYS = (("agent_attr", torch.float32, (83,)), ("forest", torch.float32, (31, 12)), ("adjacency", torch.int32, (30, 3)),
             ("node_order", torch.int32, (31,)))
@@ -79,6 +83,7 @@ class PolicyLearner:
             off += p.numel()
         self._stats = self._flat[n:]
         self._counts = torch.zeros(2, dtype=torch.int64, device=self.device)
+        self._moments = torch.zeros(2, dtype=torch.float64, device=self.device)
         with torch.no_grad():
             w = torch.cat([p.detach().reshape(-1) for p in ps])
             dist.broadcast(w, src=dist.get_global_rank(self.group, 0), group=self.group)
@@ -153,19 +158,28 @@ class PolicyLearner:
                   logits.data_ptr(), value.data_ptr(), self._stream()), name)
         return logits, value
 
-    def ppo_grad(self, mb, clip_eps=0.2, vf_coef=0.5, ent_coef=0.01):
+    def ppo_grad(self, mb, clip_eps=0.2, vf_coef=0.5, ent_coef=0.01, vf_clip=0.0, norm_adv=False, adv_eps=1e-8):
         """PPO loss of a minibatch (Rollout.minibatch's dict: the observation tensors, valid_actions, actions, log_probs
-        [E,N,...], advantages, returns, acted [E]) and its gradient, written into every parameter's .grad (allocated when
-        missing, overwritten otherwise).  The loss is stated in include/flatland_policy_b200.h (fl_policy_ppo_grad_f32).
+        [E,N,...], advantages, returns, acted [E], and values [E] when vf_clip > 0) and its gradient, written into every
+        parameter's .grad (allocated when missing, overwritten otherwise).  The loss is stated in include/flatland_policy_b200.h
+        (fl_policy_ppo_grad_f32, and FlPpoOptions for the options).
+
+        vf_clip > 0: the clipped value loss vf_coef mean(max((V - R)^2, (V_clip - R)^2)), V_clip = V_old + clip(V - V_old,
+        -vf_clip, vf_clip), with V_old = mb["values"], the behaviour critic's values.  norm_adv: the advantages normalised
+        over the agents the policy term averages over, (A - mean) / (std + adv_eps), with the mean and the unbiased standard
+        deviation of the whole minibatch (of every rank's share, with a group).  With the defaults (both off) the call writes
+        the bytes it wrote before the options existed.
 
         Returns the statistics as a float32 [8] device tensor (policy loss, value loss, entropy, approximate KL, clip
         fraction, |S|, acted rows, total loss), reused by the next call.  The one host synchronisation is the fp32 path's
         (per-level node counts), in both precisions.
 
         With a group, mb is this rank's share of the minibatch (it may have no rows), and all of this is enqueued on the
-        current stream with no torch-side host synchronisation: fl_policy_ppo_counts of the share, all_reduce of the counts,
-        fl_policy_ppo_grad_shard_* with those counts, all_reduce of the flat gradient and statistics buffer.  Every rank then
-        holds the gradient and the statistics of the whole minibatch, byte-identical across ranks."""
+        current stream with no torch-side host synchronisation: fl_policy_ppo_counts of the share, all_reduce of the counts;
+        with norm_adv, fl_policy_ppo_moments of the share and all_reduce of those float64 sums; fl_policy_ppo_grad_ex_* with
+        the minibatch's counts (and moments), all_reduce of the flat gradient and statistics buffer.  Every rank then holds the
+        gradient and the statistics of the whole minibatch, byte-identical across ranks.  Every rank must pass the same
+        norm_adv: it decides how many collectives the call makes."""
         E, N = self._check_obs(mb, MB_KEYS)
         for name, dt in ROW_KEYS:
             t = mb[name]
@@ -173,8 +187,9 @@ class PolicyLearner:
                 raise ValueError("%s must be a contiguous %s tensor of shape (%d,) on %s" % (name, dt, E, self.device))
         if not clip_eps > 0:
             raise ValueError("clip_eps must be positive")
+        opts = self._options(mb, E, vf_clip, norm_adv, adv_eps)
         if self.group is not None:
-            return self._ppo_grad_shard(mb, E, N, clip_eps, vf_coef, ent_coef)
+            return self._ppo_grad_shard(mb, E, N, clip_eps, vf_coef, ent_coef, opts)
         self._workspace(E, N)
         grads = []
         for p in self._params.values():
@@ -184,13 +199,31 @@ class PolicyLearner:
             grads.append(p.grad)
         logits, value = self._outputs(E, N)
         params = FlPpoParams(float(clip_eps), float(vf_coef), float(ent_coef))
-        fn, name = (self.lib.fl_policy_ppo_grad_bf16, "fl_policy_ppo_grad_bf16") if self.precision == "bf16" else \
-            (self.lib.fl_policy_ppo_grad_f32, "fl_policy_ppo_grad_f32")
-        _check(fn(self._weights(), self._ws.data_ptr(), self._ws.numel(), E, N,
-                  *(mb[k].data_ptr() for k, _, _ in MB_KEYS), *(mb[k].data_ptr() for k, _ in ROW_KEYS),
-                  C.byref(params), self._ptrs(grads), logits.data_ptr(), value.data_ptr(),
-                  self._stats.data_ptr(), self._stream()), name)
+        name = "fl_policy_ppo_grad_ex_bf16" if self.precision == "bf16" else "fl_policy_ppo_grad_ex_f32"
+        _check(getattr(self.lib, name)(self._weights(), self._ws.data_ptr(), self._ws.numel(), E, N,
+                                       *(mb[k].data_ptr() for k, _, _ in MB_KEYS), *(mb[k].data_ptr() for k, _ in ROW_KEYS),
+                                       None, C.byref(params), self._ptrs(grads), logits.data_ptr(), value.data_ptr(),
+                                       self._stats.data_ptr(), self._stream(), opts[1], None, C.byref(opts[0])), name)
         return self._stats
+
+    def _options(self, mb, E, vf_clip, norm_adv, adv_eps):
+        """(FlPpoOptions, pointer to the behaviour values or None), checked as the library checks them."""
+        vf_clip, adv_eps = float(vf_clip), float(adv_eps)
+        if not vf_clip >= 0:
+            raise ValueError("vf_clip must be >= 0 (0: no value clipping)")
+        if not (adv_eps >= 0 and math.isfinite(adv_eps)):
+            raise ValueError("adv_eps must be finite and >= 0")
+        if norm_adv not in (True, False, 0, 1):
+            raise ValueError("norm_adv must be a bool")
+        old = None
+        if vf_clip > 0:
+            if "values" not in mb:
+                raise KeyError("vf_clip > 0 needs mb['values'], the behaviour critic's values (Rollout.minibatch)")
+            t = mb["values"]
+            if t.device != self.device or t.dtype != torch.float32 or not t.is_contiguous() or tuple(t.shape) != (E,):
+                raise ValueError("values must be a contiguous float32 tensor of shape (%d,) on %s" % (E, self.device))
+            old = t.data_ptr()
+        return FlPpoOptions(vf_clip, int(bool(norm_adv)), adv_eps), old
 
     def _workspace(self, E, N):
         bf16 = self.precision == "bf16"
@@ -199,9 +232,10 @@ class PolicyLearner:
             self._ws = None
             self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
 
-    def _ppo_grad_shard(self, mb, E, N, clip_eps, vf_coef, ent_coef):
-        """ppo_grad of one rank's share: this rank's contribution computed with the minibatch's counts, then summed over the
-        group.  A share with no rows contributes zero counts, gradients and statistics and joins the same collectives."""
+    def _ppo_grad_shard(self, mb, E, N, clip_eps, vf_coef, ent_coef, opts):
+        """ppo_grad of one rank's share: this rank's contribution computed with the minibatch's counts (and, with norm_adv,
+        its advantage moments), then summed over the group.  A share with no rows contributes zero counts, moments, gradients
+        and statistics and joins the same collectives."""
         for p, v in zip(self._params.values(), self._grad_views):
             if p.grad is None or p.grad.data_ptr() != v.data_ptr() or p.grad.shape != v.shape or p.grad.stride() != v.stride():
                 p.grad = v
@@ -212,16 +246,25 @@ class PolicyLearner:
         else:
             self._counts.zero_()
         dist.all_reduce(self._counts, group=self.group)
+        norm = opts[0].norm_adv == 1
+        if norm:
+            if E > 0:
+                _check(self.lib.fl_policy_ppo_moments(E, N, mb["valid_actions"].data_ptr(), mb["acted"].data_ptr(),
+                                                      mb["advantages"].data_ptr(), self._moments.data_ptr(), stream),
+                       "fl_policy_ppo_moments")
+            else:
+                self._moments.zero_()
+            dist.all_reduce(self._moments, group=self.group)
         logits, value = self._outputs(E, N)
         if E > 0:
             self._workspace(E, N)
             params = FlPpoParams(float(clip_eps), float(vf_coef), float(ent_coef))
-            fn, name = (self.lib.fl_policy_ppo_grad_shard_bf16, "fl_policy_ppo_grad_shard_bf16") if self.precision == "bf16" \
-                else (self.lib.fl_policy_ppo_grad_shard_f32, "fl_policy_ppo_grad_shard_f32")
-            _check(fn(self._weights(), self._ws.data_ptr(), self._ws.numel(), E, N,
-                      *(mb[k].data_ptr() for k, _, _ in MB_KEYS), *(mb[k].data_ptr() for k, _ in ROW_KEYS),
-                      self._counts.data_ptr(), C.byref(params), self._ptrs(self._grad_views), logits.data_ptr(),
-                      value.data_ptr(), self._stats.data_ptr(), stream), name)
+            name = "fl_policy_ppo_grad_ex_bf16" if self.precision == "bf16" else "fl_policy_ppo_grad_ex_f32"
+            _check(getattr(self.lib, name)(self._weights(), self._ws.data_ptr(), self._ws.numel(), E, N,
+                                           *(mb[k].data_ptr() for k, _, _ in MB_KEYS), *(mb[k].data_ptr() for k, _ in ROW_KEYS),
+                                           self._counts.data_ptr(), C.byref(params), self._ptrs(self._grad_views),
+                                           logits.data_ptr(), value.data_ptr(), self._stats.data_ptr(), stream, opts[1],
+                                           self._moments.data_ptr() if norm else None, C.byref(opts[0])), name)
         else:
             self._flat.zero_()
         dist.all_reduce(self._flat, group=self.group)

@@ -21,7 +21,8 @@ LAYERS = pw.N_TRANSFORMER
 EXPORTS = ["fl_policy_abi_version", "fl_policy_workspace_bytes", "fl_policy_forward", "fl_policy_workspace_bytes_f32",
            "fl_policy_forward_f32", "fl_policy_workspace_bytes_grad_f32", "fl_policy_ppo_grad_f32", "fl_policy_workspace_bytes_grad_bf16",
            "fl_policy_ppo_grad_bf16", "fl_policy_forward_train_bf16", "fl_policy_tc_product_bf16", "fl_policy_ppo_counts",
-           "fl_policy_ppo_grad_shard_f32", "fl_policy_ppo_grad_shard_bf16", "fl_policy_choose_actions",
+           "fl_policy_ppo_grad_shard_f32", "fl_policy_ppo_grad_shard_bf16", "fl_policy_ppo_moments", "fl_policy_ppo_grad_ex_f32",
+           "fl_policy_ppo_grad_ex_bf16", "fl_policy_choose_actions",
            "fl_policy_sample_actions", "fl_policy_gae",
            "fl_policy_linear", "fl_policy_linear_debug", "fl_policy_debug_clocks", "fl_policy_launch_count"]
 
@@ -38,6 +39,11 @@ class FlPolicyWeights(C.Structure):
 class FlPpoParams(C.Structure):
     """Mirror of `struct FlPpoParams` (include/flatland_policy_b200.h)."""
     _fields_ = [("clip_eps", C.c_float), ("vf_coef", C.c_float), ("ent_coef", C.c_float)]
+
+
+class FlPpoOptions(C.Structure):
+    """Mirror of `struct FlPpoOptions` (include/flatland_policy_b200.h): clipped value loss and advantage normalisation."""
+    _fields_ = [("vf_clip", C.c_float), ("norm_adv", C.c_int32), ("adv_eps", C.c_float)]
 
 
 class FlTcProduct(C.Structure):
@@ -91,6 +97,12 @@ def lib():
     for name in ("fl_policy_ppo_grad_shard_f32", "fl_policy_ppo_grad_shard_bf16"):
         getattr(L, name).restype = C.c_int
         getattr(L, name).argtypes = [P, P, C.c_size_t, C.c_int64, C.c_int64] + [P] * 11 + [C.POINTER(FlPpoParams), P, P, P, P, P]
+    L.fl_policy_ppo_moments.restype = C.c_int
+    L.fl_policy_ppo_moments.argtypes = [C.c_int64, C.c_int64, P, P, P, P, P]
+    for name in ("fl_policy_ppo_grad_ex_f32", "fl_policy_ppo_grad_ex_bf16"):
+        getattr(L, name).restype = C.c_int
+        getattr(L, name).argtypes = [P, P, C.c_size_t, C.c_int64, C.c_int64] + [P] * 11 + [C.POINTER(FlPpoParams), P, P, P, P, P] + \
+            [P, P, C.POINTER(FlPpoOptions)]
     L.fl_policy_tc_product_bf16.restype = C.c_int
     L.fl_policy_tc_product_bf16.argtypes = [C.POINTER(FlTcProduct), P, C.c_size_t, P]
     L.fl_policy_choose_actions.restype = C.c_int

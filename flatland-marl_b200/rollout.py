@@ -117,7 +117,8 @@ class Rollout:
     def minibatch(self, row_ids):
         """Rows k * E + e (step k < T, environment e) of the last collect(), gathered into the dict PolicyLearner.ppo_grad
         takes: the observation tensors, valid_actions, actions and log_probs [M, N, ...] of those rows, advantages and returns
-        [M] of the last advantages() call, and acted [M].  row_ids: a sequence or tensor of ints; ids given on the host are
+        [M] of the last advantages() call, acted [M], and values [M] (the behaviour critic's value of each row, the V_old of
+        ppo_grad's vf_clip).  row_ids: a sequence or tensor of ints; ids given on the host are
         range-checked there, a device tensor is used as it is (no host synchronisation).  Plain torch gathers."""
         if not self._have_adv:
             raise ValueError("call advantages() after collect() before taking minibatches")
@@ -133,4 +134,5 @@ class Rollout:
         rows = lambda t: t[: self.T].reshape((n,) + tuple(t.shape[2:])).index_select(0, ids)
         mb = {k: rows(buf[k]) for k in self.MINIBATCH_KEYS}
         mb["advantages"], mb["returns"], mb["acted"] = rows(self._adv), rows(self._ret), rows(buf["acted"])
+        mb["values"] = rows(buf["values"])
         return mb

@@ -205,6 +205,64 @@ int fl_policy_ppo_grad_shard_bf16(const float *const *d_weights, void *d_workspa
                                   float *const *d_grads,
                                   float *d_logits, float *d_value, float *d_stats, void *stream);
 
+/* Options of the PPO loss: clipped value loss and advantage normalisation over the whole minibatch.  Every symbol (S, rows, A,
+ * R, V, r, the tie rule, the arithmetic) is that of fl_policy_ppo_grad_f32, and for a shard that of fl_policy_ppo_grad_shard_*.
+ *   - norm_adv = 1: A_S = the row advantage listed once per agent of S (the set the policy term averages over), of the whole
+ *     minibatch: n = |S_g|, and the float64 sums sum_S A, sum_S A^2 of all its shards.  mu = sum A / n; sigma = the unbiased
+ *     standard deviation, sqrt(max(0, (sum A^2 - (sum A)^2 / n) / (n - 1))), 0 when n < 2 (torch's A_S.std()).  Then
+ *       A_hat = (A - mu) / (sigma + adv_eps),  0 where sigma + adv_eps = 0,
+ *     formed in float64 and rounded once to fp32, replaces A everywhere in the policy term and in its statistics.
+ *   - vf_clip > 0: V_old = d_old_values [E] f32, the behaviour critic's value of the row, V_clip = V_old + clip(V - V_old,
+ *     -vf_clip, vf_clip), and the value term becomes vf_coef mean_rows(max((V - R)^2, (V_clip - R)^2)).  d/dV = 2 (V - R)
+ *     where (V - R)^2 >= (V_clip - R)^2, ties included, and 0 otherwise: exact, since the clipped square can only be strictly
+ *     larger when V lies outside the band, where V_clip does not depend on V.  Statistic 1 is the mean of that max term and
+ *     statistic 7 is L; the other statistics keep their meaning.
+ * vf_clip < 0 or NaN, norm_adv other than 0 and 1, adv_eps < 0 or not finite: FL_ERR_BAD_ARG. */
+typedef struct FlPpoOptions {
+    float   vf_clip;    /* > 0: clipped value loss with this half-width; 0: off */
+    int32_t norm_adv;   /* 1: normalise advantages over S of the whole minibatch; 0: off */
+    float   adv_eps;    /* >= 0 and finite */
+} FlPpoOptions;
+
+/* fl_policy_ppo_moments writes d_moments [2] f64 = [sum_S A, sum_S A^2] of these E rows (d_advantages [E] f32; S from
+ * d_valid_actions and d_acted as in fl_policy_ppo_counts).  One kernel on `stream` (one CTA, a fixed-order reduction, no
+ * atomics: the same inputs give the same bytes), no host synchronisation.  Argument errors as fl_policy_ppo_counts. */
+int fl_policy_ppo_moments(int64_t E, int64_t N, const uint8_t *d_valid_actions, const uint8_t *d_acted, const float *d_advantages,
+                          double *d_moments, void *stream);
+
+/* fl_policy_ppo_grad_ex_f32 / _bf16: fl_policy_ppo_grad_shard_f32 / _bf16 with the options above, arguments in the same order
+ * plus d_old_values (may be NULL when vf_clip == 0), d_global_moments ([sum_S A, sum_S A^2] f64 of the whole minibatch, the
+ * sum over its shards of fl_policy_ppo_moments, read on the device) and opts.
+ *   - d_global_counts NULL: these rows are the whole minibatch and their counts are computed in the workspace, as
+ *     fl_policy_ppo_grad_f32 / _bf16 do.  d_global_moments NULL likewise: the moments of these rows, computed in the
+ *     workspace.  d_global_moments is not read when norm_adv = 0.
+ *   - With vf_clip = 0 and norm_adv = 0 a call writes the bytes of fl_policy_ppo_grad_f32 / _bf16 (d_global_counts NULL) or
+ *     of fl_policy_ppo_grad_shard_f32 / _bf16, with the same launches: those four calls are this path with the options off.
+ *   - norm_adv = 1 with d_global_moments NULL adds one single-CTA launch (the moments); vf_clip adds none.  The workspace
+ *     size, the determinism and the one host synchronisation are those of fl_policy_ppo_grad_f32.
+ * FL_ERR_BAD_ARG before any CUDA call for the argument errors of fl_policy_ppo_grad_f32, a NULL opts, a bad option, a NULL
+ * d_old_values with vf_clip > 0, and d_global_moments without d_global_counts. */
+int fl_policy_ppo_grad_ex_f32(const float *const *d_weights, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
+                              const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
+                              const int32_t *d_node_order, const uint8_t *d_valid_actions,
+                              const uint8_t *d_actions, const float *d_old_log_probs,
+                              const float *d_advantages, const float *d_returns,
+                              const uint8_t *d_acted, const int64_t *d_global_counts,
+                              const FlPpoParams *params,
+                              float *const *d_grads,
+                              float *d_logits, float *d_value, float *d_stats, void *stream,
+                              const float *d_old_values, const double *d_global_moments, const FlPpoOptions *opts);
+int fl_policy_ppo_grad_ex_bf16(const float *const *d_weights, void *d_workspace, size_t workspace_bytes, int64_t E, int64_t N,
+                               const float *d_agent_attr, const float *d_forest, const int32_t *d_adjacency,
+                               const int32_t *d_node_order, const uint8_t *d_valid_actions,
+                               const uint8_t *d_actions, const float *d_old_log_probs,
+                               const float *d_advantages, const float *d_returns,
+                               const uint8_t *d_acted, const int64_t *d_global_counts,
+                               const FlPpoParams *params,
+                               float *const *d_grads,
+                               float *d_logits, float *d_value, float *d_stats, void *stream,
+                               const float *d_old_values, const double *d_global_moments, const FlPpoOptions *opts);
+
 /* One tensor-core product of fl_policy_ppo_grad_bf16, exposed for tests.  bf16-rounded operands, fp32 accumulation; every
  * other term in fp32.  X(m, k) = x1[row(m) ldx1 + k] (k < K1), x2[m ldx2 + k - K1] (K1 <= k < K = K1 + K2); row(m) = idx ?
  * idx[m] : m.  Row strides in floats.

@@ -17,6 +17,12 @@ the bf16 behaviour policy and the fp32 learner.  The card's name and power limit
 
     python tools/learner_bench.py --out profiles/learner_bench_b200.json [--calls 5]
     python tools/learner_bench.py --bf16 --out profiles/learner_bench_bf16_b200.json
+
+With --options the run times, instead, the loss options of ppo_grad: options off against norm_adv=True, vf_clip=0.2 on the
+same minibatch (mb["values"] the behaviour critic's), alternated call by call, for the fp32 and the bf16 learner at both
+shapes.  The difference is the moments launch and the options' arithmetic in the loss kernel.
+
+    python tools/learner_bench.py --options --out profiles/learner_bench_options_b200.json
 """
 import argparse
 import json
@@ -177,10 +183,46 @@ def run_case(config, E, T, calls, with_bf16=False):
     return r
 
 
+def run_options_case(config, E, T, calls):
+    """ppo_grad with the options off and on (norm_adv, vf_clip = 0.2), alternated call by call, both precisions."""
+    learner = fb.PolicyLearner(None, seed=0)
+    batch = fb.BatchedRailEnv(bench.load_worlds(config, E), auto_reset=True)
+    batch.reset()
+    actor = learner.actor("bf16")
+    for _ in range(10):
+        batch.step(actor.get_actions(batch.obs))
+    ro = fb.Rollout(batch, actor, T=T, seed=1234)
+    ro.collect()
+    ro.advantages()
+    mb = ro.minibatch(list(range(E)))
+    r = dict(config=config, rows=E, agents_per_row=batch.N, agents=E * batch.N)
+    names = ("policy_loss", "value_loss", "entropy", "approx_kl", "clip_fraction", "S", "acted_rows", "loss")
+    for prec in ("fp32", "bf16"):
+        lr = learner if prec == "fp32" else fb.PolicyLearner(learner.state_dict(), seed=0, precision="bf16")
+        off = lambda: lr.ppo_grad(mb)
+        on = lambda: lr.ppo_grad(mb, vf_clip=0.2, norm_adv=True)
+        s_off, s_on = off().cpu().numpy(), on().cpu().numpy()
+        t_off, t_on = [], []
+        for _ in range(calls):
+            t_off.append(timed(off))
+            t_on.append(timed(on))
+        med = lambda x: round(float(np.median(x)), 3)
+        r[prec] = dict(off_ms=med(t_off), on_ms=med(t_on), on_minus_off_ms=round(med(t_on) - med(t_off), 3),
+                       off_ms_calls=[round(x, 3) for x in t_off], on_ms_calls=[round(x, 3) for x in t_on],
+                       stats_off=dict(zip(names, [float(x) for x in s_off])), stats_on=dict(zip(names, [float(x) for x in s_on])))
+        if lr is not learner:
+            del lr
+    print(json.dumps(r), flush=True)
+    del ro, batch, learner
+    torch.cuda.empty_cache()
+    return r
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--calls", type=int, default=5, help="alternated timed calls per implementation")
     ap.add_argument("--bf16", action="store_true", help="also time the bf16 learner and profile both")
+    ap.add_argument("--options", action="store_true", help="time ppo_grad's loss options off against on, both precisions")
     ap.add_argument("--out", required=True, help="JSON file the results are written to (its directory is created)")
     args = ap.parse_args()
     if not torch.cuda.is_available():
@@ -192,7 +234,10 @@ def main():
         power = "unknown"
     out = dict(gpu=torch.cuda.get_device_name(0), power_limit=power, calls=args.calls)
     print(json.dumps(out), flush=True)
-    out["cases"] = [run_case(config, E, T, args.calls, args.bf16) for config, E, T in CASES]
+    if args.options:
+        out["cases"] = [run_options_case(config, E, T, args.calls) for config, E, T in CASES]
+    else:
+        out["cases"] = [run_case(config, E, T, args.calls, args.bf16) for config, E, T in CASES]
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, "w") as f:
         json.dump(out, f, indent=1)
